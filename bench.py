@@ -2,6 +2,7 @@
 """bench.py -- poses/sec of full DDIM sampling (H hypotheses x T steps) through diffpose_nw_b200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cpn1024|gt1024x5|sweep|sweep1m|twostage|evalloop]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -13,10 +14,17 @@ strong-sharded over the ranks; sweep1m = configs[3] at any N; twostage = configs
 
   value      device-timed throughput, inputs already resident in HBM (rotating through a pool larger than L2)
   e2e        same metric through the public API with pinned HOST buffers: H2D of x and D2H of x_T inside the timed region
+  --steps K  the number of timed steps, in the device-timed region and again in the e2e one (host clock: K >= 200 steadies it)
   roofline   tensor bound: algorithmic FLOPs (24.65 MFLOP per pose-forward, SURVEY.md 8d) / dp_sample device time
   cpu_baseline  the oracle port (PyTorch CPU restatement of the reference) timed on the host cores, bounded sample
   --impl reference   the reference's CPU implementation of the path (oracle port; the reference is pure Python and
                      /root/reference does not exist on the GPU box) on all host threads, same config/metric.
+  --dump-outputs DIR  after every measurement, write the arrays the last timed step returned to its caller as DIR/<name>.npy:
+                     x_T (float32: the sampled poses; the hypothesis mean when H > 1) and, for evalloop, metric_sums (float64
+                     [sum MPJPE, sum P-MPJPE, poses] accumulated over the K timed steps).  Inputs and weights are seeded, so two
+                     builds run with the same arguments can be compared output for output.  At most 64 MB (64 000 000 bytes)
+                     in all: a larger array keeps a fixed, seeded sample of its rows.  With N ranks every rank writes
+                     <name>_rank<r>.npy.  Choose a DIR outside the source tree.
 """
 from __future__ import annotations
 
@@ -33,6 +41,8 @@ sys.path.insert(0, ROOT)
 
 FLOP_PER_POSE_FORWARD = 24.65e6          # minimal algorithmic work, SURVEY.md section 8d
 ROW_BYTES = 17 * 5 * 4                   # one uvxyz pose, fp32
+DUMP_BYTES = 64_000_000                  # --dump-outputs: all files of all ranks together, .npy headers included
+NPY_HEADER_BYTES = 4096                  # room kept per file for its .npy header (128 bytes for these shapes)
 METRIC = "poses/sec, full DDIM sampling (H hyps x T steps)"
 
 WORKLOADS = {
@@ -100,6 +110,22 @@ def ncu_traffic():
 def l2_note(pool_n, batch_bytes):
     return (f"inputs rotate through a pool of {pool_n} distinct buffers = {pool_n * batch_bytes / 2**20:.0f} MiB (> 126 MiB L2), written once at set-up in "
             "order, so every timed step reads a batch that is not cache resident; weights (1.6 MB) stay L2-resident by design")
+
+
+def dump_outputs(path, arrays, budget, suffix=""):
+    """Write each tensor as path/<name><suffix>.npy, the files together at most `budget` bytes.  One whose data does not fit
+    its share (less the room for its header) keeps a sorted sample of its rows drawn with a fixed seed, so the same
+    arguments select the same rows in every run."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = budget // len(arrays) - NPY_HEADER_BYTES
+    for name, t in arrays.items():
+        a = t.cpu().numpy()
+        if a.nbytes > share:
+            row_bytes = a.nbytes // a.shape[0]
+            keep = np.random.default_rng(0).choice(a.shape[0], max(0, share) // row_bytes, replace=False)
+            a = a[np.sort(keep)]
+        np.save(os.path.join(path, name + suffix + ".npy"), a)
 
 
 def bench_config(wl, world):
@@ -232,11 +258,16 @@ def main():
     ap.add_argument("--workload", default="cpn1024", choices=sorted(WORKLOADS))
     ap.add_argument("--engine", default="auto", choices=["auto", "fp32", "tcx", "tcg"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm times a slice sized by its own speed")
         return run_reference(args, wl)
 
     import torch
@@ -348,6 +379,8 @@ def main():
         out = step(args.steps + args.warmup + i)
     timing_note = (f"{ramp} set-up + {args.warmup} warm-up steps, barrier + synchronize, {lead_in} untimed lead-in steps, CUDA event, "
                    f"{args.steps} timed steps, CUDA event, barrier + synchronize")
+    if args.dump_outputs and wl.get("with_metrics"):
+        msums.zero_()       # the dumped sums then cover exactly the K timed steps
     l0 = _lib.launch_count()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     if sampler:
@@ -359,6 +392,11 @@ def main():
     barrier()
     if sampler:
         sampler.t1 = time.time()
+    dump = None
+    if args.dump_outputs:       # held on the device (the e2e leg adds to msums) and written after every measurement
+        dump = {"x_T": out}
+        if wl.get("with_metrics"):
+            dump["metric_sums"] = msums.clone()
     gc.enable()
     launches = _lib.launch_count() - l0
     ms = ev0.elapsed_time(ev1)
@@ -400,9 +438,9 @@ def main():
 
         host_tg = targets.cpu().pin_memory() if (wl.get("with_metrics") and hs is not None) else None      # evaluation: targets travel with the batch
         hs_sums = msums if host_tg is not None else None
-        # at least 200 batches (>= 20 ms): a host-clock window of 20 batches (2 ms) measures scheduling jitter of the rank
-        # processes rather than the pipeline (8 ranks, max over ranks: 0.87 "efficiency" at 20 batches, 0.99 at 2000)
-        e_steps = min(max(args.steps, 200), 2000) if poses_per_step * H * T <= 200000 else max(3, min(args.steps, 200))
+        # K batches, as in the device-timed region.  A host-clock window of 20 batches (2 ms) measures scheduling jitter of the
+        # rank processes as much as the pipeline (8 ranks, max over ranks: 0.87 "efficiency" at 20 batches, 0.99 at 2000)
+        e_steps = args.steps
         last = None
         for i in range(3):
             e2e_serial(i) if hs is None else hs.submit(host_in[i & 1], host_tg, hs_sums)
@@ -471,6 +509,8 @@ def main():
             line["cpu_baseline"] = {"value": v, "unit": "poses/s", "cores": os.cpu_count() or 1, "kind": "port",
                                     "sample": f"{n_cpu}-pose slice of the workload (H={H}, T={T}), {reps} reps in {dt:.1f} s after 1 warm-up, torch CPU threads={os.cpu_count()}"}
         print(json.dumps(line), flush=True)
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump, DUMP_BYTES // world, f"_rank{rank}" if world > 1 else "")
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()

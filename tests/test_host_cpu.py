@@ -200,8 +200,8 @@ def test_ema_helper_and_copies_keep_no_stale_state():
     ema.ema(m)
     assert m._packed_version is None, "EMAHelper.ema() must invalidate the packed device copy"
     want = p.detach().clone()
-    m2 = ema.ema_copy(torch.nn.DataParallel(m))
-    assert isinstance(m2, torch.nn.DataParallel) and torch.equal(m2.module.atten_layers[2].self_attn.linears[1].weight, want)
+    m2 = ema.ema_copy(torch.nn.DataParallel(m))     # with a GPU visible, the module may now live on cuda:0
+    assert isinstance(m2, torch.nn.DataParallel) and torch.equal(m2.module.atten_layers[2].self_attn.linears[1].weight.cpu(), want)
     assert set(ema.state_dict()) == {k for k, _ in m.named_parameters()}
     m._handle = "native pointer"
     c = copy.deepcopy(m)
@@ -242,3 +242,52 @@ def test_bench_reference_arm_contract():
     assert set(d["config"]) == {"workload", "batch", "batch_is", "n_hyp", "T", "eta", "l2"}
     for name, wl in bench.WORKLOADS.items():      # every workload names a BASELINE config and a schedule inside the 51-entry beta table
         assert "configs[" in wl["name"] and max(wl["seq"]) < 51 and wl["batch"] >= 1
+
+
+def test_bench_dump_outputs_stays_in_budget(tmp_path):
+    """`bench.py --dump-outputs`: the files of all ranks together stay within 64 MB (headers included) even for the
+    million-pose output of sweep1m; a larger array keeps the same seeded, sorted sample of rows in every run; a small one
+    is written whole; names carry the rank suffix only when it is given."""
+    import bench
+    n = 1_000_000
+    x = torch.arange(n, dtype=torch.float32)[:, None, None].expand(n, 17, 5)      # every value of a row is its index
+    sums = torch.tensor([1.0, 2.0, 3.0], dtype=torch.float64)
+
+    def written(d):
+        return {f: os.path.getsize(os.path.join(d, f)) for f in os.listdir(d)}
+
+    for arrays in ({"x_T": x}, {"x_T": x, "metric_sums": sums}):
+        runs = []
+        for k in range(2):
+            d = str(tmp_path / f"{len(arrays)}_{k}")
+            bench.dump_outputs(d, arrays, bench.DUMP_BYTES)
+            files = written(d)
+            assert set(files) == {name + ".npy" for name in arrays} and sum(files.values()) <= bench.DUMP_BYTES
+            runs.append(np.load(os.path.join(d, "x_T.npy")))
+        a, b = runs
+        assert a.dtype == np.float32 and a.shape[1:] == (17, 5) and 0.9 * bench.DUMP_BYTES / len(arrays) < a.nbytes
+        assert np.array_equal(a, b)
+        rows = a[:, 0, 0]
+        assert (np.diff(rows) > 0).all() and (a == rows[:, None, None]).all()
+        if "metric_sums" in arrays:
+            s = np.load(os.path.join(str(tmp_path / "2_0"), "metric_sums.npy"))
+            assert s.dtype == np.float64 and np.array_equal(s, sums.numpy())
+    world = 4
+    d = str(tmp_path / "ranks")
+    for r in range(world):
+        bench.dump_outputs(d, {"x_T": x}, bench.DUMP_BYTES // world, f"_rank{r}")
+    files = written(d)
+    assert set(files) == {f"x_T_rank{r}.npy" for r in range(world)} and sum(files.values()) <= bench.DUMP_BYTES
+    small = torch.randn(1024, 17, 5)
+    bench.dump_outputs(str(tmp_path / "small"), {"x_T": small}, bench.DUMP_BYTES)
+    assert np.array_equal(np.load(str(tmp_path / "small" / "x_T.npy")), small.numpy())
+
+
+def test_bench_rejects_bad_arguments(tmp_path):
+    """No timed step (--steps 0) and a dump of the reference arm are argument errors, reported before any work."""
+    import subprocess
+    import sys
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "out")]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=300)
+        assert out.returncode == 2 and "error:" in out.stderr and out.stdout == "", (extra, out.stderr[-500:])
+    assert os.listdir(tmp_path) == []
