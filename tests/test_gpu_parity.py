@@ -334,21 +334,64 @@ def test_mask_device_copy_is_cached_and_follows_in_place_edits():
 
 
 def test_metrics_kernel_many_poses_vs_oracle():
-    """The warp-per-pose MPJPE / P-MPJPE kernel on 3001 random poses (several grid strides, ragged last block) against the
-    oracle's restatement of common/loss.py (numpy float64 SVD per pose), including mirrored poses (reflection branch)."""
+    """The warp-per-pose MPJPE / P-MPJPE kernel against the oracle's restatement of common/loss.py (numpy float64 SVD per
+    pose) on 2 x 9472 + 13 poses: the grid is capped at 148 x 8 blocks of 8 warps (9472 poses per pass), so the grid-stride
+    loop runs three passes, the last one ragged.  Mirrored predictions (reflection branch), and the edges of svd3 /
+    pose_errors spread over all passes: planar targets and predictions of thickness 0, 1e-6 and 1e-4 m (rank-deficient
+    cross-covariance; on exactly planar sets zeta * zeta overflows to inf and the rotation angle comes out 0, not NaN), a
+    collinear prediction (rank 1), pred == gt, a similarity transform with and without a reflection, a camera-frame offset
+    (root at z = 5 m), millimetre units (tolerance x 1000), and a zero-extent prediction, where the reference divides 0 by
+    0: its P-MPJPE is NaN and the kernel's must be too."""
     g = torch.Generator().manual_seed(77)
-    n = 3001
+    n = 2 * 148 * 8 * 8 + 13
     gt = torch.randn(n, 17, 3, generator=g) * 0.3
     pred = gt + torch.randn(n, 17, 3, generator=g) * 0.05
     pred[::7, :, 0] *= -1.0                      # mirrored predictions: det(R) < 0 before the sign fix
-    pred[5] = gt[5] * 1.7 + 0.3                  # a pure similarity transform: P-MPJPE ~ 0
-    sums, pp = D.pose_error_sums(pred.to(dev()), gt.to(dev()), per_pose=True)
-    want_p = O.p_mpjpe_per_pose(O.root_centre(pred).numpy(), O.root_centre(gt).numpy())
-    want_m = (O.root_centre(pred) - O.root_centre(gt)).norm(dim=-1).mean(dim=-1).numpy()
-    np.testing.assert_allclose(pp[:, 0].cpu().numpy(), want_m, atol=2e-7)
-    np.testing.assert_allclose(pp[:, 1].cpu().numpy(), want_p, atol=1e-6)
-    s = sums.cpu().numpy()
-    assert s[2] == n and abs(s[0] - want_m.astype(np.float64).sum()) < 1e-4 and abs(s[1] - want_p.sum()) < 1e-4
+    noise = lambda: torch.randn(17, 3, generator=g) * 0.05
+    q, _ = torch.linalg.qr(torch.randn(3, 3, generator=g, dtype=torch.float64))
+    rot = (q * torch.sign(torch.linalg.det(q))).float()                       # det +1
+    refl = rot @ torch.diag(torch.tensor([1.0, 1.0, -1.0]))                   # det -1
+    special = {}
+    for th in (0.0, 1e-6, 1e-4):
+        special[f"planar gt {th:g}"] = lambda gi, th=th: (gi * torch.tensor([1, 1, th / 0.3]),) * 2
+        special[f"planar pred {th:g}"] = lambda gi, th=th: (gi, (gi + noise()) * torch.tensor([1, 1, th / 0.3]))
+        special[f"planar both {th:g}"] = lambda gi, th=th: (gi * torch.tensor([1, 1, th / 0.3]), (gi + noise()) * torch.tensor([1, 1, th / 0.3]))
+    special["collinear pred"] = lambda gi: (gi, torch.randn(17, 1, generator=g) * 0.3 * torch.tensor([[0.48, -0.6, 0.64]]))
+    special["pred == gt"] = lambda gi: (gi, gi.clone())
+    special["similarity"] = lambda gi: (gi, 1.7 * gi @ rot + 0.3)             # P-MPJPE ~ 0
+    special["similarity + reflection"] = lambda gi: (gi, 1.7 * gi @ refl + 0.3)
+    special["camera frame"] = lambda gi: (gi + torch.tensor([0.1, -0.2, 5.0]), gi + noise() + torch.tensor([0.1, -0.2, 5.0]))
+    special["zero extent"] = lambda gi: (gi, torch.full((17, 3), 0.2))
+    where = {}
+    for k, (name, make) in enumerate(special.items()):
+        i = n - 1 if name == "zero extent" else 3 + k * (n // len(special))
+        if name.startswith("planar gt"):
+            gt[i], _ = make(gt[i])
+            pred[i] = gt[i] + noise()
+        else:
+            gt[i], pred[i] = make(gt[i])
+        where[name] = i
+    nan_row = where["zero extent"]
+    for unit in (1.0, 1000.0):                   # metres, millimetres
+        p, t_ = pred * unit, gt * unit
+        sums, pp = D.pose_error_sums(p.to(dev()), t_.to(dev()), per_pose=True)
+        # the zero-extent pose: the reference's y0 / ny is 0 / 0 = NaN, on which numpy's SVD then raises; the kernel has no
+        # exception to raise and must return NaN rather than a number
+        want_p = np.full(n, np.nan)
+        want_p[:-1] = O.p_mpjpe_per_pose(O.root_centre(p[:-1]).numpy(), O.root_centre(t_[:-1]).numpy())
+        want_m = (O.root_centre(p) - O.root_centre(t_)).norm(dim=-1).mean(dim=-1).numpy()
+        got = pp.cpu().numpy()
+        for name, i in where.items():
+            print(f"metrics unit={unit:g} {name}: mpjpe {got[i, 0]:.6g} (ref {want_m[i]:.6g}) p_mpjpe {got[i, 1]:.6g} (ref {want_p[i]:.6g})")
+        np.testing.assert_allclose(got[:, 0], want_m, atol=2e-7 * unit)
+        np.testing.assert_allclose(got[:, 1], want_p, atol=1e-6 * unit)   # NaN exactly where the reference has NaN
+        assert nan_row == n - 1 and np.isnan(got[nan_row, 1])
+        assert np.isfinite(got[np.arange(n) != nan_row]).all()
+        s = sums.cpu().numpy()
+        assert s[2] == n and abs(s[0] - want_m.astype(np.float64).sum()) < 1e-4 * unit and np.isnan(s[1])
+        s2, _ = D.pose_error_sums(p[:-1].to(dev()), t_[:-1].to(dev()))     # without the zero-extent pose (the last row)
+        s2 = s2.cpu().numpy()
+        assert s2[2] == n - 1 and abs(s2[1] - want_p[:-1].sum()) < 1e-4 * unit
 
 
 @pytest.mark.parametrize("engine", ["fp32", "tcx", "auto"])
