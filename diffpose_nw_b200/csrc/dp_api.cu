@@ -5,6 +5,7 @@
 #include <cstring>
 #include <new>
 #include "dp_internal.h"
+#include "dp_tc_layout.cuh"
 
 namespace dp {
 
@@ -13,17 +14,6 @@ static std::atomic<long> g_launches{0};
 
 void set_error(const std::string& msg) { g_err = msg; }
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-
-int ensure_capacity(float** p, size_t* cap, size_t need_floats) {
-  if (*cap >= need_floats && *p != nullptr) return DP_OK;
-  if (*p) cudaFree(*p);
-  *p = nullptr;
-  *cap = 0;
-  size_t n = need_floats < 1024 ? 1024 : need_floats;
-  DP_CUDA(cudaMalloc(reinterpret_cast<void**>(p), n * sizeof(float)));
-  *cap = n;
-  return DP_OK;
-}
 
 // dst[k*ld + col0 + n] = src[n*K + k]: a torch.nn.Linear weight [N][K] becomes an input-major [K][N] panel.
 __global__ void pack_transpose_kernel(float* __restrict__ dst, const float* __restrict__ src, int K, int N, int ld,
@@ -231,7 +221,7 @@ static int pack_fp32(dp_model* m, const float* p, const float* adj_host, cudaStr
   DP_CUDA(cudaMemcpyAsync(mut(w.t2m), t2m.data(), P * sizeof(float), cudaMemcpyHostToDevice, s));
   DP_CUDA(cudaMemcpyAsync(mut(w.t1s), t1s.data(), NP * sizeof(float), cudaMemcpyHostToDevice, s));
   DP_CUDA(cudaMemcpyAsync(mut(w.t2s), t2s.data(), NP * sizeof(float), cudaMemcpyHostToDevice, s));
-  DP_CUDA(cudaMemcpyAsync(m->dw, &m->hw, sizeof(Weights), cudaMemcpyHostToDevice, s));
+  DP_CUDA(cudaMemcpyAsync(m->dw.get<Weights>(), &m->hw, sizeof(Weights), cudaMemcpyHostToDevice, s));
   // the host vectors above go out of scope: finish the copies first (pack is not on the hot path)
   DP_CUDA(cudaStreamSynchronize(s));
   return DP_OK;
@@ -257,9 +247,38 @@ static int check_device(dp_handle h, const char* what) {
 // engine that runs a forward call: AUTO -> the split-precision engine (a forward output is not damped by a DDIM schedule,
 // so it gets the accurate path), explicit settings are honoured
 static int forward_engine(dp_handle h) {
-  if (h->engine == DP_ENGINE_FP32 || !tc2_supported(h->d)) return DP_ENGINE_FP32;
+  if (h->engine == DP_ENGINE_FP32 || !tc_supported(h->d)) return DP_ENGINE_FP32;
   if (h->engine == DP_ENGINE_TCG) return DP_ENGINE_TCG;
   return DP_ENGINE_TCX;
+}
+
+static int run_engine(dp_handle h, int eng, const EngineCall& c, cudaStream_t s) {
+  if (eng == DP_ENGINE_TCG) return tc2_run(h, c, s);
+  if (eng == DP_ENGINE_TCX) return tcx_run(h, c, s);
+  return simt_run(h, c, s);
+}
+
+// GCNdiff.forward / GCNpose.forward (models/gcndiff.py:101-113, models/gcnpose.py:101-113): one pass with per-sample
+// timesteps, in chunks that bound the per-sample embedding table (chunk * n_layer * hid floats).  That table goes into
+// the buffer the sampler caches its per-step table in, so that cache is dropped.  emit_uvxyz (tcx only): out is
+// [n][n_pts][c_in + c_out] = [uv | xyz - xyz_root] (runners/diffpose_frame.py:337-343).
+static int forward_chunks(dp_handle h, int eng, const float* x, const float* t, const unsigned char* mask, float* out, long n,
+                          bool emit_uvxyz, cudaStream_t s) {
+  const Dims& d = h->d;
+  const long chunk = 1L << 16;
+  const int wd = emit_uvxyz ? d.c_in + d.c_out : d.c_out;
+  const StepsArg none{};
+  if (d.has_temb) h->temb_t.clear();
+  for (long o = 0; o < n; o += chunk) {
+    const long nn = (n - o < chunk) ? (n - o) : chunk;
+    if (d.has_temb) DP_TRY(simt_temb(h, t + o, 1, nullptr, nn, s));
+    EngineCall c;
+    c.x_in = x + (size_t)o * d.n_pts * d.c_in; c.x_is_repeated = 1; c.out = out + (size_t)o * d.n_pts * wd;
+    c.n_pose = nn; c.inl = &none; c.mask = mask; c.forward_only = true;
+    c.emit_uvxyz = emit_uvxyz;
+    DP_TRY(run_engine(h, eng, c, s));
+  }
+  return DP_OK;
 }
 
 extern "C" {
@@ -282,21 +301,19 @@ int dp_create(dp_handle* out, int n_pts, int c_in, int c_out, int hid, int n_lay
   DP_REQUIRE(m != nullptr, "dp_create: out of host memory");
   m->d = Dims{n_pts, c_in, c_out, hid, n_layer, n_head, has_temb ? 1 : 0};
   m->n_params = param_count(m->d);
+  Weights tmp{};
+  m->blob_floats = carve(tmp, m->d, nullptr);
   cudaError_t e = cudaGetDevice(&m->device);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&m->sm_count, cudaDevAttrMultiProcessorCount, m->device);
-  if (e == cudaSuccess) {
-    Weights tmp{};
-    m->blob_floats = carve(tmp, m->d, nullptr);
-    e = cudaMalloc(reinterpret_cast<void**>(&m->blob), m->blob_floats * sizeof(float));
-  }
-  if (e == cudaSuccess) e = cudaMemset(m->blob, 0, m->blob_floats * sizeof(float));
-  if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&m->dw), sizeof(Weights));
+  if (e == cudaSuccess && (m->blob.reserve(m->blob_floats * sizeof(float)) != DP_OK || m->dw.reserve(sizeof(Weights)) != DP_OK))
+    e = cudaErrorMemoryAllocation;
+  if (e == cudaSuccess) e = cudaMemset(m->blob.get<float>(), 0, m->blob_floats * sizeof(float));
   if (e != cudaSuccess) {
     set_error(std::string("dp_create: ") + cudaGetErrorString(e));
-    dp_destroy(m);
+    delete m;
     return DP_ERR_CUDA;
   }
-  carve(m->hw, m->d, m->blob);
+  carve(m->hw, m->d, m->blob.get<float>());
   *out = m;
   return DP_OK;
 }
@@ -312,8 +329,8 @@ int dp_pack(dp_handle h, const float* params, long n_floats, const float* adj_ho
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   DP_TRY(check_device(h, "dp_pack"));
   DP_TRY(pack_fp32(h, params, adj_host, s));
-  tcx_invalidate(h);                          // the split-precision blocks are rebuilt lazily, on that engine's next use
-  if (tc2_supported(h->d)) DP_TRY(tc2_pack(h, s));
+  h->tcx_packed = false;                      // the split-precision blocks are rebuilt lazily, on that engine's next use
+  if (tc_supported(h->d)) DP_TRY(tc2_pack(h, s));
   h->temb_t.clear();
   h->packed = true;
   return DP_OK;
@@ -322,7 +339,7 @@ int dp_pack(dp_handle h, const float* params, long n_floats, const float* adj_ho
 int dp_set_engine(dp_handle h, int engine) {
   DP_REQUIRE(h, "dp_set_engine: NULL handle");
   DP_REQUIRE(engine == DP_ENGINE_AUTO || engine == DP_ENGINE_FP32 || engine == DP_ENGINE_TCX || engine == DP_ENGINE_TCG, "dp_set_engine: unknown engine");
-  if ((engine == DP_ENGINE_TCX && !tcx_supported(h->d)) || (engine == DP_ENGINE_TCG && !tc2_supported(h->d))) {
+  if ((engine == DP_ENGINE_TCX || engine == DP_ENGINE_TCG) && !tc_supported(h->d)) {
     set_error("dp_set_engine: the tensor-core engines need hid_dim=96, n_head=4, n_pts=17 and coords_dim <= 5");
     return DP_ERR_UNSUPPORTED;
   }
@@ -332,7 +349,7 @@ int dp_set_engine(dp_handle h, int engine) {
 
 int dp_get_engine(dp_handle h) {
   if (!h) return DP_ERR_INVALID;
-  if (h->engine == DP_ENGINE_FP32 || !tc2_supported(h->d)) return DP_ENGINE_FP32;
+  if (h->engine == DP_ENGINE_FP32 || !tc_supported(h->d)) return DP_ENGINE_FP32;
   if (h->engine == DP_ENGINE_TCX) return DP_ENGINE_TCX;
   return DP_ENGINE_TCG;   // AUTO = the fp16-operand tensor-core engine (its error is damped by the DDIM schedule)
 }
@@ -349,14 +366,7 @@ int dp_forward(dp_handle h, const float* x, const float* t, const unsigned char*
   DP_REQUIRE(!h->d.has_temb || t != nullptr, "dp_forward: t is required for the diffusion denoiser");
   if (n == 0) return DP_OK;
   DP_TRY(check_device(h, "dp_forward"));
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  // Per-sample timesteps need a per-sample embedding table (computed in chunks into the same buffer the sampler caches
-  // its per-step table in, so that cache is dropped).
-  if (h->d.has_temb) h->temb_t.clear();
-  const int eng = forward_engine(h);
-  if (eng == DP_ENGINE_TCX) return tcx_forward(h, x, t, mask, out, n, 0, s);
-  if (eng == DP_ENGINE_TCG) return tc2_forward(h, x, t, mask, out, n, s);
-  return simt_forward(h, x, t, mask, out, n, s);
+  return forward_chunks(h, forward_engine(h), x, t, mask, out, n, false, static_cast<cudaStream_t>(stream));
 }
 
 int dp_lift(dp_handle h, const float* uv, const unsigned char* mask, float* out_uvxyz, long n, void* stream) {
@@ -368,12 +378,12 @@ int dp_lift(dp_handle h, const float* uv, const unsigned char* mask, float* out_
   DP_TRY(check_device(h, "dp_lift"));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int eng = forward_engine(h);
-  if (eng == DP_ENGINE_TCX) return tcx_forward(h, uv, nullptr, mask, out_uvxyz, n, 1, s);   // glue fused into the kernel's store
+  if (eng == DP_ENGINE_TCX) return forward_chunks(h, eng, uv, nullptr, mask, out_uvxyz, n, true, s);   // glue fused into the kernel's store
   const Dims& d = h->d;
-  DP_TRY(ensure_capacity(&h->lift_scratch, &h->lift_cap, (size_t)n * d.n_pts * d.c_out));
-  if (eng == DP_ENGINE_TCG) DP_TRY(tc2_forward(h, uv, nullptr, mask, h->lift_scratch, n, s));
-  else DP_TRY(simt_forward(h, uv, nullptr, mask, h->lift_scratch, n, s));
-  return lift_glue_launch(uv, h->lift_scratch, out_uvxyz, n, d.n_pts, d.c_in, d.c_out, s);
+  DP_TRY(h->lift_scratch.reserve((size_t)n * d.n_pts * d.c_out * sizeof(float)));
+  float* xyz = h->lift_scratch.get<float>();
+  DP_TRY(forward_chunks(h, eng, uv, nullptr, mask, xyz, n, false, s));
+  return lift_glue_launch(uv, xyz, out_uvxyz, n, d.n_pts, d.c_in, d.c_out, s);
 }
 
 static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
@@ -395,20 +405,15 @@ static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float*
   } else {
     // long schedules (> 64 steps) live in a device buffer that is uploaded when the schedule CHANGES, not per call; the
     // upload reads the handle's own copy, and the one synchronisation below only happens on such a change
-    const bool same = h->steps != nullptr && h->steps_host.size() == (size_t)n_steps &&
+    const bool same = h->steps.get<dp_step>() != nullptr && h->steps_host.size() == (size_t)n_steps &&
                       std::memcmp(h->steps_host.data(), steps_host, n_steps * sizeof(dp_step)) == 0;
     if (!same) {
-      if (h->steps_cap < (size_t)n_steps) {
-        if (h->steps) cudaFree(h->steps);
-        h->steps = nullptr; h->steps_cap = 0;
-        DP_CUDA(cudaMalloc(reinterpret_cast<void**>(&h->steps), (size_t)n_steps * sizeof(dp_step)));
-        h->steps_cap = n_steps;
-      }
+      DP_TRY(h->steps.reserve((size_t)n_steps * sizeof(dp_step)));
       h->steps_host.assign(steps_host, steps_host + n_steps);
-      DP_CUDA(cudaMemcpyAsync(h->steps, h->steps_host.data(), n_steps * sizeof(dp_step), cudaMemcpyHostToDevice, s));
+      DP_CUDA(cudaMemcpyAsync(h->steps.get<dp_step>(), h->steps_host.data(), n_steps * sizeof(dp_step), cudaMemcpyHostToDevice, s));
       DP_CUDA(cudaStreamSynchronize(s));
     }
-    steps_dev = h->steps;
+    steps_dev = h->steps.get<dp_step>();
   }
   // batch-invariant time embeddings: one row per step (models/gcndiff.py:103-106, :51).  The table depends only
   // on the weights and the schedule, so it is kept across calls until either changes.
@@ -417,30 +422,30 @@ static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float*
     for (int i = 0; same && i < n_steps; ++i) same = (h->temb_t[i] == steps_host[i].t);
     if (!same) {
       DP_TRY(simt_temb(h, steps_dev ? &steps_dev->t : nullptr, sizeof(dp_step) / sizeof(float), &inl, n_steps, s));
-      if (tc2_supported(d)) DP_TRY(tc2_tau(h, n_steps, s));
+      if (tc_supported(d)) DP_TRY(tc2_tau(h, n_steps, s));
       h->temb_t.resize(n_steps);
       for (int i = 0; i < n_steps; ++i) h->temb_t[i] = steps_host[i].t;
     }
   }
 
+  EngineCall c;
+  c.x_in = x_in; c.x_is_repeated = x_is_repeated; c.out = x_out; c.n_pose = n_pose; c.n_hyp = n_hyp;
+  c.n_steps = n_steps; c.steps_dev = steps_dev; c.inl = &inl; c.noise = noise; c.mask = mask;
+  const bool mean = mean_over_hyp && n_hyp > 1;
   const int eng = dp_get_engine(h);
   // default engine: the hypothesis mean -- and, for dp_sample_eval, the MPJPE / P-MPJPE sums -- are fused into the kernel's
   // final store (one launch, no [H*B] scratch)
-  if (eng == DP_ENGINE_TCG)
-    return tc2_sample(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_dev, &inl, n_steps, noise, mask, mean_over_hyp, targets, sums, s);
-  float* dst = x_out;
-  const int row_floats = d.n_pts * d.c_out;
-  if (mean_over_hyp && n_hyp > 1) {
-    DP_TRY(ensure_capacity(&h->hyp_scratch, &h->hyp_cap, (size_t)n_pose * n_hyp * row_floats));
-    dst = h->hyp_scratch;
+  if (eng == DP_ENGINE_TCG) {
+    c.mean_over_hyp = mean; c.gt = targets; c.sums = sums;
+    return tc2_run(h, c, s);
   }
-  int rc;
-  if (eng == DP_ENGINE_TCX)
-    rc = tcx_sample(h, x_in, x_is_repeated, dst, n_pose, n_hyp, steps_dev, &inl, n_steps, noise, mask, s);
-  else
-    rc = simt_sample(h, x_in, x_is_repeated, dst, n_pose, n_hyp, steps_dev, &inl, n_steps, noise, mask, s);
-  if (rc != DP_OK) return rc;
-  if (mean_over_hyp && n_hyp > 1) DP_TRY(hyp_mean_launch(dst, x_out, n_pose, n_hyp, row_floats, s));
+  const int row_floats = d.n_pts * d.c_out;
+  if (mean) {
+    DP_TRY(h->hyp_scratch.reserve((size_t)n_pose * n_hyp * row_floats * sizeof(float)));
+    c.out = h->hyp_scratch.get<float>();
+  }
+  DP_TRY(run_engine(h, eng, c, s));
+  if (mean) DP_TRY(hyp_mean_launch(c.out, x_out, n_pose, n_hyp, row_floats, s));
   if (targets != nullptr) DP_TRY(metrics_launch(x_out, d.c_out, d.c_out - 3, targets, n_pose, d.n_pts, sums, nullptr, s));
   return DP_OK;
 }
@@ -621,17 +626,6 @@ const char* dp_last_error(void) { return g_err.c_str(); }
 const char* dp_version(void) { return "diffpose_b200 0.2 (sm_100a)"; }
 int dp_device(dp_handle h) { return h ? h->device : DP_ERR_INVALID; }
 
-void dp_destroy(dp_handle h) {
-  if (!h) return;
-  tcx_free(h);
-  tc2_free(h);
-  if (h->blob) cudaFree(h->blob);
-  if (h->dw) cudaFree(h->dw);
-  if (h->temb) cudaFree(h->temb);
-  if (h->steps) cudaFree(h->steps);
-  if (h->hyp_scratch) cudaFree(h->hyp_scratch);
-  if (h->lift_scratch) cudaFree(h->lift_scratch);
-  delete h;
-}
+void dp_destroy(dp_handle h) { delete h; }
 
 }  // extern "C"

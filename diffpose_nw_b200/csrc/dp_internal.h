@@ -76,8 +76,66 @@ struct StepsArg {
   dp_step s[kMaxInlineSteps];
 };
 
-struct TcxPack;  // defined in dp_tcx.cu
-struct Tc2Pack;  // defined in dp_tc2.cu
+// A grow-only device allocation that frees itself.  reserve() keeps the block when it is large enough; otherwise it frees
+// it, contents and all, before allocating the new one (at least 4 KB).  If cudaMalloc fails the buffer is left empty, so
+// the next reserve() allocates again instead of handing out a freed pointer.
+class DevBuf {
+ public:
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { if (p_) cudaFree(p_); }
+  template <class T>
+  T* get() const { return static_cast<T*>(p_); }
+  int reserve(size_t bytes) {
+    if (p_ && bytes_ >= bytes) return DP_OK;
+    if (p_) cudaFree(p_);
+    p_ = nullptr; bytes_ = 0;
+    if (bytes < 4096) bytes = 4096;
+    void* p = nullptr;
+    DP_CUDA(cudaMalloc(&p, bytes));
+    p_ = p; bytes_ = bytes;
+    return DP_OK;
+  }
+
+ private:
+  void* p_ = nullptr;
+  size_t bytes_ = 0;
+};
+
+// One engine launch: a sampler call, or one chunk of a forward call (forward_only).  dp_api.cu decides which engine runs
+// and which tails it fuses, and sets only the fields that engine implements; the rest keep these defaults.
+struct EngineCall {
+  const float* x_in = nullptr;
+  int x_is_repeated = 0;         // 1: x_in holds all n_pose * n_hyp rows; 0: one row per pose, read for every hypothesis
+  float* out = nullptr;
+  long n_pose = 0;
+  int n_hyp = 1;
+  int n_steps = 1;
+  const dp_step* steps_dev = nullptr;   // the handle's step table when n_steps > kMaxInlineSteps, else NULL
+  const StepsArg* inl = nullptr;        // the step scalars otherwise (zero for a forward call)
+  const float* noise = nullptr;
+  const unsigned char* mask = nullptr;
+  bool forward_only = false;
+  // fused by tcg only
+  bool mean_over_hyp = false;    // out is [n_pose, n_pts, c], the mean over each pose's hypotheses
+  const float* gt = nullptr;     // fused evaluation tail, see dp_sample_eval
+  double* sums = nullptr;
+  // fused by tcx only
+  bool emit_uvxyz = false;       // forward of GCNpose: out is [n, n_pts, c_in + c_out] = [uv | xyz - xyz_root] (dp_lift)
+};
+
+// Opts `Kernel` into `bytes` of dynamic shared memory once per device (function attributes are per device).
+template <auto Kernel>
+int smem_opt_in(int device, int bytes) {
+  static bool done[64] = {};
+  bool& d = done[device & 63];
+  if (!d) {
+    DP_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    d = true;
+  }
+  return DP_OK;
+}
 
 }  // namespace dp
 
@@ -90,63 +148,49 @@ struct dp_model {
   bool packed = false;
   long n_params = 0;
 
-  float* blob = nullptr;          // packed fp32 weights
+  dp::DevBuf blob;                // packed fp32 weights
   size_t blob_floats = 0;
   dp::Weights hw{};               // host copy of the device pointers
-  dp::Weights* dw = nullptr;      // the same struct in device memory
+  dp::DevBuf dw;                  // the same struct in device memory
 
-  float* temb = nullptr;          // [n_rows][n_layer][hid] time-embedding table scratch
-  size_t temb_cap = 0;            // capacity in floats
+  dp::DevBuf temb;                // [n_rows][n_layer][hid] fp32 time-embedding table scratch
   std::vector<float> temb_t;      // timesteps the table currently holds (sampler schedule cache; empty = invalid)
-  dp_step* steps = nullptr;       // device copy of the step scalars, only used when n_steps > kMaxInlineSteps
-  size_t steps_cap = 0;
+  dp::DevBuf steps;               // device copy of the step scalars, only used when n_steps > kMaxInlineSteps
   std::vector<dp_step> steps_host;   // what `steps` currently holds (a long schedule is uploaded once, not per call)
-  float* hyp_scratch = nullptr;   // [n_pose*n_hyp, n_pts, c]: hypothesis mean of the engines that do not fuse it (fp32, tcx)
-  size_t hyp_cap = 0;
-  float* lift_scratch = nullptr;  // [n, n_pts, c_out]: dp_lift on the engines that do not fuse the glue
-  size_t lift_cap = 0;
+  dp::DevBuf hyp_scratch;         // [n_pose*n_hyp, n_pts, c] fp32: hypothesis mean of the engines that do not fuse it (fp32, tcx)
+  dp::DevBuf lift_scratch;        // [n, n_pts, c_out] fp32: dp_lift on the engines that do not fuse the glue
 
-  dp::TcxPack* tcx = nullptr;     // split-precision tensor-core engine state (hi/lo fp16 weight blocks, packed lazily)
-  dp::Tc2Pack* tc2 = nullptr;     // default tensor-core engine state
+  dp::DevBuf tc2_blocks;          // default tensor-core engine: fp16 weight blocks, io blocks, per-layer parameters (dp_pack)
+  dp::DevBuf tc2_tau;             //   and the GC2 bias blocks of the cached sampler schedule
+  dp::DevBuf tcx_blocks;          // split-precision engine: hi/lo fp16 weight blocks, packed lazily
+  bool tcx_packed = false;        //   from the current fp32 blob (cleared by dp_pack, set on the engine's next use)
   long last_launch[6] = {0, 0, 0, 0, 0, 0};
   long long* trace = nullptr;     // caller-owned device buffer for the hand-over timestamps (dp_set_trace)
   int trace_cap = 0;
 };
 
 namespace dp {
+// dp_last_launch_info: grid, block, dynamic shared memory, poses per tile, engine, tiles of the last engine launch
+inline void record_launch(dp_model* m, long grid, long threads, long smem, long tile_poses, int engine, long n_tiles) {
+  long* l = m->last_launch;
+  l[0] = grid; l[1] = threads; l[2] = smem; l[3] = tile_poses; l[4] = engine; l[5] = n_tiles;
+}
+// The engines: each fills its kernel arguments from the call and launches.  A sampler call reads m->temb as the table of
+// its schedule, a forward call as the per-sample table of its chunk (simt_temb).
+int simt_run(dp_model* m, const EngineCall& c, cudaStream_t s);
+int tcx_run(dp_model* m, const EngineCall& c, cudaStream_t s);
+int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s);
 // dp_simt.cu
 // time-embedding table [n_t][n_layer][hid]: t comes from t_dev[i*t_stride] or, when t_dev is NULL, from inl.s[i].t
 int simt_temb(dp_model* m, const float* t_dev, int t_stride, const StepsArg* inl, long n_t, cudaStream_t s);
-int simt_forward(dp_model* m, const float* x, const float* t, const unsigned char* mask, float* out, long n,
-                 cudaStream_t s);
-int simt_sample(dp_model* m, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                const dp_step* steps_dev, const StepsArg* inl, int n_steps, const float* noise,
-                const unsigned char* mask, cudaStream_t s);
-int ensure_capacity(float** p, size_t* cap, size_t need_floats);
-// dp_tcx.cu
-bool tcx_supported(const Dims& d);
-void tcx_invalidate(dp_model* m);   // after dp_pack: the split weights are rebuilt on the engine's next use
-void tcx_free(dp_model* m);
-int tcx_sample(dp_model* m, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-               const dp_step* steps_dev, const StepsArg* inl, int n_steps, const float* noise,
-               const unsigned char* mask, cudaStream_t s);
-int tcx_forward(dp_model* m, const float* x, const float* t, const unsigned char* mask, float* out, long n, int emit_uvxyz, cudaStream_t s);
 // dp_lab.cu
 int tc_lab(const void* image_dev, int image_bytes, const dp_mma_op* ops_host, int n_ops, float* out_dev, int ncols,
            const void* tmem_image_dev, int tmem_col0, int tmem_ncols, cudaStream_t s);
 void tc_lab_cycles(long long* out2);
 // dp_tc2.cu
-bool tc2_supported(const Dims& d);
-int tc2_forward(dp_model* m, const float* x, const float* t, const unsigned char* mask, float* out, long n, cudaStream_t s);
 int tc2_pack(dp_model* m, cudaStream_t s);
 // after simt_temb filled m->temb for a sampler schedule: the same embeddings as GC2 bias blocks of the tcg engine
 int tc2_tau(dp_model* m, int n_steps, cudaStream_t s);
-void tc2_free(dp_model* m);
-// mean_over_hyp: x_out is [n_pose, n_pts, c], the hypothesis mean fused into the kernel's final store
-// gt / sums (optional): fused evaluation tail, see dp_sample_eval
-int tc2_sample(dp_model* m, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-               const dp_step* steps_dev, const StepsArg* inl, int n_steps, const float* noise,
-               const unsigned char* mask, int mean_over_hyp, const float* gt, double* sums, cudaStream_t s);
 // dp_metrics.cu
 int metrics_launch(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
                    double* sums, float* per_pose, cudaStream_t s);

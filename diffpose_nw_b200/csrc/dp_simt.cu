@@ -1,7 +1,7 @@
 // fp32 engine: one persistent kernel runs the whole DDIM loop (every step, every layer) for a tile of
 // pose-hypotheses per CTA with all activations resident in shared memory.  Every contraction is an fp32
-// FMA chain, so this engine is the on-device bit-level reference for the tensor-core engine and serves the
-// configurations that engine does not cover (hid_dim != 96, per-sample timesteps, GCNpose).
+// FMA chain, so this engine is the on-device bit-level reference for the tensor-core engines and the only one for
+// the configurations they do not cover (hid_dim != 96, n_head != 4, coordinates wider than 5).
 //
 // Reference semantics restated here (paths relative to the reference repository):
 //   GCNdiff.forward            models/gcndiff.py:101-113      GCNpose.forward   models/gcnpose.py:101-113
@@ -431,19 +431,13 @@ size_t simt_smem_bytes(int H, int P) {
 template <int CL>
 int launch_simt(dp_model* m, const SimtArgs& a, const StepsArg& inl, cudaStream_t s) {
   const size_t smem = simt_smem_bytes(32 * CL, a.P);
-  static bool configured[64] = {};          // function attributes are per device
-  bool& done = configured[m->device & 63];
-  if (!done) {
-    DP_CUDA(cudaFuncSetAttribute(simt_kernel<CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    done = true;
-  }
+  DP_TRY(smem_opt_in<simt_kernel<CL>>(m->device, 227 * 1024));
   const long n_tiles = (a.n_rows + a.P - 1) / a.P;
   const int grid = (int)min((long)m->sm_count, n_tiles);
   simt_kernel<CL><<<grid, kThreads, smem, s>>>(a, inl);
   count_launch();
   DP_CUDA(cudaGetLastError());
-  m->last_launch[0] = grid; m->last_launch[1] = kThreads; m->last_launch[2] = (long)smem;
-  m->last_launch[3] = a.P; m->last_launch[4] = DP_ENGINE_FP32; m->last_launch[5] = n_tiles;
+  record_launch(m, grid, kThreads, (long)smem, a.P, DP_ENGINE_FP32, n_tiles);
   return DP_OK;
 }
 
@@ -472,15 +466,15 @@ int pick_tile(const dp_model* m, long n_rows) {
 int simt_temb(dp_model* m, const float* t_dev, int t_stride, const StepsArg* inl, long n_t, cudaStream_t s) {
   if (!m->d.has_temb || n_t == 0) return DP_OK;
   const Dims& d = m->d;
-  int rc = ensure_capacity(&m->temb, &m->temb_cap, (size_t)n_t * d.n_layer * d.hid);
-  if (rc != DP_OK) return rc;
+  DP_TRY(m->temb.reserve((size_t)n_t * d.n_layer * d.hid * sizeof(float)));
+  float* temb = m->temb.get<float>();
   StepsArg dummy{};
   const int H = d.hid;
   if (n_t >= 64) {
     constexpr int kTB = 12;
     const size_t smem = (size_t)kTB * (H + 8 * H) * sizeof(float);      // 41.5 KB at hid = 96 (48 KB without opt-in: hid <= 111)
     if (smem <= 48 * 1024) {
-      temb_kernel<kTB><<<(unsigned)((n_t + kTB - 1) / kTB), 4 * H, smem, s>>>(m->dw, d, t_dev, t_stride, inl ? *inl : dummy, n_t, m->temb);
+      temb_kernel<kTB><<<(unsigned)((n_t + kTB - 1) / kTB), 4 * H, smem, s>>>(m->dw.get<Weights>(), d, t_dev, t_stride, inl ? *inl : dummy, n_t, temb);
       count_launch();
       DP_CUDA(cudaGetLastError());
       return DP_OK;
@@ -489,44 +483,19 @@ int simt_temb(dp_model* m, const float* t_dev, int t_stride, const StepsArg* inl
   constexpr int kTB = 4;
   const size_t smem = (size_t)kTB * (H + 8 * H) * sizeof(float);
   const long grid = (n_t + kTB - 1) / kTB;
-  temb_kernel<kTB><<<(unsigned)grid, 4 * H, smem, s>>>(m->dw, d, t_dev, t_stride, inl ? *inl : dummy, n_t, m->temb);
+  temb_kernel<kTB><<<(unsigned)grid, 4 * H, smem, s>>>(m->dw.get<Weights>(), d, t_dev, t_stride, inl ? *inl : dummy, n_t, temb);
   count_launch();
   DP_CUDA(cudaGetLastError());
   return DP_OK;
 }
 
-int simt_sample(dp_model* m, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                const dp_step* steps_dev, const StepsArg* inl, int n_steps, const float* noise,
-                const unsigned char* mask, cudaStream_t s) {
+int simt_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   SimtArgs a{};
-  a.w = m->dw; a.d = m->d; a.x_in = x_in; a.x_is_repeated = x_is_repeated; a.out = x_out;
-  a.n_rows = n_pose * n_hyp; a.n_pose = n_pose; a.n_steps = n_steps; a.forward_only = 0;
-  a.temb = m->temb; a.noise = noise; a.mask = mask; a.steps_dev = steps_dev;
+  a.w = m->dw.get<Weights>(); a.d = m->d; a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
+  a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_steps = c.n_steps; a.forward_only = c.forward_only;
+  a.temb = m->temb.get<float>(); a.noise = c.noise; a.mask = c.mask; a.steps_dev = c.steps_dev;
   a.P = pick_tile(m, a.n_rows);
-  return dispatch_simt(m, a, *inl, s);
-}
-
-int simt_forward(dp_model* m, const float* x, const float* t, const unsigned char* mask, float* out, long n,
-                 cudaStream_t s) {
-  const Dims& d = m->d;
-  const long chunk = 1L << 16;  // bounds the per-sample embedding table (chunk * n_layer * hid floats)
-  StepsArg none{};
-  for (long o = 0; o < n; o += chunk) {
-    const long nn = (n - o < chunk) ? (n - o) : chunk;
-    if (d.has_temb) {
-      int rc = simt_temb(m, t + o, 1, nullptr, nn, s);
-      if (rc != DP_OK) return rc;
-    }
-    SimtArgs a{};
-    a.w = m->dw; a.d = d; a.x_in = x + (size_t)o * d.n_pts * d.c_in; a.x_is_repeated = 1;
-    a.out = out + (size_t)o * d.n_pts * d.c_out;
-    a.n_rows = nn; a.n_pose = nn; a.n_steps = 1; a.forward_only = 1;
-    a.temb = m->temb; a.noise = nullptr; a.mask = mask; a.steps_dev = nullptr;
-    a.P = pick_tile(m, nn);
-    int rc = dispatch_simt(m, a, none, s);
-    if (rc != DP_OK) return rc;
-  }
-  return DP_OK;
+  return dispatch_simt(m, a, *c.inl, s);
 }
 
 }  // namespace dp

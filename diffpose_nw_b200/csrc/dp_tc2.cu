@@ -35,35 +35,25 @@
 #include "dp_internal.h"
 #include "dp_sm100.cuh"
 #include "dp_metrics_dev.cuh"
+#include "dp_tc_layout.cuh"
 
 namespace dp {
 
 namespace {
 
 using namespace sm100;
+using namespace tc;
 
-constexpr int NP = 17;
-constexpr int TM = 128;              // tile rows = UMMA M
-constexpr int TP = 7;                // poses per tile
 constexpr int PS = 18;               // tile rows per pose: 17 joints + 1 pad row, so every pose starts on an even row and the
                                      // rows of a warp (32) always begin 0, 14, 10 or 6 rows into a pose -> one softmax code path
 constexpr int TR = TP * PS;          // 126 rows carry poses
-constexpr int H = 96;
 constexpr int NSTAGE = 4;
-constexpr int WK = 112;              // weight block K extent: 96 weights + 16 (bias slab; k=96 hi, k=97 lo)
-constexpr int W_LBO = 12 * 128;      // bytes between K-adjacent 8x8 core matrices of a weight block
-constexpr int W_SBO = 128;           // bytes between N-adjacent core matrices
-constexpr int WBLK_BYTES = (WK / 8) * W_LBO;        // 21504
-constexpr int A_LBO = 16 * 128 + 16; // 2064: chunk column stride (+16 B skews consecutive chunk columns across banks)
-constexpr int ABLK_BYTES = 12 * A_LBO;              // 24768
-constexpr int ONES_BYTES = 2 * A_LBO;               // 4128
 constexpr int T_ROWS = 256;                         // tall graph operand: rows 128..144 hold the matrix
 constexpr int T_LBO = T_ROWS * 16 + 16;             // 4112
 constexpr int TALL_BYTES = 2 * T_LBO;               // 8224: K = joints 0..15 (joint 16 goes through the side operands below)
 constexpr int SIDE_LBO = 256;                       // side buffer [16 rows x 96 ch]: 8-channel groups 256 B apart
 constexpr int SIDE_BYTES = 12 * SIDE_LBO;           // 3072
 constexpr int A16_BYTES = A_LBO;                    // joint-16 operand of a graph matrix: one chunk column [128 rows x 8]
-constexpr int BLOCKS_PER_LAYER = 14;
 constexpr int OUT_LBO = 256;                        // output-convolution block: N = 16 rows, K-adjacent core matrices 256 B apart
 constexpr int LP_LHAT_BYTES = 4 * NP * 16;          // per-layer parameters: L^ as fp16 [4 chunk columns][17 rows][8]
 constexpr int LP_JS_BYTES = PS * 16;                //   + the joint slab rows (1, 1, r_hi, r_hi, r_lo, 0, 0, 0), r = row sums of L^
@@ -75,7 +65,6 @@ constexpr int kComputeThreads = 256;
 constexpr int kProducerWarp = 8, kIssuerWarp = 9;
 constexpr int kThreads = kComputeThreads + 64;
 constexpr int NEV = 4;               // depth of the two hand-over rings ("operands ready", "accumulator ready")
-constexpr int TMEM_COLS = 512;
 constexpr uint32_t COL_X = 0;        // residual stream
 constexpr uint32_t COL_ACC = 96;     // GEMM accumulators (up to 288 columns)
 constexpr uint32_t COL_S0 = 96;      // attention: scores of the even head of a pair [128 x 128]; its probabilities
@@ -86,7 +75,6 @@ constexpr uint32_t COL_TA0 = 448;    // fp16 A operands kept in tensor memory (4
 constexpr uint32_t COL_TA1 = 384;    //   only ever feed a GEMM as A skip shared memory (its bandwidth bounds the epilogues)
 
 // shared memory map (bytes)
-constexpr int al16(int x) { return (x + 15) / 16 * 16; }
 constexpr int OFF_A = 0;                                   // three fp16 operand blocks; fp32 scratch [128][17] aliases block 0
 constexpr int OFF_SIDE = OFF_A + 3 * ABLK_BYTES;           // per operand block: the joint-16 rows of the 7 poses, compacted (rows 7..15 zero)
 constexpr int OFF_A16 = OFF_SIDE + 3 * SIDE_BYTES;         // per graph matrix (T1, T2, L^): element (18p+i, p) = G[i][16]
@@ -1167,36 +1155,14 @@ __global__ void tc2_tau_kernel(uint8_t* __restrict__ dst, const float* __restric
 
 }  // namespace
 
-struct Tc2Pack {
-  uint8_t* blocks = nullptr;   // [n_layer][14][WBLK_BYTES] then [2][WBLK_BYTES] (io blocks) then [n_layer][LP_BYTES]
-  size_t bytes = 0;
-  uint8_t* tau = nullptr;      // [n_steps][n_layer][LP_TAU_BYTES] of the cached schedule
-  size_t tau_bytes = 0;
-};
-
 // m->temb holds the [n_steps][n_layer][96] table of the schedule (simt_temb): derive the GC2 bias blocks from it
 int tc2_tau(dp_model* m, int n_steps, cudaStream_t s) {
-  if (!m->tc2 || !m->d.has_temb) return DP_OK;
-  const size_t need = (size_t)n_steps * m->d.n_layer * LP_TAU_BYTES;
-  if (m->tc2->tau_bytes < need) {
-    if (m->tc2->tau) cudaFree(m->tc2->tau);
-    m->tc2->tau = nullptr; m->tc2->tau_bytes = 0;
-    DP_CUDA(cudaMalloc(reinterpret_cast<void**>(&m->tc2->tau), need));
-    m->tc2->tau_bytes = need;
-  }
-  tc2_tau_kernel<<<n_steps * m->d.n_layer, H, 0, s>>>(m->tc2->tau, m->temb, m->dw, m->d.n_layer);
+  if (!m->d.has_temb) return DP_OK;
+  DP_TRY(m->tc2_tau.reserve((size_t)n_steps * m->d.n_layer * LP_TAU_BYTES));
+  tc2_tau_kernel<<<n_steps * m->d.n_layer, H, 0, s>>>(m->tc2_tau.get<uint8_t>(), m->temb.get<float>(), m->dw.get<Weights>(), m->d.n_layer);
   count_launch();
   DP_CUDA(cudaGetLastError());
   return DP_OK;
-}
-
-void tc2_free(dp_model* m) {
-  if (m->tc2) {
-    if (m->tc2->blocks) cudaFree(m->tc2->blocks);
-    if (m->tc2->tau) cudaFree(m->tc2->tau);
-    delete m->tc2;
-    m->tc2 = nullptr;
-  }
 }
 
 // `bias` points at the first of the 96 bias values of this block (or NULL)
@@ -1210,19 +1176,15 @@ static int pack_block(uint8_t* dst, const float* W, int ldw, int k0, int n0, con
 
 int tc2_pack(dp_model* m, cudaStream_t s) {
   const Dims& d = m->d;
-  if (!m->tc2) m->tc2 = new Tc2Pack();
+  // [n_layer][14][WBLK_BYTES] weight blocks, then [2][WBLK_BYTES] io blocks, then [n_layer][LP_BYTES] per-layer parameters
   const size_t wbytes = (size_t)d.n_layer * BLOCKS_PER_LAYER * WBLK_BYTES;
   const size_t need = wbytes + 2 * WBLK_BYTES + (size_t)d.n_layer * LP_BYTES;
-  if (m->tc2->bytes < need) {
-    if (m->tc2->blocks) cudaFree(m->tc2->blocks);
-    m->tc2->blocks = nullptr; m->tc2->bytes = 0;
-    DP_CUDA(cudaMalloc(reinterpret_cast<void**>(&m->tc2->blocks), need));
-    m->tc2->bytes = need;
-  }
-  DP_CUDA(cudaMemsetAsync(m->tc2->blocks, 0, need, s));
+  DP_TRY(m->tc2_blocks.reserve(need));
+  uint8_t* blocks = m->tc2_blocks.get<uint8_t>();
+  DP_CUDA(cudaMemsetAsync(blocks, 0, need, s));
   for (int l = 0; l < d.n_layer; ++l) {
     const LayerW& L = m->hw.layer[l];
-    uint8_t* b = m->tc2->blocks + (size_t)l * BLOCKS_PER_LAYER * WBLK_BYTES;
+    uint8_t* b = blocks + (size_t)l * BLOCKS_PER_LAYER * WBLK_BYTES;
     int i = 0;
     // consumption order of the issuer: q, k, v, o, fc1 (two output halves), fc2 (two input halves; the first carries b2,
     // which the kernel adds to the residual stream), cheb1 x3, cheb2 x3
@@ -1232,35 +1194,30 @@ int tc2_pack(dp_model* m, cudaStream_t s) {
     for (int part = 0; part < 2; ++part) DP_TRY(pack_block(b + (size_t)(i++) * WBLK_BYTES, L.w2, H, part * H, 0, part == 0 ? L.b2 : nullptr, s));
     for (int part = 0; part < 3; ++part) DP_TRY(pack_block(b + (size_t)(i++) * WBLK_BYTES, L.wc1, H, part * H, 0, part == 0 ? L.bc1 : nullptr, s));
     for (int part = 0; part < 3; ++part) DP_TRY(pack_block(b + (size_t)(i++) * WBLK_BYTES, L.wc2, H, part * H, 0, part == 0 ? L.bc2 : nullptr, s));
-    tc2_pack_lparams_kernel<<<1, 128, 0, s>>>(m->tc2->blocks + wbytes + 2 * WBLK_BYTES + (size_t)l * LP_BYTES, L.lhat);
+    tc2_pack_lparams_kernel<<<1, 128, 0, s>>>(blocks + wbytes + 2 * WBLK_BYTES + (size_t)l * LP_BYTES, L.lhat);
     count_launch();
     DP_CUDA(cudaGetLastError());
   }
-  tc2_pack_io_kernel<<<18, 256, 0, s>>>(m->tc2->blocks + wbytes, m->hw.win, m->hw.bin, m->hw.wout, d.c_in, d.c_out);
+  tc2_pack_io_kernel<<<18, 256, 0, s>>>(blocks + wbytes, m->hw.win, m->hw.bin, m->hw.wout, d.c_in, d.c_out);
   count_launch();
   DP_CUDA(cudaGetLastError());
   return DP_OK;
 }
 
-bool tc2_supported(const Dims& d) {
-  return d.hid == 96 && d.n_head == 4 && d.n_pts == 17 && d.c_in >= 1 && d.c_in <= 5 && d.c_out >= 1 && d.c_out <= 5;
-}
-
-static int tc2_launch(dp_model* m, Tc2Args& a, const StepsArg* inl, cudaStream_t s) {
-  if (!m->tc2 || !m->tc2->blocks) { set_error("tensor-core engine: weights are not packed"); return DP_ERR_STATE; }
-  static bool configured[64] = {};          // function attributes are per device
-  bool& done = configured[m->device & 63];
-  if (!done) {
-    DP_CUDA(cudaFuncSetAttribute(tc2_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    DP_CUDA(cudaFuncSetAttribute(tc2_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    DP_CUDA(cudaFuncSetAttribute(tc2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    done = true;
-  }
+int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
+  const uint8_t* blocks = m->tc2_blocks.get<uint8_t>();
+  if (!blocks) { set_error("tensor-core engine: weights are not packed"); return DP_ERR_STATE; }
+  DP_TRY((smem_opt_in<tc2_kernel<false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<true, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true>>(m->device, SMEM_BYTES)));
   const size_t wbytes = (size_t)m->d.n_layer * BLOCKS_PER_LAYER * WBLK_BYTES;
-  a.w = m->dw; a.wpack = m->tc2->blocks; a.ioblocks = m->tc2->blocks + wbytes; a.lparams = m->tc2->blocks + wbytes + 2 * WBLK_BYTES;
-  a.n_layer = m->d.n_layer; a.c_in = m->d.c_in; a.c_out = m->d.c_out; a.has_temb = m->d.has_temb;
-  a.temb = m->temb; a.tau = m->tc2->tau;
-  a.trace = m->trace; a.trace_cap = m->trace_cap;
+  Tc2Args a{};
+  a.w = m->dw.get<Weights>(); a.wpack = blocks; a.ioblocks = blocks + wbytes; a.lparams = blocks + wbytes + 2 * WBLK_BYTES;
+  a.n_layer = m->d.n_layer; a.c_in = m->d.c_in; a.c_out = m->d.c_out; a.forward_only = c.forward_only; a.has_temb = m->d.has_temb;
+  a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
+  a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_hyp = c.n_hyp; a.mean_over_hyp = c.mean_over_hyp; a.n_steps = c.n_steps;
+  a.temb = m->temb.get<float>(); a.tau = m->tc2_tau.get<uint8_t>(); a.noise = c.noise; a.mask = c.mask; a.steps_dev = c.steps_dev;
+  a.gt = c.gt; a.sums = c.sums; a.trace = m->trace; a.trace_cap = m->trace_cap;
   const long n_tiles = (a.n_rows + TP - 1) / TP;
   if (n_tiles > 0x7fffffffL) { set_error("tensor-core engine: more than 2^31 tiles of 7 poses in one call"); return DP_ERR_INVALID; }
   int grid = (int)(n_tiles < m->sm_count ? n_tiles : m->sm_count);
@@ -1271,40 +1228,11 @@ static int tc2_launch(dp_model* m, Tc2Args& a, const StepsArg* inl, cudaStream_t
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true>, a, *inl));
-  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false>, a, *inl));
-  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false>, a, *inl));
+  if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true>, a, *c.inl));
+  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false>, a, *c.inl));
+  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false>, a, *c.inl));
   count_launch();
-  m->last_launch[0] = grid; m->last_launch[1] = kThreads; m->last_launch[2] = SMEM_BYTES;
-  m->last_launch[3] = TP; m->last_launch[4] = DP_ENGINE_TCG; m->last_launch[5] = n_tiles;
-  return DP_OK;
-}
-
-int tc2_sample(dp_model* m, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-               const dp_step* steps_dev, const StepsArg* inl, int n_steps, const float* noise,
-               const unsigned char* mask, int mean_over_hyp, const float* gt, double* sums, cudaStream_t s) {
-  Tc2Args a{};
-  a.gt = gt; a.sums = sums;
-  a.x_in = x_in; a.x_is_repeated = x_is_repeated; a.out = x_out;
-  a.n_rows = n_pose * n_hyp; a.n_pose = n_pose; a.n_hyp = n_hyp; a.mean_over_hyp = (mean_over_hyp && n_hyp > 1) ? 1 : 0;
-  a.n_steps = n_steps; a.noise = noise; a.mask = mask;
-  a.steps_dev = steps_dev; a.forward_only = 0;
-  return tc2_launch(m, a, inl, s);
-}
-
-// GCNdiff.forward / GCNpose.forward (models/gcndiff.py:101-113, models/gcnpose.py:101-113): one pass, per-sample timesteps
-int tc2_forward(dp_model* m, const float* x, const float* t, const unsigned char* mask, float* out, long n, cudaStream_t s) {
-  const Dims& d = m->d;
-  const long chunk = 1L << 16;  // bounds the per-sample embedding table (chunk * n_layer * hid floats)
-  StepsArg none{};
-  for (long o = 0; o < n; o += chunk) {
-    const long nn = (n - o < chunk) ? (n - o) : chunk;
-    if (d.has_temb) DP_TRY(simt_temb(m, t + o, 1, nullptr, nn, s));
-    Tc2Args a{};
-    a.x_in = x + (size_t)o * d.n_pts * d.c_in; a.x_is_repeated = 1; a.out = out + (size_t)o * d.n_pts * d.c_out;
-    a.n_rows = nn; a.n_pose = nn; a.n_hyp = 1; a.n_steps = 1; a.noise = nullptr; a.mask = mask; a.steps_dev = nullptr; a.forward_only = 1;
-    DP_TRY(tc2_launch(m, a, &none, s));
-  }
+  record_launch(m, grid, kThreads, SMEM_BYTES, TP, DP_ENGINE_TCG, n_tiles);
   return DP_OK;
 }
 

@@ -25,41 +25,29 @@
 #include <cmath>
 #include "dp_internal.h"
 #include "dp_sm100.cuh"
+#include "dp_tc_layout.cuh"
 
 namespace dp {
 
 namespace {
 
 using namespace sm100;
+using namespace tc;
 
-constexpr int NP = 17;
-constexpr int TM = 128;              // tile rows = UMMA M
-constexpr int TP = 7;                // poses per tile
 constexpr int TR = TP * NP;          // 119 valid rows (row = pose * 17 + joint)
-constexpr int H = 96;
 constexpr int XLD = 100;             // fp32 row stride (floats): thread-per-row float4 access is conflict free
 constexpr int NSTAGE = 3;
-constexpr int WK = 112;              // weight block K extent: 96 weights + 16 (bias slab; k=96 hi, k=97 lo)
-constexpr int W_LBO = 12 * 128;      // bytes between K-adjacent 8x8 core matrices of a weight block
-constexpr int W_SBO = 128;           // bytes between N-adjacent core matrices
-constexpr int WBLK_BYTES = (WK / 8) * W_LBO;        // 21504
-constexpr int A_LBO = 16 * 128 + 16; // 2064: +16 B skews consecutive K chunks across banks
 constexpr int A_SBO = 128;
-constexpr int ABLK_BYTES = 12 * A_LBO;              // 24768
 constexpr int PAIR_BYTES = 2 * ABLK_BYTES;          // an operand = (hi block, lo block)
-constexpr int ONES_BYTES = 2 * A_LBO;               // 4128
-constexpr int BLOCKS_PER_LAYER = 14;                // each one a (hi, lo) pair of ring entries
 constexpr int NNB = NP;              // neighbour-list capacity: any graph.  The lists are padded to the longest row of the graph in
                                      // use (9 = the largest 2-hop neighbourhood of the H36M tree, support of T2 = 2L^2 - I)
 constexpr int kComputeThreads = 512;   // 16 compute warps: the fp32 shared-memory phases are latency bound, so the kernel wants warps
 constexpr int kThreads = kComputeThreads + 32;
 constexpr int kParts = kComputeThreads / TM;          // 4 threads per tile row: 24 of the 96 channels each
 constexpr int PC = H / kParts;                        // 24
-constexpr int TMEM_COLS = 512;
 constexpr int XS = 8;                // x_t / eps row stride (floats)
 
-// shared memory map (bytes)
-constexpr int al16(int x) { return (x + 15) / 16 * 16; }
+// shared memory map (bytes); each of the BLOCKS_PER_LAYER weight blocks is a (hi, lo) pair of ring entries
 constexpr int al128(int x) { return (x + 127) / 128 * 128; }
 constexpr int OFF_X = 0;                                   // fp32 residual stream [119][100]
 constexpr int OFF_P0 = al128(OFF_X + TR * XLD * 4);        // operand pair 0 (hi, lo); aliased by the fp32 buffer S0 [119][100]
@@ -801,28 +789,6 @@ __global__ void tcx_pack_block_kernel(uint8_t* __restrict__ dst, const float* __
 
 }  // namespace
 
-struct TcxPack {
-  uint8_t* blocks = nullptr;   // [n_layer][14][2][WBLK_BYTES]
-  size_t bytes = 0;
-  bool valid = false;          // packed from the current fp32 blob (packing is lazy: first use after dp_pack)
-};
-
-bool tcx_supported(const Dims& d) {
-  return d.hid == 96 && d.n_head == 4 && d.n_pts == 17 && d.c_in >= 1 && d.c_in <= 5 && d.c_out >= 1 && d.c_out <= 5;
-}
-
-void tcx_free(dp_model* m) {
-  if (m->tcx) {
-    if (m->tcx->blocks) cudaFree(m->tcx->blocks);
-    delete m->tcx;
-    m->tcx = nullptr;
-  }
-}
-
-void tcx_invalidate(dp_model* m) {
-  if (m->tcx) m->tcx->valid = false;
-}
-
 static int pack_block(uint8_t* dst, const float* W, int ldw, int k0, int n0, const float* bias, cudaStream_t s) {
   tcx_pack_block_kernel<<<12, 256, 0, s>>>(dst, W, ldw, k0, n0, bias);
   count_launch();
@@ -832,19 +798,12 @@ static int pack_block(uint8_t* dst, const float* W, int ldw, int k0, int n0, con
 
 // Lazy: the split weights (3 MB) are built the first time this engine runs after a dp_pack, not on every weight load.
 static int tcx_ensure_packed(dp_model* m, cudaStream_t s) {
+  if (m->tcx_packed) return DP_OK;
   const Dims& d = m->d;
-  if (!m->tcx) m->tcx = new TcxPack();
-  if (m->tcx->valid) return DP_OK;
-  const size_t need = (size_t)d.n_layer * BLOCKS_PER_LAYER * 2 * WBLK_BYTES;
-  if (m->tcx->bytes < need) {
-    if (m->tcx->blocks) cudaFree(m->tcx->blocks);
-    m->tcx->blocks = nullptr; m->tcx->bytes = 0;
-    DP_CUDA(cudaMalloc(reinterpret_cast<void**>(&m->tcx->blocks), need));
-    m->tcx->bytes = need;
-  }
+  DP_TRY(m->tcx_blocks.reserve((size_t)d.n_layer * BLOCKS_PER_LAYER * 2 * WBLK_BYTES));
   for (int l = 0; l < d.n_layer; ++l) {
     const LayerW& L = m->hw.layer[l];
-    uint8_t* b = m->tcx->blocks + (size_t)l * BLOCKS_PER_LAYER * 2 * WBLK_BYTES;
+    uint8_t* b = m->tcx_blocks.get<uint8_t>() + (size_t)l * BLOCKS_PER_LAYER * 2 * WBLK_BYTES;
     int i = 0;
     // consumption order of the kernel: q, k, v, o, fc1 (two output halves), fc2 (two input halves), cheb1 x3, cheb2 x3
     for (int part = 0; part < 3; ++part) DP_TRY(pack_block(b + (size_t)(i++) * 2 * WBLK_BYTES, L.wqkv, 3 * H, 0, part * H, L.bqkv, s));
@@ -854,56 +813,25 @@ static int tcx_ensure_packed(dp_model* m, cudaStream_t s) {
     for (int part = 0; part < 3; ++part) DP_TRY(pack_block(b + (size_t)(i++) * 2 * WBLK_BYTES, L.wc1, H, part * H, 0, part == 0 ? L.bc1 : nullptr, s));
     for (int part = 0; part < 3; ++part) DP_TRY(pack_block(b + (size_t)(i++) * 2 * WBLK_BYTES, L.wc2, H, part * H, 0, part == 0 ? L.bc2 : nullptr, s));
   }
-  m->tcx->valid = true;
+  m->tcx_packed = true;
   return DP_OK;
 }
 
-static int tcx_launch(dp_model* m, TcxArgs& a, const StepsArg* inl, cudaStream_t s) {
+int tcx_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   DP_TRY(tcx_ensure_packed(m, s));
-  static bool configured[64] = {};          // function attributes are per device
-  bool& done = configured[m->device & 63];
-  if (!done) {
-    DP_CUDA(cudaFuncSetAttribute(tcx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    done = true;
-  }
-  a.w = m->dw; a.wpack = m->tcx->blocks; a.n_layer = m->d.n_layer; a.c_in = m->d.c_in; a.c_out = m->d.c_out; a.has_temb = m->d.has_temb;
-  a.temb = m->temb;
+  DP_TRY(smem_opt_in<tcx_kernel>(m->device, SMEM_BYTES));
+  TcxArgs a{};
+  a.w = m->dw.get<Weights>(); a.wpack = m->tcx_blocks.get<uint8_t>(); a.n_layer = m->d.n_layer; a.c_in = m->d.c_in; a.c_out = m->d.c_out;
+  a.forward_only = c.forward_only; a.has_temb = m->d.has_temb; a.emit_uvxyz = c.emit_uvxyz;
+  a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
+  a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_steps = c.n_steps;
+  a.temb = m->temb.get<float>(); a.noise = c.noise; a.mask = c.mask; a.steps_dev = c.steps_dev;
   const long n_tiles = (a.n_rows + TP - 1) / TP;
   const int grid = (int)(n_tiles < m->sm_count ? n_tiles : m->sm_count);
-  tcx_kernel<<<grid, kThreads, SMEM_BYTES, s>>>(a, *inl);
+  tcx_kernel<<<grid, kThreads, SMEM_BYTES, s>>>(a, *c.inl);
   count_launch();
   DP_CUDA(cudaGetLastError());
-  m->last_launch[0] = grid; m->last_launch[1] = kThreads; m->last_launch[2] = SMEM_BYTES;
-  m->last_launch[3] = TP; m->last_launch[4] = DP_ENGINE_TCX; m->last_launch[5] = n_tiles;
-  return DP_OK;
-}
-
-int tcx_sample(dp_model* m, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-               const dp_step* steps_dev, const StepsArg* inl, int n_steps, const float* noise,
-               const unsigned char* mask, cudaStream_t s) {
-  TcxArgs a{};
-  a.x_in = x_in; a.x_is_repeated = x_is_repeated; a.out = x_out;
-  a.n_rows = n_pose * n_hyp; a.n_pose = n_pose; a.n_steps = n_steps; a.noise = noise; a.mask = mask;
-  a.steps_dev = steps_dev; a.forward_only = 0;
-  return tcx_launch(m, a, inl, s);
-}
-
-// GCNdiff.forward / GCNpose.forward (models/gcndiff.py:101-113, models/gcnpose.py:101-113): one pass, per-sample timesteps.
-// emit_uvxyz (GCNpose only): out is [n,17,c_in+c_out] = [uv | xyz - xyz_root] (runners/diffpose_frame.py:337-343).
-int tcx_forward(dp_model* m, const float* x, const float* t, const unsigned char* mask, float* out, long n, int emit_uvxyz, cudaStream_t s) {
-  const Dims& d = m->d;
-  const long chunk = 1L << 16;  // bounds the per-sample embedding table (chunk * n_layer * hid floats)
-  const int wd = emit_uvxyz ? d.c_in + d.c_out : d.c_out;
-  StepsArg none{};
-  for (long o = 0; o < n; o += chunk) {
-    const long nn = (n - o < chunk) ? (n - o) : chunk;
-    if (d.has_temb) DP_TRY(simt_temb(m, t + o, 1, nullptr, nn, s));
-    TcxArgs a{};
-    a.x_in = x + (size_t)o * d.n_pts * d.c_in; a.x_is_repeated = 1; a.out = out + (size_t)o * d.n_pts * wd;
-    a.n_rows = nn; a.n_pose = nn; a.n_steps = 1; a.noise = nullptr; a.mask = mask; a.steps_dev = nullptr; a.forward_only = 1;
-    a.emit_uvxyz = emit_uvxyz;
-    DP_TRY(tcx_launch(m, a, &none, s));
-  }
+  record_launch(m, grid, kThreads, SMEM_BYTES, TP, DP_ENGINE_TCX, n_tiles);
   return DP_OK;
 }
 
