@@ -10,10 +10,10 @@ All arithmetic runs in libdiffpose_b200.so (C ABI: include/diffpose_b200.h).  No
 """
 from .graph import H36M_EDGES, adj_mx_from_edges
 from .model import EMAHelper, FusedGCNdiff, FusedGCNpose
-from .sampler import compute_alpha, ddim_steps, generalized_steps, get_beta_schedule, make_seq, sample
+from .sampler import compute_alpha, ddim_steps, generalized_steps, get_beta_schedule, make_seq, philox_noise, sample
 from .metrics import mpjpe, p_mpjpe, pose_error_sums
 from .pipeline import HostStream, evaluate_shard, lift_and_refine, reduce_metrics, shard_range
 
 __all__ = ["H36M_EDGES", "adj_mx_from_edges", "FusedGCNdiff", "FusedGCNpose", "EMAHelper", "compute_alpha", "ddim_steps",
-           "generalized_steps", "get_beta_schedule", "make_seq", "sample", "mpjpe", "p_mpjpe", "pose_error_sums",
+           "generalized_steps", "get_beta_schedule", "make_seq", "philox_noise", "sample", "mpjpe", "p_mpjpe", "pose_error_sums",
            "HostStream", "evaluate_shard", "lift_and_refine", "reduce_metrics", "shard_range"]

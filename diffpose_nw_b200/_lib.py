@@ -23,6 +23,16 @@ class DpMmaOp(ctypes.Structure):
     _fields_ = [(n, ctypes.c_uint) for n in ("a_off", "a_lbo", "a_sbo", "b_off", "b_lbo", "b_sbo", "idesc", "tmem_col", "accumulate")]
 
 
+class DpNoiseKey(ctypes.Structure):
+    """dp_noise_key: the keyed noise stream of one call (include/diffpose_b200.h)."""
+    _fields_ = [("seed", ctypes.c_ulonglong), ("pose_offset", ctypes.c_long), ("step_offset", ctypes.c_int)]
+
+
+def noise_key(seed, pose_offset=0, step_offset=0):
+    """A DpNoiseKey for a Python int seed (taken modulo 2^64, so negative seeds are valid too)."""
+    return DpNoiseKey(int(seed) & 0xFFFFFFFFFFFFFFFF, int(pose_offset), int(step_offset))
+
+
 # name -> (restype, argtypes); kept in one table so tests can check every header symbol is exported
 _P, _I, _L = ctypes.c_void_p, ctypes.c_int, ctypes.c_long
 SIGNATURES = {
@@ -37,9 +47,13 @@ SIGNATURES = {
     "dp_forward": (_I, [_P, _P, _P, _P, _P, _L, _P]),
     "dp_sample": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, _P, _I, _P]),
     "dp_sample_eval": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, _P, _I, _P, _P, _P]),
+    "dp_sample_keyed": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _P]),
+    "dp_noise_fill": (_I, [ctypes.POINTER(DpNoiseKey), _I, _L, _I, _I, _I, _P, _P]),
     "dp_hstream_create": (_I, [ctypes.POINTER(_P), _P, _L, _I, _I, _I]),
     "dp_hstream_submit": (_I, [_P, _P, _L, ctypes.POINTER(DpStep), _I, _P, _P, _P, _P, ctypes.POINTER(_I)]),
     "dp_hstream_submit_eval": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, _P, _P, _P, _P, ctypes.POINTER(_I)]),
+    "dp_hstream_submit_keyed": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, ctypes.POINTER(DpNoiseKey), _P, _P, _P,
+                                     ctypes.POINTER(_I)]),
     "dp_hstream_wait": (_I, [_P, _I]),
     "dp_hstream_destroy": (None, [_P]),
     "dp_metrics": (_I, [_P, _I, _I, _P, _L, _I, _P, _P, _P]),

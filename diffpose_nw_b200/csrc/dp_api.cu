@@ -386,12 +386,38 @@ int dp_lift(dp_handle h, const float* uv, const unsigned char* mask, float* out_
   return lift_glue_launch(uv, xyz, out_uvxyz, n, d.n_pts, d.c_in, d.c_out, s);
 }
 
+// The keyed stream of a call (dp_philox.cuh); the pose index is one 32-bit counter word.
+static int make_key(const dp_noise_key* k, long n_pose, const char* what, NoiseKey* out) {
+  if (k->pose_offset < 0 || k->step_offset < 0 || n_pose > (1L << 32) || k->pose_offset > (1L << 32) - n_pose) {
+    set_error(std::string(what) + ": the key needs pose_offset >= 0, step_offset >= 0 and pose_offset + n_pose <= 2^32");
+    return DP_ERR_INVALID;
+  }
+  out->k0 = (uint32_t)(k->seed & 0xffffffffull); out->k1 = (uint32_t)(k->seed >> 32);
+  out->pose_offset = (uint32_t)k->pose_offset; out->step_offset = (uint32_t)k->step_offset; out->on = 1;
+  return DP_OK;
+}
+
+// dp_sample, dp_sample_eval, dp_sample_keyed and the host-stream submits: at most one of noise and key is given.
 static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                       const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
+                       const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
                        int mean_over_hyp, const float* targets, double* sums, void* stream) {
   DP_REQUIRE(h && x_in && x_out && steps_host, "dp_sample: NULL argument");
   DP_REQUIRE(n_pose >= 0 && n_hyp >= 1 && n_steps >= 1, "dp_sample: n_pose >= 0, n_hyp >= 1, n_steps >= 1 required");
   DP_REQUIRE(h->d.has_temb, "dp_sample: handle was created with has_temb = 0 (GCNpose has no sampler)");
+  DP_REQUIRE(!(noise && key), "dp_sample: give either a noise tensor or a noise key, not both");
+  if (targets != nullptr) {
+    DP_REQUIRE(sums != nullptr, "dp_sample_eval: NULL argument");
+    DP_REQUIRE(h->d.c_out >= 3, "dp_sample_eval: the model's output needs at least the three xyz coordinates");
+    DP_REQUIRE(n_hyp == 1 || mean_over_hyp, "dp_sample_eval: with n_hyp > 1 the metrics are those of the hypothesis mean (set mean_over_hyp)");
+  }
+  NoiseKey nk{};
+  if (key != nullptr) {
+    DP_TRY(make_key(key, n_pose, "dp_sample_keyed", &nk));
+    // every c1 = 0 (eta = 0): the noise term is skipped, as with a NULL noise pointer
+    bool any = false;
+    for (int i = 0; i < n_steps; ++i) any = any || steps_host[i].c1 != 0.f;
+    nk.on = any ? 1 : 0;
+  }
   if (!h->packed) { set_error("dp_sample: dp_pack has not been called"); return DP_ERR_STATE; }
   if (n_pose == 0) return DP_OK;
   DP_TRY(check_device(h, "dp_sample"));
@@ -430,7 +456,7 @@ static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float*
 
   EngineCall c;
   c.x_in = x_in; c.x_is_repeated = x_is_repeated; c.out = x_out; c.n_pose = n_pose; c.n_hyp = n_hyp;
-  c.n_steps = n_steps; c.steps_dev = steps_dev; c.inl = &inl; c.noise = noise; c.mask = mask;
+  c.n_steps = n_steps; c.steps_dev = steps_dev; c.inl = &inl; c.noise = noise; c.key = nk; c.mask = mask;
   const bool mean = mean_over_hyp && n_hyp > 1;
   const int eng = dp_get_engine(h);
   // default engine: the hypothesis mean -- and, for dp_sample_eval, the MPJPE / P-MPJPE sums -- are fused into the kernel's
@@ -453,16 +479,31 @@ static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float*
 int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
               const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
               int mean_over_hyp, void* stream) {
-  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, mask, mean_over_hyp, nullptr, nullptr, stream);
+  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, nullptr, mask, mean_over_hyp, nullptr, nullptr, stream);
 }
 
 int dp_sample_eval(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
                    const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
                    int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
   DP_REQUIRE(h && targets_xyz && sums, "dp_sample_eval: NULL argument");
-  DP_REQUIRE(h->d.c_out >= 3, "dp_sample_eval: the model's output needs at least the three xyz coordinates");
-  DP_REQUIRE(n_hyp == 1 || mean_over_hyp, "dp_sample_eval: with n_hyp > 1 the metrics are those of the hypothesis mean (set mean_over_hyp)");
-  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, mask, mean_over_hyp, targets_xyz, sums, stream);
+  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, nullptr, mask, mean_over_hyp, targets_xyz, sums, stream);
+}
+
+int dp_sample_keyed(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                    const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask,
+                    int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
+  DP_REQUIRE(key, "dp_sample_keyed: NULL key");
+  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, nullptr, key, mask, mean_over_hyp, targets_xyz, sums, stream);
+}
+
+int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, int n_pts, int c, float* out, void* stream) {
+  DP_REQUIRE(key, "dp_noise_fill: NULL key");
+  DP_REQUIRE(n_steps >= 0 && n_pose >= 0 && n_hyp >= 1 && n_pts >= 1 && c >= 1, "dp_noise_fill: n_steps >= 0, n_pose >= 0, n_hyp >= 1, n_pts >= 1, c >= 1 required");
+  NoiseKey nk{};
+  DP_TRY(make_key(key, n_pose, "dp_noise_fill", &nk));
+  if (n_steps == 0 || n_pose == 0) return DP_OK;
+  DP_REQUIRE(out, "dp_noise_fill: NULL output");
+  return noise_fill_launch(nk, n_steps, n_pose, n_hyp, n_pts * c, out, static_cast<cudaStream_t>(stream));
 }
 
 int dp_metrics(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
@@ -551,7 +592,8 @@ int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, 
 }
 
 static int hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose, const dp_step* steps_host,
-                          int n_steps, const float* noise_dev, const unsigned char* mask_dev, float* out_host, void* stream, int* slot_out) {
+                          int n_steps, const float* noise_dev, const dp_noise_key* key, const unsigned char* mask_dev, float* out_host,
+                          void* stream, int* slot_out) {
   DP_REQUIRE(s && x_host && out_host && steps_host && slot_out, "dp_hstream_submit: NULL argument");
   DP_REQUIRE(n_pose >= 1 && n_pose <= s->max_pose, "dp_hstream_submit: batch exceeds the max_pose this stream was created for");
   DP_TRY(check_device(s->h, "dp_hstream_submit"));
@@ -568,10 +610,8 @@ static int hstream_submit(dp_hstream_t s, const float* x_host, const float* targ
   // the sampler on the caller's stream, once the input is there and the slot's previous result has left the device
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_in[k], 0));
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_out[k], 0));
-  if (targets_host != nullptr)
-    DP_TRY(dp_sample_eval(s->h, s->x_dev[k], 0, s->out_dev[k], n_pose, s->n_hyp, steps_host, n_steps, noise_dev, mask_dev, s->mean, s->gt_dev[k], sums_dev, stream));
-  else
-    DP_TRY(dp_sample(s->h, s->x_dev[k], 0, s->out_dev[k], n_pose, s->n_hyp, steps_host, n_steps, noise_dev, mask_dev, s->mean, stream));
+  DP_TRY(sample_impl(s->h, s->x_dev[k], 0, s->out_dev[k], n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key, mask_dev, s->mean,
+                     targets_host != nullptr ? s->gt_dev[k] : nullptr, sums_dev, stream));
   DP_CUDA(cudaEventRecord(s->ev_done[k], cs));
   // D2H on the copy-out stream
   DP_CUDA(cudaStreamWaitEvent(s->s_out, s->ev_done[k], 0));
@@ -584,13 +624,21 @@ static int hstream_submit(dp_hstream_t s, const float* x_host, const float* targ
 
 int dp_hstream_submit(dp_hstream_t s, const float* x_host, long n_pose, const dp_step* steps_host, int n_steps, const float* noise_dev,
                       const unsigned char* mask_dev, float* out_host, void* stream, int* slot_out) {
-  return hstream_submit(s, x_host, nullptr, nullptr, n_pose, steps_host, n_steps, noise_dev, mask_dev, out_host, stream, slot_out);
+  return hstream_submit(s, x_host, nullptr, nullptr, n_pose, steps_host, n_steps, noise_dev, nullptr, mask_dev, out_host, stream, slot_out);
 }
 
 int dp_hstream_submit_eval(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose, const dp_step* steps_host,
                            int n_steps, const float* noise_dev, const unsigned char* mask_dev, float* out_host, void* stream, int* slot_out) {
   DP_REQUIRE(targets_host && sums_dev, "dp_hstream_submit_eval: NULL argument");
-  return hstream_submit(s, x_host, targets_host, sums_dev, n_pose, steps_host, n_steps, noise_dev, mask_dev, out_host, stream, slot_out);
+  return hstream_submit(s, x_host, targets_host, sums_dev, n_pose, steps_host, n_steps, noise_dev, nullptr, mask_dev, out_host, stream, slot_out);
+}
+
+int dp_hstream_submit_keyed(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
+                            const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask_dev,
+                            float* out_host, void* stream, int* slot_out) {
+  DP_REQUIRE(key, "dp_hstream_submit_keyed: NULL key");
+  DP_REQUIRE(!targets_host || sums_dev, "dp_hstream_submit_keyed: targets_host needs sums_dev");
+  return hstream_submit(s, x_host, targets_host, sums_dev, n_pose, steps_host, n_steps, nullptr, key, mask_dev, out_host, stream, slot_out);
 }
 
 int dp_hstream_wait(dp_hstream_t s, int slot) {

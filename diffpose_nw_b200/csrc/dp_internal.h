@@ -7,6 +7,7 @@
 #include <vector>
 #include "../../include/diffpose_b200.h"
 #include "../../include/diffpose_b200_diag.h"
+#include "dp_philox.cuh"
 
 namespace dp {
 
@@ -115,6 +116,7 @@ struct EngineCall {
   const dp_step* steps_dev = nullptr;   // the handle's step table when n_steps > kMaxInlineSteps, else NULL
   const StepsArg* inl = nullptr;        // the step scalars otherwise (zero for a forward call)
   const float* noise = nullptr;
+  NoiseKey key{};                       // key.on: the noise is the keyed stream (dp_philox.cuh) and `noise` is NULL
   const unsigned char* mask = nullptr;
   bool forward_only = false;
   // fused by tcg only
@@ -197,4 +199,6 @@ int metrics_launch(const float* pred, int pred_stride, int pred_offset, const fl
 int hyp_mean_launch(const float* x, float* out, long n_pose, int n_hyp, int row_floats, cudaStream_t s);
 // out[n][n_pts][c_in + c_out] = [uv | xyz - xyz[root]] (runners/diffpose_frame.py:337-343 with out-of-place root-centring)
 int lift_glue_launch(const float* uv, const float* xyz, float* out, long n, int n_pts, int c_in, int c_out, cudaStream_t s);
+// out[k][h * n_pose + p][e] = philox_normal(key, step_offset + k, pose_offset + p, h, e), e < row_floats (dp_noise_fill)
+int noise_fill_launch(const NoiseKey& key, int n_steps, long n_pose, int n_hyp, int row_floats, float* out, cudaStream_t s);
 }  // namespace dp

@@ -39,6 +39,7 @@ struct SimtArgs {
   int forward_only;
   const float* temb;   // [n_steps | n_rows][n_layer][hid]
   const float* noise;  // [n_steps][n_rows][17][c] or NULL
+  NoiseKey key;        // key.on: z from the keyed stream instead (noise is NULL)
   const unsigned char* mask;
   const dp_step* steps_dev;
   int P;
@@ -332,6 +333,12 @@ __global__ void __launch_bounds__(kThreads, 1) simt_kernel(SimtArgs a, StepsArg 
           if (a.noise) {
             const float z = a.noise[((size_t)step * a.n_rows + g0) * NP * cin + idx];
             nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
+          } else if (a.key.on) {
+            // hypothesis-major row g = h * n_pose + b
+            const long g = g0 + r / NP, h = g / a.n_pose;
+            const float z = philox_normal(a.key, a.key.step_offset + (uint32_t)step, a.key.pose_offset + (uint32_t)(g - h * a.n_pose),
+                                          (uint32_t)h, (uint32_t)((r % NP) * cin + c));
+            nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
           }
           xt[r * 8 + c] = __fadd_rn(nx, __fmul_rn(st.c2, et));
         }
@@ -493,7 +500,7 @@ int simt_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   SimtArgs a{};
   a.w = m->dw.get<Weights>(); a.d = m->d; a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
   a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_steps = c.n_steps; a.forward_only = c.forward_only;
-  a.temb = m->temb.get<float>(); a.noise = c.noise; a.mask = c.mask; a.steps_dev = c.steps_dev;
+  a.temb = m->temb.get<float>(); a.noise = c.noise; a.key = c.key; a.mask = c.mask; a.steps_dev = c.steps_dev;
   a.P = pick_tile(m, a.n_rows);
   return dispatch_simt(m, a, *c.inl, s);
 }

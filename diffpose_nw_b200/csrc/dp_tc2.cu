@@ -134,6 +134,7 @@ struct Tc2Args {
   double* sums;              //   mean, if any) adds its MPJPE / P-MPJPE to sums[0..1] and 1 to sums[2] (common/loss.py, dp_metrics)
   long long* trace;          // optional diagnostic: CTA 0 records clock64() at every hand-over (see dp_set_trace)
   int trace_cap;
+  NoiseKey key;              // key.on: z from the keyed stream instead of noise (NULL); runs the KEYED instantiation
 };
 
 // ------------------------------------------------------------------------------------------------ compute-warp pieces
@@ -372,7 +373,9 @@ __device__ __forceinline__ __half* tall_elem(uint8_t* smem, int which, int trow,
 // TRACE = true compiles the clock64() stamps of dp_set_trace in; the production instantiation carries none of it.
 // EVAL = true compiles the fused evaluation tail (dp_sample_eval) in: ~3 000 instructions that the plain sampler instantiation
 // does not carry either.
-template <bool TRACE, bool EVAL>
+// KEYED = true draws z from the keyed stream (a.key, dp_philox.cuh) instead of reading a.noise; the unkeyed instantiations
+// carry none of the Philox code, so their schedule is the one they had before keyed noise existed.
+template <bool TRACE, bool EVAL, bool KEYED>
 __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg inl) {
   auto signal_ready = [](Ctx& c) { signal_ready_t<TRACE>(c); };
   auto signal_ready_tmem = [](Ctx& c) { signal_ready_t<TRACE, false>(c); };
@@ -968,6 +971,15 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
             long grow = g0 + p;       // row of the caller's hypothesis-major arrays (noise, eps)
             if (a.mean_over_hyp) { const long b = grow / a.n_hyp; grow = (grow - b * a.n_hyp) * a.n_pose + b; }
             const size_t o = ((size_t)grow * NP + i) * co;
+            // keyed noise: this thread's elements e0 .. e0 + 2 of row (b, h) lie in at most two Philox quads
+            uint4 qa = make_uint4(0, 0, 0, 0), qb = qa;
+            const uint32_t e0 = (uint32_t)(i * co + n0);
+            if (KEYED) {
+              const long h = grow / a.n_pose;
+              const uint32_t s = a.key.step_offset + (uint32_t)step, b = a.key.pose_offset + (uint32_t)(grow - h * a.n_pose);
+              qa = philox_quad(a.key, s, b, (uint32_t)h, e0 >> 2);
+              qb = ((e0 + (uint32_t)(n1 - n0) - 1u) >> 2) != (e0 >> 2) ? philox_quad(a.key, s, b, (uint32_t)h, (e0 >> 2) + 1u) : qa;
+            }
 #pragma unroll
             for (int k = 0; k < 3; ++k) {
               const int n = n0 + k;
@@ -979,6 +991,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
                 const float x0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(et[k], st.sqrt_1m_at)), st.sqrt_at);
                 float nx = __fmul_rn(st.sqrt_an, x0);
                 if (a.noise) nx = __fadd_rn(nx, __fmul_rn(st.c1, a.noise[(size_t)step * a.n_rows * NP * co + o + n]));
+                else if (KEYED) {
+                  const uint32_t e = e0 + (uint32_t)k;
+                  nx = __fadd_rn(nx, __fmul_rn(st.c1, philox_box_muller((e >> 2) == (e0 >> 2) ? qa : qb, e & 3u)));
+                }
                 xt[r * XS + n] = __fadd_rn(nx, __fmul_rn(st.c2, et[k]));
               }
             }
@@ -1207,16 +1223,18 @@ int tc2_pack(dp_model* m, cudaStream_t s) {
 int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   const uint8_t* blocks = m->tc2_blocks.get<uint8_t>();
   if (!blocks) { set_error("tensor-core engine: weights are not packed"); return DP_ERR_STATE; }
-  DP_TRY((smem_opt_in<tc2_kernel<false, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<true, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<true, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, true>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, true>>(m->device, SMEM_BYTES)));
   const size_t wbytes = (size_t)m->d.n_layer * BLOCKS_PER_LAYER * WBLK_BYTES;
   Tc2Args a{};
   a.w = m->dw.get<Weights>(); a.wpack = blocks; a.ioblocks = blocks + wbytes; a.lparams = blocks + wbytes + 2 * WBLK_BYTES;
   a.n_layer = m->d.n_layer; a.c_in = m->d.c_in; a.c_out = m->d.c_out; a.forward_only = c.forward_only; a.has_temb = m->d.has_temb;
   a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
   a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_hyp = c.n_hyp; a.mean_over_hyp = c.mean_over_hyp; a.n_steps = c.n_steps;
-  a.temb = m->temb.get<float>(); a.tau = m->tc2_tau.get<uint8_t>(); a.noise = c.noise; a.mask = c.mask; a.steps_dev = c.steps_dev;
+  a.temb = m->temb.get<float>(); a.tau = m->tc2_tau.get<uint8_t>(); a.noise = c.noise; a.key = c.key; a.mask = c.mask; a.steps_dev = c.steps_dev;
   a.gt = c.gt; a.sums = c.sums; a.trace = m->trace; a.trace_cap = m->trace_cap;
   const long n_tiles = (a.n_rows + TP - 1) / TP;
   if (n_tiles > 0x7fffffffL) { set_error("tensor-core engine: more than 2^31 tiles of 7 poses in one call"); return DP_ERR_INVALID; }
@@ -1228,9 +1246,12 @@ int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true>, a, *c.inl));
-  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false>, a, *c.inl));
-  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false>, a, *c.inl));
+  // a keyed call runs a keyed instantiation (without the hand-over trace, which only the plain sampler records)
+  if (a.key.on && a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true>, a, *c.inl));
+  else if (a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, true>, a, *c.inl));
+  else if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false>, a, *c.inl));
+  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false, false>, a, *c.inl));
+  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, false>, a, *c.inl));
   count_launch();
   record_launch(m, grid, kThreads, SMEM_BYTES, TP, DP_ENGINE_TCG, n_tiles);
   return DP_OK;

@@ -104,6 +104,7 @@ struct TcxArgs {
   int n_steps;
   const float* temb;         // sampler: [n_steps][n_layer][96]; forward: [n_rows][n_layer][96]
   const float* noise;
+  NoiseKey key;              // key.on: z from the keyed stream instead (noise is NULL)
   const unsigned char* mask;
   const dp_step* steps_dev;
 };
@@ -747,6 +748,12 @@ __global__ void __launch_bounds__(kThreads, 1) tcx_kernel(TcxArgs a, StepsArg in
             if (a.noise) {
               const float z = a.noise[((size_t)step * a.n_rows + g0) * NP * co + idx];
               nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
+            } else if (a.key.on) {
+              // hypothesis-major row g = h * n_pose + b
+              const long g = g0 + r / NP, h = g / a.n_pose;
+              const float z = philox_normal(a.key, a.key.step_offset + (uint32_t)step, a.key.pose_offset + (uint32_t)(g - h * a.n_pose),
+                                            (uint32_t)h, (uint32_t)((r % NP) * co + c));
+              nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
             }
             xt[r * XS + c] = __fadd_rn(nx, __fmul_rn(st.c2, et));
           }
@@ -825,7 +832,7 @@ int tcx_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   a.forward_only = c.forward_only; a.has_temb = m->d.has_temb; a.emit_uvxyz = c.emit_uvxyz;
   a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
   a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_steps = c.n_steps;
-  a.temb = m->temb.get<float>(); a.noise = c.noise; a.mask = c.mask; a.steps_dev = c.steps_dev;
+  a.temb = m->temb.get<float>(); a.noise = c.noise; a.key = c.key; a.mask = c.mask; a.steps_dev = c.steps_dev;
   const long n_tiles = (a.n_rows + TP - 1) / TP;
   const int grid = (int)(n_tiles < m->sm_count ? n_tiles : m->sm_count);
   tcx_kernel<<<grid, kThreads, SMEM_BYTES, s>>>(a, *c.inl);

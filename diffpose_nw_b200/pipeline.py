@@ -9,6 +9,8 @@ exchange nothing inside the loop; one all-reduce of three fp64 partial sums ends
 """
 from __future__ import annotations
 
+import ctypes
+
 import torch
 
 from .metrics import pose_error_sums
@@ -23,21 +25,24 @@ def shard_range(n, rank, world):
 
 
 def lift_and_refine(model_diff, x_uvxyz=None, *, model_pose=None, input_2d=None, src_mask=None, seq, betas, eta=0.0,
-                    test_times=1, noise=None, targets=None, sums=None):
+                    test_times=1, noise=None, targets=None, sums=None, seed=None, pose_offset=0):
     """Two-stage inference for one batch.  Give either `x_uvxyz` [B,17,5] or (`model_pose`, `input_2d` [B,17,2]).
     Returns the hypothesis-averaged uvxyz [B,17,5].  With `targets` [B,17,3] and `sums` (CUDA fp64 [3]) the MPJPE / P-MPJPE
-    partial sums of the batch are accumulated by the sampler launch itself (`dp_sample_eval`)."""
+    partial sums of the batch are accumulated by the sampler launch itself (`dp_sample_eval`).  `seed` draws the noise in
+    the kernel (keyed stream, see `sample`); `pose_offset` is the global index of the batch's first pose."""
     if x_uvxyz is None:
         # lift + out-of-place root-centring (SURVEY.md 8a quirk 4) + concat in ONE launch (dp_lift); the sampler below is
         # the second and last launch of the batch (kernel-side repeat, hypothesis mean fused into its final store)
         x_uvxyz = getattr(model_pose, "module", model_pose).lift(input_2d, src_mask)
     return sample(model_diff, x_uvxyz, src_mask, seq, betas, eta=eta, noise=noise, n_hyp=test_times,
-                  repeat_input=True, mean_over_hyp=True, targets=targets, sums=sums)
+                  repeat_input=True, mean_over_hyp=True, targets=targets, sums=sums, seed=seed, pose_offset=pose_offset)
 
 
 def evaluate_shard(model_diff, x_uvxyz, targets_3d, *, src_mask=None, seq, betas, eta=0.0, test_times=1, noise=None,
-                   batch_size=None, model_pose=None, input_2d=None):
-    """Sample this rank's poses and return fp64 partial sums [sum mpjpe, sum p_mpjpe, n] (metres) on the device."""
+                   batch_size=None, model_pose=None, input_2d=None, seed=None, pose_offset=0):
+    """Sample this rank's poses and return fp64 partial sums [sum mpjpe, sum p_mpjpe, n] (metres) on the device.
+    With `seed` the noise is the keyed stream and `pose_offset` the global index of this shard's first pose (the `lo` of
+    `shard_range`): every pose then draws the same noise whatever the number of ranks or the batch size."""
     n = targets_3d.shape[0]
     dev = targets_3d.device
     sums = torch.zeros(3, device=dev, dtype=torch.float64)
@@ -51,7 +56,8 @@ def evaluate_shard(model_diff, x_uvxyz, targets_3d, *, src_mask=None, seq, betas
         # sampler + metrics of the batch in one launch (two with the lifter in front)
         lift_and_refine(model_diff, None if x_uvxyz is None else x_uvxyz[lo:hi], model_pose=model_pose,
                         input_2d=None if input_2d is None else input_2d[lo:hi], src_mask=src_mask, seq=seq,
-                        betas=betas, eta=eta, test_times=test_times, noise=nz, targets=targets_3d[lo:hi], sums=sums)
+                        betas=betas, eta=eta, test_times=test_times, noise=nz, targets=targets_3d[lo:hi], sums=sums,
+                        seed=seed, pose_offset=pose_offset + lo)
     return sums
 
 
@@ -82,11 +88,13 @@ class HostStream:
 
     Results come back in submission order.  `depth` batches are in flight; every buffer is allocated once.  A returned
     tensor aliases a ring buffer and stays valid for the next `depth` submits.
+
+    eta > 0 needs `seed`: the kernel then draws the noise from the keyed stream (`dp_hstream_submit_keyed`), and the poses
+    of consecutive batches are numbered like one big call, so the results equal one `sample(seed=...)` over all batches.
     """
 
-    def __init__(self, model_diff, batch, seq, betas, eta=0.0, test_times=1, src_mask=None, depth=3, device=None):
+    def __init__(self, model_diff, batch, seq, betas, eta=0.0, test_times=1, src_mask=None, depth=3, device=None, seed=None):
         import collections
-        import ctypes
         from . import _lib
         from .sampler import ddim_steps
         self.model = getattr(model_diff, "module", model_diff)
@@ -96,8 +104,11 @@ class HostStream:
         self.B, self.H, self.depth = batch, test_times, depth
         self.steps = ddim_steps(betas, seq, eta)
         self.T = len(self.steps)
-        if any(s.c1 != 0.0 for s in self.steps):
-            raise RuntimeError("HostStream draws no noise: use eta = 0, or call sample() with noise= per batch")
+        self._keyed = seed is not None and any(s.c1 != 0.0 for s in self.steps)
+        if any(s.c1 != 0.0 for s in self.steps) and seed is None:
+            raise RuntimeError("HostStream takes no noise tensor: use eta = 0, or pass seed= for keyed in-kernel noise")
+        self.seed = seed
+        self.n_submitted = 0                       # poses submitted so far: the default pose_offset of the next batch
         self.model._ensure_packed(self.dev)
         self._lib = _lib.load()
         self._mask = self.model._mask_bytes(src_mask, self.dev)
@@ -122,10 +133,11 @@ class HostStream:
             _lib.check(rc, "dp_hstream_wait")
         return self.out_host[hb][:n]
 
-    def submit(self, x_host, targets_host=None, sums=None):
+    def submit(self, x_host, targets_host=None, sums=None, pose_offset=None):
         """Queue one pinned host batch [n<=B,17,c] (fp32, contiguous).  Returns the oldest finished result when the ring is
         full, else None.  With `targets_host` [n,17,3] (pinned fp32) and `sums` (CUDA fp64 [3]) the batch's MPJPE / P-MPJPE
-        partial sums are accumulated by the sampler launch itself (`dp_hstream_submit_eval`)."""
+        partial sums are accumulated by the sampler launch itself (`dp_hstream_submit_eval`).  With a seed, `pose_offset`
+        is the global index of the batch's first pose; it defaults to the number of poses submitted before."""
         n = x_host.shape[0]
         if n > self.B:
             raise RuntimeError(f"batch of {n} poses exceeds the {self.B} this HostStream was built for")
@@ -138,21 +150,29 @@ class HostStream:
         hb = self._hpos
         self._hpos = (hb + 1) % len(self.out_host)
         stream = torch.cuda.current_stream(self.dev).cuda_stream
-        if targets_host is None:
-            rc = self._lib.dp_hstream_submit(self.hs, x_host.data_ptr(), n, self.steps, self.T, None, self._mask_ptr,
-                                             self.out_host[hb].data_ptr(), stream, self._slot_ref)
-        else:
+        if targets_host is not None:
             if (targets_host.is_cuda or targets_host.dtype is not torch.float32 or not targets_host.is_contiguous()
                     or tuple(targets_host.shape) != (n, 17, 3)):
                 raise RuntimeError(f"targets_host must be a contiguous fp32 HOST tensor [{n},17,3]")
             if sums is None or not sums.is_cuda or sums.dtype is not torch.float64 or sums.numel() != 3:
                 raise RuntimeError("fused evaluation needs `sums`: a CUDA float64 tensor of 3 elements")
+        if self._keyed:
+            from . import _lib
+            key = _lib.noise_key(self.seed, self.n_submitted if pose_offset is None else pose_offset)
+            rc = self._lib.dp_hstream_submit_keyed(self.hs, x_host.data_ptr(), None if targets_host is None else targets_host.data_ptr(),
+                                                   None if targets_host is None else sums.data_ptr(), n, self.steps, self.T,
+                                                   ctypes.byref(key), self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
+        elif targets_host is None:
+            rc = self._lib.dp_hstream_submit(self.hs, x_host.data_ptr(), n, self.steps, self.T, None, self._mask_ptr,
+                                             self.out_host[hb].data_ptr(), stream, self._slot_ref)
+        else:
             rc = self._lib.dp_hstream_submit_eval(self.hs, x_host.data_ptr(), targets_host.data_ptr(), sums.data_ptr(), n, self.steps, self.T,
                                                   None, self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
         if rc != 0:
             from . import _lib
             _lib.check(rc, "dp_hstream_submit")
         self._pending.append((self._slot.value, hb, n, x_host, targets_host))
+        self.n_submitted += n
         return ret
 
     def drain(self):

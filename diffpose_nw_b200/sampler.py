@@ -107,12 +107,17 @@ def _unwrap(model):
 
 
 def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_input=False, mean_over_hyp=False,
-           steps=None, targets=None, sums=None):
+           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0):
     """Run the DDIM loop on the device and return x_T.
 
     x: [n_hyp*n_pose,17,c] hypothesis-major (what `.repeat(test_times,1,1)` produces), or [n_pose,17,c] with
     `repeat_input=True` to let the kernel read each pose n_hyp times instead of materialising the repeat.
     noise: optional [T, n_hyp*n_pose, 17, c] standard-normal draws replacing `torch.randn_like` (:65).
+    seed: draw the noise inside the kernel from the keyed stream (`dp_sample_keyed`, include/diffpose_b200.h) instead: one
+    launch, no noise tensor, and every pose receives the same draws however the work is split, as long as each piece
+    passes the global index of its first pose as `pose_offset` (and a call that runs step k of a schedule alone passes
+    `step_offset=k`).  `philox_noise` writes the same stream out.  Not together with `noise`; no effect when eta = 0.
+    Without `noise` and `seed`, eta > 0 draws with torch.randn, in chunks of at most NOISE_CHUNK_BYTES.
     mean_over_hyp: fuse `mean(reshape(n_hyp,-1,17,c),0)` (runners/diffpose_frame.py:382) after the loop.
     targets, sums: fused evaluation (`dp_sample_eval`): targets [n_pose,17,3] on the device and a CUDA fp64 tensor of 3
     partial sums `[sum mpjpe, sum p_mpjpe, n]` that every finished pose is added to in the same launch (:384-387); with
@@ -136,7 +141,13 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     c = m._c_in
     nz = None
     draw = False
-    if noise is not None:
+    key = None
+    if seed is not None and noise is not None:
+        raise RuntimeError("sample: pass either seed= (keyed in-kernel noise) or noise=, not both")
+    if seed is not None:
+        if any(s.c1 != 0.0 for s in steps):   # eta = 0: the seed has no effect, the call is the unkeyed one
+            key = _lib.noise_key(seed, pose_offset, step_offset)
+    elif noise is not None:
         nz = torch.as_tensor(noise, device=dev).detach().to(torch.float32).contiguous()
         if tuple(nz.shape) != (T, total, m.n_pts, c):
             raise RuntimeError(f"noise must be [{T},{total},{m.n_pts},{c}], got {tuple(nz.shape)}")
@@ -161,7 +172,11 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
 
     def launch(x_t, out_t, n_p, nz_t, repeated, lo=0):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        if tg is None:
+        if key is not None:
+            rc = lib.dp_sample_keyed(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
+                                     ctypes.byref(key), mask_ptr, 1 if mean_over_hyp else 0,
+                                     None if tg is None else tg.data_ptr(), None if tg is None else sums.data_ptr(), stream)
+        elif tg is None:
             rc = lib.dp_sample(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
                                nz_t.data_ptr() if nz_t is not None else None, mask_ptr, 1 if mean_over_hyp else 0, stream)
         else:
@@ -212,22 +227,43 @@ def generalized_steps(x, src_mask, seq, model, b, **kwargs):
     Returns `(xs, x0_preds)` with `xs = [x, x_T]` and `x0_preds = []`: the fused kernel keeps the intermediate
     x_t / x0 on chip (the only consumer in the reference takes `[0][-1]`).  Pass `return_all=True` to get the
     full per-step lists (one single-step launch per step; slower, for debugging and parity tests).
-    Extra keyword `noise=[T,n,17,c]` supplies the per-step normal draws.
+    Extra keyword `noise=[T,n,17,c]` supplies the per-step normal draws; `seed=` draws them in the kernel from the keyed
+    stream instead (see `sample`), the same stream with and without `return_all`.
     """
     eta = kwargs.get("eta", 0)
     noise = kwargs.get("noise", None)
+    seed = kwargs.get("seed", None)
     with torch.no_grad():
         if not kwargs.get("return_all", False):
-            return [x, sample(model, x, src_mask, seq, b, eta=eta, noise=noise)], []
+            return [x, sample(model, x, src_mask, seq, b, eta=eta, noise=noise, seed=seed)], []
+        if seed is not None and noise is not None:
+            raise RuntimeError("generalized_steps: pass either seed= or noise=, not both")
         steps = ddim_steps(b, seq, eta)
         xs, x0_preds = [x], []
         for k in range(len(steps)):
             one = (_lib.DpStep * 1)(steps[k])
             xt = xs[-1]
             nz = None if noise is None else noise[k:k + 1]
-            nxt = sample(model, xt, src_mask, None, b, noise=nz, steps=one)
+            nxt = sample(model, xt, src_mask, None, b, noise=nz, steps=one, seed=seed, step_offset=k)
             # x0 is recovered from the update rule: x_next = sqrt(an) x0 + c1 z + c2 eps, eps = (xt - sqrt(at) x0)/sqrt(1-at)
             et = _unwrap(model)(xt, src_mask, torch.full((xt.shape[0],), steps[k].t, device=xt.device), 0)
             x0_preds.append((xt - et * steps[k].sqrt_1m_at) / steps[k].sqrt_at)
             xs.append(nxt)
         return xs, x0_preds
+
+
+def philox_noise(seed, n_steps, n_pose, n_hyp=1, *, pose_offset=0, step_offset=0, device=None, n_pts=17, c=5):
+    """The keyed noise stream of `sample(seed=...)` as a CUDA tensor [n_steps, n_hyp*n_pose, n_pts, c] (hypothesis-major, the
+    layout of `noise=`), written by `dp_noise_fill`: `sample(..., noise=philox_noise(seed, T, n, H, pose_offset=o))` equals
+    `sample(..., seed=seed, pose_offset=o)` bit for bit."""
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    if dev.type != "cuda":
+        raise RuntimeError("philox_noise: the stream is written on a CUDA device (diffpose_nw_b200 has no CPU path)")
+    out = torch.empty(n_steps, n_hyp * n_pose, n_pts, c, device=dev, dtype=torch.float32)
+    lib = _lib.load()
+    key = _lib.noise_key(seed, pose_offset, step_offset)
+    with torch.cuda.device(dev):
+        rc = lib.dp_noise_fill(ctypes.byref(key), n_steps, n_pose, n_hyp, n_pts, c, out.data_ptr() if out.numel() else None,
+                               torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(rc, "dp_noise_fill")
+    return out

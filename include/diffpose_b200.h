@@ -146,6 +146,41 @@ int dp_sample_eval(dp_handle h, const float* x_in, int x_is_repeated, float* x_o
                    const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
                    int mean_over_hyp, const float* targets_xyz, double* sums, void* stream);
 
+/* Keyed noise: the sampler kernels draw z themselves from a counter-based stream, so a call needs no noise tensor and the
+ * value every (pose, hypothesis, step, element) receives does not depend on how the work is split into calls, batches,
+ * tiles or ranks.  The stream (this definition is part of the ABI):
+ *   Philox4x32-10 (Salmon et al., SC'11; the round function and constants of Random123 / cuRAND Philox4_32_10)
+ *   key      (seed & 0xffffffff, seed >> 32)
+ *   counter  (e >> 2, s, b, h) as 32-bit words c0..c3, for element e = joint * c + coord (c = 5 for uvxyz) of
+ *            global pose b = pose_offset + local pose, hypothesis h, step s = step_offset + k (k = execution index in
+ *            the call, 0 = the first, largest t)
+ *   normal   with output words x0..x3, l = e & 3, m = l >> 1:
+ *            u1 = ((x[2m] >> 8) + 1) 2^-24 in (0, 1],  u2 = (x[2m+1] >> 8) 2^-24 in [0, 1),
+ *            z = sqrtf(-2 logf(u1)) * (l even ? cospif(2 u2) : sinpif(2 u2)), every operation IEEE-rounded fp32.
+ * Offset rules: a caller that splits one logical call into pieces gives each piece the global index of its first pose as
+ * pose_offset (a rank: the start of its shard; a batch loop: the start of the batch), so the pieces together draw what one
+ * call over all poses would.  A caller that runs the steps of one schedule as separate calls gives the call that runs
+ * step k step_offset = k.  The pose index is one 32-bit word: pose_offset < 0, step_offset < 0 or
+ * pose_offset + n_pose > 2^32 return DP_ERR_INVALID.  Different seeds (including seeds that differ only in their high
+ * 32 bits) are different streams. */
+typedef struct dp_noise_key {
+  unsigned long long seed;
+  long pose_offset;
+  int step_offset;
+} dp_noise_key;
+
+/* dp_sample (targets_xyz = NULL) or dp_sample_eval (targets_xyz and sums given) with the keyed stream in place of the noise
+ * tensor: one launch, no [T, n_pose*n_hyp, n_pts, c] buffer.  Same engines, layouts and graph-capture rules as dp_sample;
+ * the key travels by value in the kernel arguments.  When every c1 = 0 (eta = 0) the key has no effect. */
+int dp_sample_keyed(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                    const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask,
+                    int mean_over_hyp, const float* targets_xyz, double* sums, void* stream);
+
+/* Writes the keyed stream as out [n_steps][n_hyp*n_pose][n_pts][c] (hypothesis-major: row h*n_pose + p is pose
+ * pose_offset + p, hypothesis h; step k is s = step_offset + k) -- the layout of dp_sample's `noise`.  So
+ * dp_sample(noise = out) equals dp_sample_keyed(key) bit for bit. */
+int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, int n_pts, int c, float* out, void* stream);
+
 /* Batches that live in HOST memory.  Replaces the copy-in / sample / copy-out sequence of the evaluation loop
  * (runners/diffpose_frame.py:333-335 `input_2d.to(self.device)` ..., :365 generalized_steps, :387 `.cpu()`), which the
  * reference runs strictly one after the other, by a ring of `depth` slots: the host->device copy of batch i+1 and the
@@ -169,6 +204,12 @@ int dp_hstream_submit(dp_hstream_t s, const float* x_host, long n_pose, const dp
 int dp_hstream_submit_eval(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
                            const dp_step* steps_host, int n_steps, const float* noise_dev, const unsigned char* mask_dev, float* out_host,
                            void* stream, int* slot);
+/* dp_hstream_submit (targets_host = NULL) or dp_hstream_submit_eval with keyed noise (dp_sample_keyed) instead of a
+ * noise tensor: an eta > 0 schedule through the ring.  key->pose_offset numbers the batch's first pose; giving each batch
+ * the count of poses submitted before it draws what one dp_sample_keyed over all batches would. */
+int dp_hstream_submit_keyed(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
+                            const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask_dev,
+                            float* out_host, void* stream, int* slot);
 int dp_hstream_wait(dp_hstream_t s, int slot);
 void dp_hstream_destroy(dp_hstream_t s);
 
