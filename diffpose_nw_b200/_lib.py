@@ -45,15 +45,11 @@ SIGNATURES = {
     "dp_device": (_I, [_P]),
     "dp_lift": (_I, [_P, _P, _P, _P, _L, _P]),
     "dp_forward": (_I, [_P, _P, _P, _P, _P, _L, _P]),
-    "dp_sample": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, _P, _I, _P]),
-    "dp_sample_eval": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, _P, _I, _P, _P, _P]),
-    "dp_sample_keyed": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _P]),
+    "dp_sample": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _P]),
     "dp_noise_fill": (_I, [ctypes.POINTER(DpNoiseKey), _I, _L, _I, _I, _I, _P, _P]),
     "dp_hstream_create": (_I, [ctypes.POINTER(_P), _P, _L, _I, _I, _I]),
-    "dp_hstream_submit": (_I, [_P, _P, _L, ctypes.POINTER(DpStep), _I, _P, _P, _P, _P, ctypes.POINTER(_I)]),
-    "dp_hstream_submit_eval": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, _P, _P, _P, _P, ctypes.POINTER(_I)]),
-    "dp_hstream_submit_keyed": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, ctypes.POINTER(DpNoiseKey), _P, _P, _P,
-                                     ctypes.POINTER(_I)]),
+    "dp_hstream_submit": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _P, _P,
+                               ctypes.POINTER(_I)]),
     "dp_hstream_wait": (_I, [_P, _I]),
     "dp_hstream_destroy": (None, [_P]),
     "dp_metrics": (_I, [_P, _I, _I, _P, _L, _I, _P, _P, _P]),

@@ -397,22 +397,21 @@ static int make_key(const dp_noise_key* k, long n_pose, const char* what, NoiseK
   return DP_OK;
 }
 
-// dp_sample, dp_sample_eval, dp_sample_keyed and the host-stream submits: at most one of noise and key is given.
-static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                       const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
-                       int mean_over_hyp, const float* targets, double* sums, void* stream) {
+int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+              const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+              int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
   DP_REQUIRE(h && x_in && x_out && steps_host, "dp_sample: NULL argument");
   DP_REQUIRE(n_pose >= 0 && n_hyp >= 1 && n_steps >= 1, "dp_sample: n_pose >= 0, n_hyp >= 1, n_steps >= 1 required");
   DP_REQUIRE(h->d.has_temb, "dp_sample: handle was created with has_temb = 0 (GCNpose has no sampler)");
   DP_REQUIRE(!(noise && key), "dp_sample: give either a noise tensor or a noise key, not both");
-  if (targets != nullptr) {
-    DP_REQUIRE(sums != nullptr, "dp_sample_eval: NULL argument");
-    DP_REQUIRE(h->d.c_out >= 3, "dp_sample_eval: the model's output needs at least the three xyz coordinates");
-    DP_REQUIRE(n_hyp == 1 || mean_over_hyp, "dp_sample_eval: with n_hyp > 1 the metrics are those of the hypothesis mean (set mean_over_hyp)");
+  if (targets_xyz != nullptr) {
+    DP_REQUIRE(sums != nullptr, "dp_sample: targets_xyz needs sums");
+    DP_REQUIRE(h->d.c_out >= 3, "dp_sample: the model's output needs at least the three xyz coordinates");
+    DP_REQUIRE(n_hyp == 1 || mean_over_hyp, "dp_sample: with n_hyp > 1 the metrics are those of the hypothesis mean (set mean_over_hyp)");
   }
   NoiseKey nk{};
   if (key != nullptr) {
-    DP_TRY(make_key(key, n_pose, "dp_sample_keyed", &nk));
+    DP_TRY(make_key(key, n_pose, "dp_sample", &nk));
     // every c1 = 0 (eta = 0): the noise term is skipped, as with a NULL noise pointer
     bool any = false;
     for (int i = 0; i < n_steps; ++i) any = any || steps_host[i].c1 != 0.f;
@@ -459,10 +458,10 @@ static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float*
   c.n_steps = n_steps; c.steps_dev = steps_dev; c.inl = &inl; c.noise = noise; c.key = nk; c.mask = mask;
   const bool mean = mean_over_hyp && n_hyp > 1;
   const int eng = dp_get_engine(h);
-  // default engine: the hypothesis mean -- and, for dp_sample_eval, the MPJPE / P-MPJPE sums -- are fused into the kernel's
+  // default engine: the hypothesis mean -- and, with targets_xyz, the MPJPE / P-MPJPE sums -- are fused into the kernel's
   // final store (one launch, no [H*B] scratch)
   if (eng == DP_ENGINE_TCG) {
-    c.mean_over_hyp = mean; c.gt = targets; c.sums = sums;
+    c.mean_over_hyp = mean; c.gt = targets_xyz; c.sums = sums;
     return tc2_run(h, c, s);
   }
   const int row_floats = d.n_pts * d.c_out;
@@ -472,28 +471,8 @@ static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float*
   }
   DP_TRY(run_engine(h, eng, c, s));
   if (mean) DP_TRY(hyp_mean_launch(c.out, x_out, n_pose, n_hyp, row_floats, s));
-  if (targets != nullptr) DP_TRY(metrics_launch(x_out, d.c_out, d.c_out - 3, targets, n_pose, d.n_pts, sums, nullptr, s));
+  if (targets_xyz != nullptr) DP_TRY(metrics_launch(x_out, d.c_out, d.c_out - 3, targets_xyz, n_pose, d.n_pts, sums, nullptr, s));
   return DP_OK;
-}
-
-int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-              const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
-              int mean_over_hyp, void* stream) {
-  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, nullptr, mask, mean_over_hyp, nullptr, nullptr, stream);
-}
-
-int dp_sample_eval(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                   const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
-                   int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
-  DP_REQUIRE(h && targets_xyz && sums, "dp_sample_eval: NULL argument");
-  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, nullptr, mask, mean_over_hyp, targets_xyz, sums, stream);
-}
-
-int dp_sample_keyed(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                    const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask,
-                    int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
-  DP_REQUIRE(key, "dp_sample_keyed: NULL key");
-  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, nullptr, key, mask, mean_over_hyp, targets_xyz, sums, stream);
 }
 
 int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, int n_pts, int c, float* out, void* stream) {
@@ -548,7 +527,7 @@ struct dp_hstream {
   int n_hyp = 1, mean = 0, depth = 0, head = 0;
   size_t in_floats = 0, out_floats = 0;
   cudaStream_t s_in = nullptr, s_out = nullptr;
-  std::vector<float*> x_dev, out_dev, gt_dev;     // per slot: input, result, and (evaluation) the targets of the batch
+  DevBuf x_dev[16], out_dev[16], gt_dev[16];       // per slot (depth <= 16): input, result, and (evaluation) the targets of the batch
   std::vector<cudaEvent_t> ev_in, ev_done, ev_out;
 };
 
@@ -567,16 +546,10 @@ int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, 
   cudaError_t e = cudaStreamCreateWithFlags(&s->s_in, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s->s_out, cudaStreamNonBlocking);
   for (int i = 0; i < depth && e == cudaSuccess; ++i) {
-    float *a = nullptr, *b = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
-    e = cudaMalloc(reinterpret_cast<void**>(&a), s->in_floats * sizeof(float));
-    if (e == cudaSuccess) { s->x_dev.push_back(a); e = cudaMalloc(reinterpret_cast<void**>(&b), s->out_floats * sizeof(float)); }
-    if (e == cudaSuccess) {
-      s->out_dev.push_back(b);
-      float* g = nullptr;
-      e = cudaMalloc(reinterpret_cast<void**>(&g), (size_t)max_pose * h->d.n_pts * 3 * sizeof(float));
-      if (e == cudaSuccess) s->gt_dev.push_back(g);
-    }
+    if (s->x_dev[i].reserve(s->in_floats * sizeof(float)) != DP_OK || s->out_dev[i].reserve(s->out_floats * sizeof(float)) != DP_OK ||
+        s->gt_dev[i].reserve((size_t)max_pose * h->d.n_pts * 3 * sizeof(float)) != DP_OK)
+      e = cudaErrorMemoryAllocation;
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&e0, cudaEventDisableTiming);
     if (e == cudaSuccess) { s->ev_in.push_back(e0); e = cudaEventCreateWithFlags(&e1, cudaEventDisableTiming); }
     if (e == cudaSuccess) { s->ev_done.push_back(e1); e = cudaEventCreateWithFlags(&e2, cudaEventDisableTiming); }
@@ -591,11 +564,15 @@ int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, 
   return DP_OK;
 }
 
-static int hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose, const dp_step* steps_host,
-                          int n_steps, const float* noise_dev, const dp_noise_key* key, const unsigned char* mask_dev, float* out_host,
-                          void* stream, int* slot_out) {
+int dp_hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose, const dp_step* steps_host,
+                      int n_steps, const float* noise_dev, const dp_noise_key* key, const unsigned char* mask_dev, float* out_host,
+                      void* stream, int* slot_out) {
   DP_REQUIRE(s && x_host && out_host && steps_host && slot_out, "dp_hstream_submit: NULL argument");
   DP_REQUIRE(n_pose >= 1 && n_pose <= s->max_pose, "dp_hstream_submit: batch exceeds the max_pose this stream was created for");
+  // the combinations dp_sample refuses, refused before the copies below are enqueued
+  DP_REQUIRE(!(noise_dev && key), "dp_hstream_submit: give either a noise tensor or a noise key, not both");
+  DP_REQUIRE(!targets_host || (sums_dev && (s->n_hyp == 1 || s->mean)),
+             "dp_hstream_submit: targets_host needs sums_dev and, with n_hyp > 1, a stream created with mean_over_hyp");
   DP_TRY(check_device(s->h, "dp_hstream_submit"));
   cudaStream_t cs = static_cast<cudaStream_t>(stream);
   const int k = s->head;
@@ -603,42 +580,23 @@ static int hstream_submit(dp_hstream_t s, const float* x_host, const float* targ
   const size_t in_bytes = (size_t)n_pose * row * sizeof(float), out_bytes = (size_t)n_pose * (s->mean ? 1 : s->n_hyp) * row * sizeof(float);
   // H2D on the copy-in stream, once the kernel that last read this slot's input has finished
   DP_CUDA(cudaStreamWaitEvent(s->s_in, s->ev_done[k], 0));
-  DP_CUDA(cudaMemcpyAsync(s->x_dev[k], x_host, in_bytes, cudaMemcpyHostToDevice, s->s_in));
+  DP_CUDA(cudaMemcpyAsync(s->x_dev[k].get<float>(), x_host, in_bytes, cudaMemcpyHostToDevice, s->s_in));
   if (targets_host != nullptr)
-    DP_CUDA(cudaMemcpyAsync(s->gt_dev[k], targets_host, (size_t)n_pose * s->h->d.n_pts * 3 * sizeof(float), cudaMemcpyHostToDevice, s->s_in));
+    DP_CUDA(cudaMemcpyAsync(s->gt_dev[k].get<float>(), targets_host, (size_t)n_pose * s->h->d.n_pts * 3 * sizeof(float), cudaMemcpyHostToDevice, s->s_in));
   DP_CUDA(cudaEventRecord(s->ev_in[k], s->s_in));
   // the sampler on the caller's stream, once the input is there and the slot's previous result has left the device
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_in[k], 0));
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_out[k], 0));
-  DP_TRY(sample_impl(s->h, s->x_dev[k], 0, s->out_dev[k], n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key, mask_dev, s->mean,
-                     targets_host != nullptr ? s->gt_dev[k] : nullptr, sums_dev, stream));
+  DP_TRY(dp_sample(s->h, s->x_dev[k].get<float>(), 0, s->out_dev[k].get<float>(), n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key,
+                   mask_dev, s->mean, targets_host != nullptr ? s->gt_dev[k].get<float>() : nullptr, sums_dev, stream));
   DP_CUDA(cudaEventRecord(s->ev_done[k], cs));
   // D2H on the copy-out stream
   DP_CUDA(cudaStreamWaitEvent(s->s_out, s->ev_done[k], 0));
-  DP_CUDA(cudaMemcpyAsync(out_host, s->out_dev[k], out_bytes, cudaMemcpyDeviceToHost, s->s_out));
+  DP_CUDA(cudaMemcpyAsync(out_host, s->out_dev[k].get<float>(), out_bytes, cudaMemcpyDeviceToHost, s->s_out));
   DP_CUDA(cudaEventRecord(s->ev_out[k], s->s_out));
   *slot_out = k;
   s->head = (k + 1) % s->depth;
   return DP_OK;
-}
-
-int dp_hstream_submit(dp_hstream_t s, const float* x_host, long n_pose, const dp_step* steps_host, int n_steps, const float* noise_dev,
-                      const unsigned char* mask_dev, float* out_host, void* stream, int* slot_out) {
-  return hstream_submit(s, x_host, nullptr, nullptr, n_pose, steps_host, n_steps, noise_dev, nullptr, mask_dev, out_host, stream, slot_out);
-}
-
-int dp_hstream_submit_eval(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose, const dp_step* steps_host,
-                           int n_steps, const float* noise_dev, const unsigned char* mask_dev, float* out_host, void* stream, int* slot_out) {
-  DP_REQUIRE(targets_host && sums_dev, "dp_hstream_submit_eval: NULL argument");
-  return hstream_submit(s, x_host, targets_host, sums_dev, n_pose, steps_host, n_steps, noise_dev, nullptr, mask_dev, out_host, stream, slot_out);
-}
-
-int dp_hstream_submit_keyed(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
-                            const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask_dev,
-                            float* out_host, void* stream, int* slot_out) {
-  DP_REQUIRE(key, "dp_hstream_submit_keyed: NULL key");
-  DP_REQUIRE(!targets_host || sums_dev, "dp_hstream_submit_keyed: targets_host needs sums_dev");
-  return hstream_submit(s, x_host, targets_host, sums_dev, n_pose, steps_host, n_steps, nullptr, key, mask_dev, out_host, stream, slot_out);
 }
 
 int dp_hstream_wait(dp_hstream_t s, int slot) {
@@ -651,9 +609,6 @@ void dp_hstream_destroy(dp_hstream_t s) {
   if (!s) return;
   if (s->s_in) cudaStreamSynchronize(s->s_in);
   if (s->s_out) cudaStreamSynchronize(s->s_out);
-  for (float* p : s->x_dev) cudaFree(p);
-  for (float* p : s->out_dev) cudaFree(p);
-  for (float* p : s->gt_dev) cudaFree(p);
   for (cudaEvent_t e : s->ev_in) cudaEventDestroy(e);
   for (cudaEvent_t e : s->ev_done) cudaEventDestroy(e);
   for (cudaEvent_t e : s->ev_out) cudaEventDestroy(e);
@@ -671,7 +626,7 @@ int dp_last_launch_info(dp_handle h, long* out6) {
 }
 
 const char* dp_last_error(void) { return g_err.c_str(); }
-const char* dp_version(void) { return "diffpose_b200 0.2 (sm_100a)"; }
+const char* dp_version(void) { return "diffpose_b200 0.3 (sm_100a)"; }
 int dp_device(dp_handle h) { return h ? h->device : DP_ERR_INVALID; }
 
 void dp_destroy(dp_handle h) { delete h; }

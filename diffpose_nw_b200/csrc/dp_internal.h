@@ -121,7 +121,7 @@ struct EngineCall {
   bool forward_only = false;
   // fused by tcg only
   bool mean_over_hyp = false;    // out is [n_pose, n_pts, c], the mean over each pose's hypotheses
-  const float* gt = nullptr;     // fused evaluation tail, see dp_sample_eval
+  const float* gt = nullptr;     // fused evaluation tail, see dp_sample's targets_xyz
   double* sums = nullptr;
   // fused by tcx only
   bool emit_uvxyz = false;       // forward of GCNpose: out is [n, n_pts, c_in + c_out] = [uv | xyz - xyz_root] (dp_lift)

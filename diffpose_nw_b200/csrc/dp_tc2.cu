@@ -130,7 +130,7 @@ struct Tc2Args {
   const float* noise;
   const unsigned char* mask;
   const dp_step* steps_dev;
-  const float* gt;           // fused evaluation (dp_sample_eval): targets [n_pose][17][3]; every finished pose (after the hypothesis
+  const float* gt;           // fused evaluation (dp_sample with targets_xyz): targets [n_pose][17][3]; every finished pose (after the hypothesis
   double* sums;              //   mean, if any) adds its MPJPE / P-MPJPE to sums[0..1] and 1 to sums[2] (common/loss.py, dp_metrics)
   long long* trace;          // optional diagnostic: CTA 0 records clock64() at every hand-over (see dp_set_trace)
   int trace_cap;
@@ -371,7 +371,7 @@ __device__ __forceinline__ __half* tall_elem(uint8_t* smem, int which, int trow,
 
 // ------------------------------------------------------------------------------------------------ the kernel
 // TRACE = true compiles the clock64() stamps of dp_set_trace in; the production instantiation carries none of it.
-// EVAL = true compiles the fused evaluation tail (dp_sample_eval) in: ~3 000 instructions that the plain sampler instantiation
+// EVAL = true compiles the fused evaluation tail (dp_sample with targets_xyz) in: ~3 000 instructions that the plain sampler instantiation
 // does not carry either.
 // KEYED = true draws z from the keyed stream (a.key, dp_philox.cuh) instead of reading a.noise; the unkeyed instantiations
 // carry none of the Philox code, so their schedule is the one they had before keyed noise existed.

@@ -13,6 +13,7 @@ import ctypes
 
 import torch
 
+from . import _lib
 from .metrics import pose_error_sums
 from .sampler import sample
 
@@ -28,7 +29,7 @@ def lift_and_refine(model_diff, x_uvxyz=None, *, model_pose=None, input_2d=None,
                     test_times=1, noise=None, targets=None, sums=None, seed=None, pose_offset=0):
     """Two-stage inference for one batch.  Give either `x_uvxyz` [B,17,5] or (`model_pose`, `input_2d` [B,17,2]).
     Returns the hypothesis-averaged uvxyz [B,17,5].  With `targets` [B,17,3] and `sums` (CUDA fp64 [3]) the MPJPE / P-MPJPE
-    partial sums of the batch are accumulated by the sampler launch itself (`dp_sample_eval`).  `seed` draws the noise in
+    partial sums of the batch are accumulated by the sampler launch itself (`dp_sample` with targets_xyz).  `seed` draws the noise in
     the kernel (keyed stream, see `sample`); `pose_offset` is the global index of the batch's first pose."""
     if x_uvxyz is None:
         # lift + out-of-place root-centring (SURVEY.md 8a quirk 4) + concat in ONE launch (dp_lift); the sampler below is
@@ -89,13 +90,12 @@ class HostStream:
     Results come back in submission order.  `depth` batches are in flight; every buffer is allocated once.  A returned
     tensor aliases a ring buffer and stays valid for the next `depth` submits.
 
-    eta > 0 needs `seed`: the kernel then draws the noise from the keyed stream (`dp_hstream_submit_keyed`), and the poses
+    eta > 0 needs `seed`: the kernel then draws the noise from the keyed stream (`dp_hstream_submit`'s key), and the poses
     of consecutive batches are numbered like one big call, so the results equal one `sample(seed=...)` over all batches.
     """
 
     def __init__(self, model_diff, batch, seq, betas, eta=0.0, test_times=1, src_mask=None, depth=3, device=None, seed=None):
         import collections
-        from . import _lib
         from .sampler import ddim_steps
         self.model = getattr(model_diff, "module", model_diff)
         self.dev = torch.device(device) if device is not None else self.model._device()
@@ -129,14 +129,13 @@ class HostStream:
         slot, hb, n = self._pending.popleft()[:3]
         rc = self._lib.dp_hstream_wait(self.hs, slot)
         if rc != 0:
-            from . import _lib
             _lib.check(rc, "dp_hstream_wait")
         return self.out_host[hb][:n]
 
     def submit(self, x_host, targets_host=None, sums=None, pose_offset=None):
         """Queue one pinned host batch [n<=B,17,c] (fp32, contiguous).  Returns the oldest finished result when the ring is
         full, else None.  With `targets_host` [n,17,3] (pinned fp32) and `sums` (CUDA fp64 [3]) the batch's MPJPE / P-MPJPE
-        partial sums are accumulated by the sampler launch itself (`dp_hstream_submit_eval`).  With a seed, `pose_offset`
+        partial sums are accumulated by the sampler launch itself (`dp_hstream_submit` with targets_host).  With a seed, `pose_offset`
         is the global index of the batch's first pose; it defaults to the number of poses submitted before."""
         n = x_host.shape[0]
         if n > self.B:
@@ -156,20 +155,11 @@ class HostStream:
                 raise RuntimeError(f"targets_host must be a contiguous fp32 HOST tensor [{n},17,3]")
             if sums is None or not sums.is_cuda or sums.dtype is not torch.float64 or sums.numel() != 3:
                 raise RuntimeError("fused evaluation needs `sums`: a CUDA float64 tensor of 3 elements")
-        if self._keyed:
-            from . import _lib
-            key = _lib.noise_key(self.seed, self.n_submitted if pose_offset is None else pose_offset)
-            rc = self._lib.dp_hstream_submit_keyed(self.hs, x_host.data_ptr(), None if targets_host is None else targets_host.data_ptr(),
-                                                   None if targets_host is None else sums.data_ptr(), n, self.steps, self.T,
-                                                   ctypes.byref(key), self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
-        elif targets_host is None:
-            rc = self._lib.dp_hstream_submit(self.hs, x_host.data_ptr(), n, self.steps, self.T, None, self._mask_ptr,
-                                             self.out_host[hb].data_ptr(), stream, self._slot_ref)
-        else:
-            rc = self._lib.dp_hstream_submit_eval(self.hs, x_host.data_ptr(), targets_host.data_ptr(), sums.data_ptr(), n, self.steps, self.T,
-                                                  None, self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
+        key = _lib.noise_key(self.seed, self.n_submitted if pose_offset is None else pose_offset) if self._keyed else None
+        rc = self._lib.dp_hstream_submit(self.hs, x_host.data_ptr(), None if targets_host is None else targets_host.data_ptr(),
+                                         None if targets_host is None else sums.data_ptr(), n, self.steps, self.T, None, key,
+                                         self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
         if rc != 0:
-            from . import _lib
             _lib.check(rc, "dp_hstream_submit")
         self._pending.append((self._slot.value, hb, n, x_host, targets_host))
         self.n_submitted += n

@@ -113,13 +113,13 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     x: [n_hyp*n_pose,17,c] hypothesis-major (what `.repeat(test_times,1,1)` produces), or [n_pose,17,c] with
     `repeat_input=True` to let the kernel read each pose n_hyp times instead of materialising the repeat.
     noise: optional [T, n_hyp*n_pose, 17, c] standard-normal draws replacing `torch.randn_like` (:65).
-    seed: draw the noise inside the kernel from the keyed stream (`dp_sample_keyed`, include/diffpose_b200.h) instead: one
+    seed: draw the noise inside the kernel from the keyed stream (`dp_sample`'s key, include/diffpose_b200.h) instead: one
     launch, no noise tensor, and every pose receives the same draws however the work is split, as long as each piece
     passes the global index of its first pose as `pose_offset` (and a call that runs step k of a schedule alone passes
     `step_offset=k`).  `philox_noise` writes the same stream out.  Not together with `noise`; no effect when eta = 0.
     Without `noise` and `seed`, eta > 0 draws with torch.randn, in chunks of at most NOISE_CHUNK_BYTES.
     mean_over_hyp: fuse `mean(reshape(n_hyp,-1,17,c),0)` (runners/diffpose_frame.py:382) after the loop.
-    targets, sums: fused evaluation (`dp_sample_eval`): targets [n_pose,17,3] on the device and a CUDA fp64 tensor of 3
+    targets, sums: fused evaluation (`dp_sample` with targets_xyz): targets [n_pose,17,3] on the device and a CUDA fp64 tensor of 3
     partial sums `[sum mpjpe, sum p_mpjpe, n]` that every finished pose is added to in the same launch (:384-387); with
     n_hyp > 1 this needs mean_over_hyp.  Without them nothing is evaluated.
     """
@@ -171,18 +171,10 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
             raise RuntimeError(f"targets must be [{n_pose},{m.n_pts},3], got {tuple(tg.shape)}")
 
     def launch(x_t, out_t, n_p, nz_t, repeated, lo=0):
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        if key is not None:
-            rc = lib.dp_sample_keyed(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
-                                     ctypes.byref(key), mask_ptr, 1 if mean_over_hyp else 0,
-                                     None if tg is None else tg.data_ptr(), None if tg is None else sums.data_ptr(), stream)
-        elif tg is None:
-            rc = lib.dp_sample(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
-                               nz_t.data_ptr() if nz_t is not None else None, mask_ptr, 1 if mean_over_hyp else 0, stream)
-        else:
-            rc = lib.dp_sample_eval(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
-                                    nz_t.data_ptr() if nz_t is not None else None, mask_ptr, 1 if mean_over_hyp else 0,
-                                    tg[lo:lo + n_p].data_ptr(), sums.data_ptr(), stream)
+        rc = lib.dp_sample(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
+                           nz_t.data_ptr() if nz_t is not None else None, key, mask_ptr, 1 if mean_over_hyp else 0,
+                           None if tg is None else tg[lo:lo + n_p].data_ptr(), None if tg is None else sums.data_ptr(),
+                           torch.cuda.current_stream(dev).cuda_stream)
         if rc != 0:
             _lib.check(rc, "dp_sample")
 

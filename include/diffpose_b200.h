@@ -120,32 +120,6 @@ int dp_forward(dp_handle h, const float* x, const float* t, const unsigned char*
  * in-place form leaves joints 1..16 unchanged on CPU and races on CUDA, SURVEY.md 8a quirk 4). */
 int dp_lift(dp_handle h, const float* uv, const unsigned char* mask, float* out_uvxyz, long n, void* stream);
 
-/* Replaces generalized_steps(x, src_mask, seq, model, b, eta=...) (common/utils_diff.py:46-67) plus the
- * hypothesis handling around it (runners/diffpose_frame.py:342 `.repeat(test_times,1,1)` and :382
- * `mean(reshape(test_times,-1,17,5),0)`), in ONE persistent launch for all T steps.
- *   x_in      [n_rows_in,n_pts,c] with n_rows_in = n_pose*n_hyp if x_is_repeated else n_pose
- *             (the library reads pose b for every hypothesis h when x_is_repeated = 0);
- *   x_out     [n_pose*n_hyp,n_pts,c] hypothesis-major (index h*n_pose+b) when mean_over_hyp = 0,
- *             [n_pose,n_pts,c] when mean_over_hyp = 1 (DP_ENGINE_TCG folds the mean into the kernel's final store:
- *             one launch, no [n_pose*n_hyp] intermediate);
- *   steps_host T entries in execution order (largest t first);
- *   noise     [T,n_pose*n_hyp,n_pts,c] host-drawn N(0,1) replacing randn_like (:65), or NULL (term skipped;
- *             exact when every c1 = 0, i.e. eta = 0);
- *   mask      as in dp_forward. */
-int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-              const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
-              int mean_over_hyp, void* stream);
-
-/* dp_sample followed by dp_metrics on its result, in ONE launch on DP_ENGINE_TCG: the body of the evaluation loop
- * (runners/diffpose_frame.py:365-387: generalized_steps, hypothesis mean, root-centring, mpjpe, p_mpjpe).  Every pose the
- * kernel finishes (after the hypothesis mean when n_hyp > 1, which then requires mean_over_hyp = 1) adds its MPJPE to sums[0],
- * its P-MPJPE to sums[1] and 1 to sums[2] from the tile it was computed in -- one warp per pose in the tile's tail, one atomic
- * per CTA -- instead of a second kernel re-reading x_out.  targets_xyz [n_pose,n_pts,3], sums: 3 doubles on the device
- * (accumulated into; the caller zeroes them).  Other engines run dp_sample and dp_metrics back to back. */
-int dp_sample_eval(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                   const dp_step* steps_host, int n_steps, const float* noise, const unsigned char* mask,
-                   int mean_over_hyp, const float* targets_xyz, double* sums, void* stream);
-
 /* Keyed noise: the sampler kernels draw z themselves from a counter-based stream, so a call needs no noise tensor and the
  * value every (pose, hypothesis, step, element) receives does not depend on how the work is split into calls, batches,
  * tiles or ranks.  The stream (this definition is part of the ABI):
@@ -169,16 +143,35 @@ typedef struct dp_noise_key {
   int step_offset;
 } dp_noise_key;
 
-/* dp_sample (targets_xyz = NULL) or dp_sample_eval (targets_xyz and sums given) with the keyed stream in place of the noise
- * tensor: one launch, no [T, n_pose*n_hyp, n_pts, c] buffer.  Same engines, layouts and graph-capture rules as dp_sample;
- * the key travels by value in the kernel arguments.  When every c1 = 0 (eta = 0) the key has no effect. */
-int dp_sample_keyed(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                    const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask,
-                    int mean_over_hyp, const float* targets_xyz, double* sums, void* stream);
+/* Replaces generalized_steps(x, src_mask, seq, model, b, eta=...) (common/utils_diff.py:46-67) plus the
+ * hypothesis handling around it (runners/diffpose_frame.py:342 `.repeat(test_times,1,1)` and :382
+ * `mean(reshape(test_times,-1,17,5),0)`), in ONE persistent launch for all T steps.
+ *   x_in      [n_rows_in,n_pts,c] with n_rows_in = n_pose*n_hyp if x_is_repeated else n_pose
+ *             (the library reads pose b for every hypothesis h when x_is_repeated = 0);
+ *   x_out     [n_pose*n_hyp,n_pts,c] hypothesis-major (index h*n_pose+b) when mean_over_hyp = 0,
+ *             [n_pose,n_pts,c] when mean_over_hyp = 1 (DP_ENGINE_TCG folds the mean into the kernel's final store:
+ *             one launch, no [n_pose*n_hyp] intermediate);
+ *   steps_host T entries in execution order (largest t first);
+ *   noise     [T,n_pose*n_hyp,n_pts,c] host-drawn N(0,1) replacing randn_like (:65), or NULL;
+ *   key       the keyed stream above in place of a noise tensor, or NULL: no [T,n_pose*n_hyp,n_pts,c] buffer, and the
+ *             key travels by value in the kernel arguments.  Not together with noise (DP_ERR_INVALID).  With neither,
+ *             the noise term is skipped (exact when every c1 = 0, i.e. eta = 0); when every c1 = 0 a key has no effect;
+ *   mask      as in dp_forward;
+ *   targets_xyz, sums  NULL, or the fused evaluation: dp_metrics on the result, in the same launch on DP_ENGINE_TCG -- the
+ *             body of the evaluation loop (runners/diffpose_frame.py:365-387: generalized_steps, hypothesis mean,
+ *             root-centring, mpjpe, p_mpjpe).  Every pose the kernel finishes (after the hypothesis mean when n_hyp > 1,
+ *             which then requires mean_over_hyp = 1) adds its MPJPE to sums[0], its P-MPJPE to sums[1] and 1 to sums[2]
+ *             from the tile it was computed in -- one warp per pose in the tile's tail, one atomic per CTA -- instead of a
+ *             second kernel re-reading x_out.  targets_xyz [n_pose,n_pts,3], sums: 3 doubles on the device (accumulated
+ *             into; the caller zeroes them); targets_xyz requires sums.  Other engines run the sampler and dp_metrics
+ *             back to back. */
+int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+              const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+              int mean_over_hyp, const float* targets_xyz, double* sums, void* stream);
 
 /* Writes the keyed stream as out [n_steps][n_hyp*n_pose][n_pts][c] (hypothesis-major: row h*n_pose + p is pose
  * pose_offset + p, hypothesis h; step k is s = step_offset + k) -- the layout of dp_sample's `noise`.  So
- * dp_sample(noise = out) equals dp_sample_keyed(key) bit for bit. */
+ * dp_sample(noise = out) equals dp_sample(key) bit for bit. */
 int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, int n_pts, int c, float* out, void* stream);
 
 /* Batches that live in HOST memory.  Replaces the copy-in / sample / copy-out sequence of the evaluation loop
@@ -190,26 +183,21 @@ int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, 
  *            happens here, none per batch;
  *   submit : x_host [n_pose,n_pts,c] and out_host ([n_pose*n_hyp,...] or [n_pose,...] with the mean) should be PINNED
  *            host memory (pageable memory works but serialises); enqueues copy-in, dp_sample on `stream`, copy-out and
- *            returns immediately; *slot identifies the batch.  noise_dev / mask_dev as in dp_sample (device, optional).
+ *            returns immediately; *slot identifies the batch.  noise_dev, key and mask_dev as in dp_sample (noise_dev and
+ *            mask_dev on the device; each optional, noise_dev and key not both).  key->pose_offset numbers the batch's
+ *            first pose: giving each batch the count of poses submitted before it draws what one keyed dp_sample over
+ *            all batches would.  With targets_host [n_pose,n_pts,3] (pinned; requires sums_dev, 3 doubles on the device)
+ *            the evaluation is fused in as in dp_sample: the targets travel with the batch and the kernel adds the batch's
+ *            MPJPE / P-MPJPE sums to sums_dev -- the whole body of the evaluation loop (runners/diffpose_frame.py:333-387)
+ *            per batch: two H2D copies, one launch, one D2H copy.  A refused combination enqueues nothing.
  *            A slot is reused after `depth` submits: wait for its result before that.
  *   wait   : blocks the host until the result of `slot` is in its out_host.
  * Results complete in submission order. */
 typedef struct dp_hstream* dp_hstream_t;
 int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, int mean_over_hyp, int depth);
-int dp_hstream_submit(dp_hstream_t s, const float* x_host, long n_pose, const dp_step* steps_host, int n_steps, const float* noise_dev,
+int dp_hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
+                      const dp_step* steps_host, int n_steps, const float* noise_dev, const dp_noise_key* key,
                       const unsigned char* mask_dev, float* out_host, void* stream, int* slot);
-/* The same with the evaluation fused in (dp_sample_eval): targets_host [n_pose,n_pts,3] (pinned) travels with the batch, the
- * kernel adds the batch's MPJPE / P-MPJPE sums to sums_dev (3 doubles on the device) -- the whole body of the evaluation
- * loop (runners/diffpose_frame.py:333-387) per batch: two H2D copies, one launch, one D2H copy. */
-int dp_hstream_submit_eval(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
-                           const dp_step* steps_host, int n_steps, const float* noise_dev, const unsigned char* mask_dev, float* out_host,
-                           void* stream, int* slot);
-/* dp_hstream_submit (targets_host = NULL) or dp_hstream_submit_eval with keyed noise (dp_sample_keyed) instead of a
- * noise tensor: an eta > 0 schedule through the ring.  key->pose_offset numbers the batch's first pose; giving each batch
- * the count of poses submitted before it draws what one dp_sample_keyed over all batches would. */
-int dp_hstream_submit_keyed(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
-                            const dp_step* steps_host, int n_steps, const dp_noise_key* key, const unsigned char* mask_dev,
-                            float* out_host, void* stream, int* slot);
 int dp_hstream_wait(dp_hstream_t s, int slot);
 void dp_hstream_destroy(dp_hstream_t s);
 

@@ -1,4 +1,4 @@
-"""GPU (-m gpu): keyed in-kernel noise (dp_sample_keyed, dp_hstream_submit_keyed, dp_noise_fill).
+"""GPU (-m gpu): keyed in-kernel noise (the key of dp_sample and dp_hstream_submit, dp_noise_fill).
 
 dp_noise_fill is checked against the numpy restatement (oracle/philox.py).  Every keyed call is then checked bit for bit
 against the same call fed dp_noise_fill's tensor through `noise=`, which carries the oracle parity of the noise path
@@ -200,6 +200,67 @@ def test_host_stream_keyed_equals_one_call(with_targets):
     assert torch.equal(torch.cat(got), want)
     if with_targets:
         np.testing.assert_allclose(sums.cpu().numpy(), s_want.cpu().numpy(), rtol=1e-12)
+
+
+# ------------------------------------------------------------------------------------- refused argument combinations
+def test_refused_combinations_leave_handle_and_ring_usable():
+    """dp_sample and dp_hstream_submit take every option as an argument, so a caller can pass combinations they refuse:
+    noise and key together, targets without sums, and (ring) targets with n_hyp > 1 but no mean.  Each returns
+    DP_ERR_INVALID without enqueueing anything; the next valid call on the same handle and ring gives the expected result."""
+    lib = _lib.load()
+    m = _model("tcg")
+    n, seq, seed = 40, [0, 12], 7
+    x = _poses(n, 12)
+    tg = O.synthetic_targets(x.cpu(), seed=13).to(DEV)
+    want = D.sample(m, x, None, seq, betas(), eta=1.0, seed=seed)
+    want_sums, _ = D.pose_error_sums(want, tg)
+    steps = D.ddim_steps(betas(), seq, 1.0)
+    T, h, key = len(steps), m._handle, _lib.noise_key(seed)
+    nz = D.philox_noise(seed, T, n, device=DEV)
+    stream = torch.cuda.current_stream(DEV).cuda_stream
+    out = torch.zeros_like(x)
+    sums = torch.zeros(3, device=DEV, dtype=torch.float64)
+
+    def sample(noise, targets, sums_ptr):
+        return lib.dp_sample(h, x.data_ptr(), 1, out.data_ptr(), n, 1, steps, T, noise, key, None, 0, targets, sums_ptr, stream)
+
+    assert sample(nz.data_ptr(), None, None) == -1 and b"dp_sample: " in lib.dp_last_error() and b"not both" in lib.dp_last_error()
+    assert sample(None, tg.data_ptr(), None) == -1 and b"dp_sample: " in lib.dp_last_error()
+    torch.cuda.synchronize()
+    assert out.abs().max().item() == 0
+    assert sample(None, tg.data_ptr(), sums.data_ptr()) == 0
+    torch.cuda.synchronize()
+    assert torch.equal(out, want)
+    np.testing.assert_allclose(sums.cpu().numpy(), want_sums.cpu().numpy(), rtol=1e-12)
+
+    xh, th = x.cpu().pin_memory(), tg.cpu().pin_memory()
+    oh = torch.zeros(n, 17, 5).pin_memory()
+    slot = ctypes.c_int(-1)
+    rings = [ctypes.c_void_p(), ctypes.c_void_p()]
+    try:
+        assert lib.dp_hstream_create(ctypes.byref(rings[0]), h, 64, 1, 0, 2) == 0
+        assert lib.dp_hstream_create(ctypes.byref(rings[1]), h, 64, 2, 0, 2) == 0     # two hypotheses, no mean
+
+        def submit(ring, noise, targets, sums_ptr):
+            return lib.dp_hstream_submit(ring, xh.data_ptr(), targets, sums_ptr, n, steps, T, noise, key, None, oh.data_ptr(),
+                                         stream, ctypes.byref(slot))
+
+        assert submit(rings[0], nz.data_ptr(), None, None) == -1
+        assert b"dp_hstream_submit: " in lib.dp_last_error() and b"not both" in lib.dp_last_error()
+        assert submit(rings[0], None, th.data_ptr(), None) == -1 and b"dp_hstream_submit: " in lib.dp_last_error()
+        assert submit(rings[1], None, th.data_ptr(), sums.data_ptr()) == -1 and b"mean_over_hyp" in lib.dp_last_error()
+        assert slot.value == -1
+        sums.zero_()
+        assert submit(rings[0], None, th.data_ptr(), sums.data_ptr()) == 0
+        assert slot.value == 0                     # the refused submits did not take a slot
+        assert lib.dp_hstream_wait(rings[0], slot.value) == 0
+        torch.cuda.synchronize()
+        assert torch.equal(oh, want.cpu())
+        np.testing.assert_allclose(sums.cpu().numpy(), want_sums.cpu().numpy(), rtol=1e-12)
+    finally:
+        for r in rings:
+            if r.value:
+                lib.dp_hstream_destroy(r)
 
 
 # ------------------------------------------------------------------------------------- per-step launches, determinism

@@ -193,8 +193,8 @@ def test_second_device_in_one_process():
 @pytest.mark.parametrize("engine", ["auto", "fp32"])
 @pytest.mark.parametrize("n,Hh", [(1, 1), (37, 1), (300, 1), (23, 5), (150, 3), (9, 10)])
 def test_fused_evaluation_equals_sampler_then_metrics(engine, n, Hh):
-    """dp_sample_eval (sampler + MPJPE / P-MPJPE partial sums in one launch on the default engine; one warp per finished pose
-    in the tile's tail) accumulates exactly what dp_sample followed by dp_metrics does -- ragged batches, several tiles per
+    """dp_sample with targets_xyz (sampler + MPJPE / P-MPJPE partial sums in one launch on the default engine; one warp per
+    finished pose in the tile's tail) accumulates exactly what dp_sample followed by dp_metrics does -- ragged batches, several tiles per
     CTA, hypothesis mean (poses completing across tile boundaries, H larger than a tile), accumulation over calls."""
     dev = torch.device("cuda:0")
     adj, diff, sd_d, _, _ = _models()

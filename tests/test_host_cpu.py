@@ -125,6 +125,9 @@ def test_abi_library_exports_header_symbols():
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in declared:
         assert hasattr(lib, name), f"{name} missing from libdiffpose_b200.so"
+    # one entry point per function, every option an argument: the former per-combination variants are not exported
+    for name in [f"dp_{fn}_{opt}" for fn in ("sample", "hstream_submit") for opt in ("eval", "keyed")]:
+        assert not hasattr(lib, name), f"{name} is still exported"
     lib.dp_version.restype = ctypes.c_char_p
     assert b"sm_100a" in lib.dp_version()
     assert ctypes.sizeof(_lib.DpStep) == 24

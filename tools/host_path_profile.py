@@ -50,7 +50,7 @@ xp, op = x.data_ptr(), out.data_ptr()
 
 
 def raw():
-    lib.dp_sample(model._handle, xp, 0, op, 1024, 1, steps, 2, None, None, 0, stream)
+    lib.dp_sample(model._handle, xp, 0, op, 1024, 1, steps, 2, None, None, None, 0, None, None, stream)
 
 
 torch.cuda.synchronize()
