@@ -46,13 +46,17 @@ SIGNATURES = {
     "dp_lift": (_I, [_P, _P, _P, _P, _L, _P]),
     "dp_forward": (_I, [_P, _P, _P, _P, _P, _L, _P]),
     "dp_sample": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _P]),
+    "dp_sample_grouped": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _I, _P,
+                               _P]),
     "dp_noise_fill": (_I, [ctypes.POINTER(DpNoiseKey), _I, _L, _I, _I, _I, _P, _P]),
     "dp_hstream_create": (_I, [ctypes.POINTER(_P), _P, _L, _I, _I, _I]),
     "dp_hstream_submit": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _P, _P,
                                ctypes.POINTER(_I)]),
+    "dp_hstream_submit_grouped": (_I, [_P, _P, _P, _P, _I, _P, _L, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _P,
+                                       _P, ctypes.POINTER(_I)]),
     "dp_hstream_wait": (_I, [_P, _I]),
     "dp_hstream_destroy": (None, [_P]),
-    "dp_metrics": (_I, [_P, _I, _I, _P, _L, _I, _P, _P, _P]),
+    "dp_metrics": (_I, [_P, _I, _I, _P, _L, _I, _P, _I, _P, _P, _P]),
     "dp_selftest_umma": (_I, [_P, _I, _P, _I, _P, _I, _P]),
     "dp_selftest_umma_ts": (_I, [_P, _I, _P, _I, _I, _P, _I, _P, _I, _P]),
     "dp_selftest_cycles": (_I, [ctypes.POINTER(ctypes.c_longlong)]),

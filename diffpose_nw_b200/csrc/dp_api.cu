@@ -400,10 +400,19 @@ static int make_key(const dp_noise_key* k, long n_pose, const char* what, NoiseK
 int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
               const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
               int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
+  return dp_sample_grouped(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, key, mask, mean_over_hyp, targets_xyz,
+                           nullptr, 1, sums, stream);
+}
+
+int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                      const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+                      int mean_over_hyp, const float* targets_xyz, const int* group, int n_groups, double* sums, void* stream) {
   DP_REQUIRE(h && x_in && x_out && steps_host, "dp_sample: NULL argument");
   DP_REQUIRE(n_pose >= 0 && n_hyp >= 1 && n_steps >= 1, "dp_sample: n_pose >= 0, n_hyp >= 1, n_steps >= 1 required");
   DP_REQUIRE(h->d.has_temb, "dp_sample: handle was created with has_temb = 0 (GCNpose has no sampler)");
   DP_REQUIRE(!(noise && key), "dp_sample: give either a noise tensor or a noise key, not both");
+  DP_REQUIRE(!group || targets_xyz, "dp_sample: group ids need targets_xyz");
+  DP_REQUIRE(!group || n_groups >= 1, "dp_sample: group ids need n_groups >= 1");
   if (targets_xyz != nullptr) {
     DP_REQUIRE(sums != nullptr, "dp_sample: targets_xyz needs sums");
     DP_REQUIRE(h->d.c_out >= 3, "dp_sample: the model's output needs at least the three xyz coordinates");
@@ -461,7 +470,7 @@ int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, l
   // default engine: the hypothesis mean -- and, with targets_xyz, the MPJPE / P-MPJPE sums -- are fused into the kernel's
   // final store (one launch, no [H*B] scratch)
   if (eng == DP_ENGINE_TCG) {
-    c.mean_over_hyp = mean; c.gt = targets_xyz; c.sums = sums;
+    c.mean_over_hyp = mean; c.gt = targets_xyz; c.group = group; c.n_groups = n_groups; c.sums = sums;
     return tc2_run(h, c, s);
   }
   const int row_floats = d.n_pts * d.c_out;
@@ -471,7 +480,7 @@ int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, l
   }
   DP_TRY(run_engine(h, eng, c, s));
   if (mean) DP_TRY(hyp_mean_launch(c.out, x_out, n_pose, n_hyp, row_floats, s));
-  if (targets_xyz != nullptr) DP_TRY(metrics_launch(x_out, d.c_out, d.c_out - 3, targets_xyz, n_pose, d.n_pts, sums, nullptr, s));
+  if (targets_xyz != nullptr) DP_TRY(metrics_launch(x_out, d.c_out, d.c_out - 3, targets_xyz, n_pose, d.n_pts, group, n_groups, sums, nullptr, s));
   return DP_OK;
 }
 
@@ -486,12 +495,13 @@ int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, 
 }
 
 int dp_metrics(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
-               double* sums, float* per_pose, void* stream) {
+               const int* group, int n_groups, double* sums, float* per_pose, void* stream) {
   DP_REQUIRE(pred && gt && sums, "dp_metrics: NULL argument");
   DP_REQUIRE(n_pts == kMaxPts, "dp_metrics: n_pts must be 17");
   DP_REQUIRE(pred_stride >= 3 && pred_offset >= 0 && pred_offset + 3 <= pred_stride, "dp_metrics: bad pred stride/offset");
+  DP_REQUIRE(!group || n_groups >= 1, "dp_metrics: group ids need n_groups >= 1");
   if (n <= 0) return n == 0 ? DP_OK : DP_ERR_INVALID;
-  return metrics_launch(pred, pred_stride, pred_offset, gt, n, n_pts, sums, per_pose, static_cast<cudaStream_t>(stream));
+  return metrics_launch(pred, pred_stride, pred_offset, gt, n, n_pts, group, n_groups, sums, per_pose, static_cast<cudaStream_t>(stream));
 }
 
 int dp_selftest_umma(const void* smem_image, int image_bytes, const dp_mma_op* ops_host, int n_ops, float* tmem_out, int ncols,
@@ -527,7 +537,8 @@ struct dp_hstream {
   int n_hyp = 1, mean = 0, depth = 0, head = 0;
   size_t in_floats = 0, out_floats = 0;
   cudaStream_t s_in = nullptr, s_out = nullptr;
-  DevBuf x_dev[16], out_dev[16], gt_dev[16];       // per slot (depth <= 16): input, result, and (evaluation) the targets of the batch
+  DevBuf x_dev[16], out_dev[16], gt_dev[16], grp_dev[16];   // per slot (depth <= 16): input, result, and (evaluation) the targets and
+                                                           // group ids of the batch
   std::vector<cudaEvent_t> ev_in, ev_done, ev_out;
 };
 
@@ -548,7 +559,7 @@ int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, 
   for (int i = 0; i < depth && e == cudaSuccess; ++i) {
     cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
     if (s->x_dev[i].reserve(s->in_floats * sizeof(float)) != DP_OK || s->out_dev[i].reserve(s->out_floats * sizeof(float)) != DP_OK ||
-        s->gt_dev[i].reserve((size_t)max_pose * h->d.n_pts * 3 * sizeof(float)) != DP_OK)
+        s->gt_dev[i].reserve((size_t)max_pose * h->d.n_pts * 3 * sizeof(float)) != DP_OK || s->grp_dev[i].reserve((size_t)max_pose * sizeof(int)) != DP_OK)
       e = cudaErrorMemoryAllocation;
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&e0, cudaEventDisableTiming);
     if (e == cudaSuccess) { s->ev_in.push_back(e0); e = cudaEventCreateWithFlags(&e1, cudaEventDisableTiming); }
@@ -567,12 +578,21 @@ int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, 
 int dp_hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose, const dp_step* steps_host,
                       int n_steps, const float* noise_dev, const dp_noise_key* key, const unsigned char* mask_dev, float* out_host,
                       void* stream, int* slot_out) {
+  return dp_hstream_submit_grouped(s, x_host, targets_host, nullptr, 1, sums_dev, n_pose, steps_host, n_steps, noise_dev, key, mask_dev,
+                                   out_host, stream, slot_out);
+}
+
+int dp_hstream_submit_grouped(dp_hstream_t s, const float* x_host, const float* targets_host, const int* groups_host, int n_groups,
+                              double* sums_dev, long n_pose, const dp_step* steps_host, int n_steps, const float* noise_dev,
+                              const dp_noise_key* key, const unsigned char* mask_dev, float* out_host, void* stream, int* slot_out) {
   DP_REQUIRE(s && x_host && out_host && steps_host && slot_out, "dp_hstream_submit: NULL argument");
   DP_REQUIRE(n_pose >= 1 && n_pose <= s->max_pose, "dp_hstream_submit: batch exceeds the max_pose this stream was created for");
   // the combinations dp_sample refuses, refused before the copies below are enqueued
   DP_REQUIRE(!(noise_dev && key), "dp_hstream_submit: give either a noise tensor or a noise key, not both");
   DP_REQUIRE(!targets_host || (sums_dev && (s->n_hyp == 1 || s->mean)),
              "dp_hstream_submit: targets_host needs sums_dev and, with n_hyp > 1, a stream created with mean_over_hyp");
+  DP_REQUIRE(!groups_host || targets_host, "dp_hstream_submit: groups_host needs targets_host");
+  DP_REQUIRE(!groups_host || n_groups >= 1, "dp_hstream_submit: groups_host needs n_groups >= 1");
   DP_TRY(check_device(s->h, "dp_hstream_submit"));
   cudaStream_t cs = static_cast<cudaStream_t>(stream);
   const int k = s->head;
@@ -583,12 +603,15 @@ int dp_hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_
   DP_CUDA(cudaMemcpyAsync(s->x_dev[k].get<float>(), x_host, in_bytes, cudaMemcpyHostToDevice, s->s_in));
   if (targets_host != nullptr)
     DP_CUDA(cudaMemcpyAsync(s->gt_dev[k].get<float>(), targets_host, (size_t)n_pose * s->h->d.n_pts * 3 * sizeof(float), cudaMemcpyHostToDevice, s->s_in));
+  if (groups_host != nullptr)
+    DP_CUDA(cudaMemcpyAsync(s->grp_dev[k].get<int>(), groups_host, (size_t)n_pose * sizeof(int), cudaMemcpyHostToDevice, s->s_in));
   DP_CUDA(cudaEventRecord(s->ev_in[k], s->s_in));
   // the sampler on the caller's stream, once the input is there and the slot's previous result has left the device
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_in[k], 0));
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_out[k], 0));
-  DP_TRY(dp_sample(s->h, s->x_dev[k].get<float>(), 0, s->out_dev[k].get<float>(), n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key,
-                   mask_dev, s->mean, targets_host != nullptr ? s->gt_dev[k].get<float>() : nullptr, sums_dev, stream));
+  DP_TRY(dp_sample_grouped(s->h, s->x_dev[k].get<float>(), 0, s->out_dev[k].get<float>(), n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key,
+                           mask_dev, s->mean, targets_host != nullptr ? s->gt_dev[k].get<float>() : nullptr,
+                           groups_host != nullptr ? s->grp_dev[k].get<int>() : nullptr, n_groups, sums_dev, stream));
   DP_CUDA(cudaEventRecord(s->ev_done[k], cs));
   // D2H on the copy-out stream
   DP_CUDA(cudaStreamWaitEvent(s->s_out, s->ev_done[k], 0));
@@ -626,7 +649,7 @@ int dp_last_launch_info(dp_handle h, long* out6) {
 }
 
 const char* dp_last_error(void) { return g_err.c_str(); }
-const char* dp_version(void) { return "diffpose_b200 0.3 (sm_100a)"; }
+const char* dp_version(void) { return "diffpose_b200 0.4 (sm_100a)"; }
 int dp_device(dp_handle h) { return h ? h->device : DP_ERR_INVALID; }
 
 void dp_destroy(dp_handle h) { delete h; }

@@ -122,6 +122,8 @@ struct EngineCall {
   // fused by tcg only
   bool mean_over_hyp = false;    // out is [n_pose, n_pts, c], the mean over each pose's hypotheses
   const float* gt = nullptr;     // fused evaluation tail, see dp_sample's targets_xyz
+  const int* group = nullptr;    //   and dp_sample_grouped's group ids: sums is then [n_groups][3]
+  int n_groups = 1;
   double* sums = nullptr;
   // fused by tcx only
   bool emit_uvxyz = false;       // forward of GCNpose: out is [n, n_pts, c_in + c_out] = [uv | xyz - xyz_root] (dp_lift)
@@ -194,8 +196,9 @@ int tc2_pack(dp_model* m, cudaStream_t s);
 // after simt_temb filled m->temb for a sampler schedule: the same embeddings as GC2 bias blocks of the tcg engine
 int tc2_tau(dp_model* m, int n_steps, cudaStream_t s);
 // dp_metrics.cu
+// group != NULL: pose i adds to sums[3 * group[i] ..] of [n_groups][3], and nothing when group[i] is outside [0, n_groups)
 int metrics_launch(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
-                   double* sums, float* per_pose, cudaStream_t s);
+                   const int* group, int n_groups, double* sums, float* per_pose, cudaStream_t s);
 int hyp_mean_launch(const float* x, float* out, long n_pose, int n_hyp, int row_floats, cudaStream_t s);
 // out[n][n_pts][c_in + c_out] = [uv | xyz - xyz[root]] (runners/diffpose_frame.py:337-343 with out-of-place root-centring)
 int lift_glue_launch(const float* uv, const float* xyz, float* out, long n, int n_pts, int c_in, int c_out, cudaStream_t s);

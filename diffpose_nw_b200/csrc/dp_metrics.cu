@@ -61,6 +61,43 @@ __global__ void __launch_bounds__(kMetricWarps * 32) metrics_kernel(const float*
   }
 }
 
+// The same per pose, keyed by group (dp_metrics / dp_sample_grouped with group ids): pose i adds to row group[i] of sums
+// [n_groups][3], and to nothing when the id is outside [0, n_groups).  Each warp carries the sums of its current run of
+// equal ids in registers and flushes them with three atomics when the id changes and after its last pose: a batch that
+// comes in runs of one action (as the reference's loader delivers them) costs about as many atomics as metrics_kernel.
+__global__ void __launch_bounds__(kMetricWarps * 32, 2) metrics_grouped_kernel(const float* __restrict__ pred, int ps, int po, const float* __restrict__ gt,
+                                                                            long n, const int* __restrict__ group, int n_groups,
+                                                                            double* __restrict__ sums, float* __restrict__ per_pose) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  asm volatile("griddepcontrol.wait;" ::: "memory");            // as in metrics_kernel
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  double e1s = 0.0, e2s = 0.0, cnt = 0.0;      // the current run's partial sums (identical on every lane)
+  int run = -1;                                 // and its id
+  for (long i = (long)blockIdx.x * kMetricWarps + warp; i < n; i += (long)gridDim.x * kMetricWarps) {
+    const int gi = __ldg(group + i);
+    const int j = lane < NP ? lane : 0;
+    const float* p = pred + (size_t)i * NP * ps + po + j * ps;
+    const float* g = gt + (size_t)i * NP * 3 + j * 3;
+    float pv[3], gv[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) { pv[c] = p[c]; gv[c] = g[c]; }
+    float e1f, e2f;
+    metric::pose_errors(pv, gv, lane, e1f, e2f);
+    if (gi != run) {
+      if (lane == 0 && cnt != 0.0 && (unsigned)run < (unsigned)n_groups) {
+        atomicAdd(sums + 3 * run, e1s); atomicAdd(sums + 3 * run + 1, e2s); atomicAdd(sums + 3 * run + 2, cnt);
+      }
+      run = gi; e1s = e2s = cnt = 0.0;
+    }
+    const double e1 = (double)e1f, e2 = (double)e2f;
+    e1s += e1; e2s += e2; cnt += 1.0;
+    if (per_pose && lane == 0) { per_pose[2 * i] = (float)e1; per_pose[2 * i + 1] = (float)e2; }
+  }
+  if (lane == 0 && cnt != 0.0 && (unsigned)run < (unsigned)n_groups) {
+    atomicAdd(sums + 3 * run, e1s); atomicAdd(sums + 3 * run + 1, e2s); atomicAdd(sums + 3 * run + 2, cnt);
+  }
+}
+
 // [uv | xyz - xyz[root]]: the glue between the lifter and the sampler for the engines whose forward kernel does not
 // write it directly (runners/diffpose_frame.py:337-343 with the intended out-of-place root-centring)
 __global__ void lift_glue_kernel(const float* __restrict__ uv, const float* __restrict__ xyz, float* __restrict__ out, long n, int n_pts,
@@ -78,7 +115,7 @@ __global__ void lift_glue_kernel(const float* __restrict__ uv, const float* __re
 }  // namespace
 
 int metrics_launch(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
-                   double* sums, float* per_pose, cudaStream_t s) {
+                   const int* group, int n_groups, double* sums, float* per_pose, cudaStream_t s) {
   (void)n_pts;
   long grid = (n + kMetricWarps - 1) / kMetricWarps;
   if (grid > 148 * 8) grid = 148 * 8;
@@ -88,7 +125,8 @@ int metrics_launch(const float* pred, int pred_stride, int pred_offset, const fl
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  DP_CUDA(cudaLaunchKernelEx(&cfg, metrics_kernel, pred, pred_stride, pred_offset, gt, n, sums, per_pose));
+  if (group != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, metrics_grouped_kernel, pred, pred_stride, pred_offset, gt, n, group, n_groups, sums, per_pose));
+  else DP_CUDA(cudaLaunchKernelEx(&cfg, metrics_kernel, pred, pred_stride, pred_offset, gt, n, sums, per_pose));
   count_launch();
   DP_CUDA(cudaGetLastError());
   return DP_OK;

@@ -131,7 +131,8 @@ struct Tc2Args {
   const unsigned char* mask;
   const dp_step* steps_dev;
   const float* gt;           // fused evaluation (dp_sample with targets_xyz): targets [n_pose][17][3]; every finished pose (after the hypothesis
-  double* sums;              //   mean, if any) adds its MPJPE / P-MPJPE to sums[0..1] and 1 to sums[2] (common/loss.py, dp_metrics)
+  double* sums;              //   mean, if any) adds its MPJPE / P-MPJPE to sums[0..1] and 1 to sums[2] (common/loss.py, dp_metrics), or to
+                             //   row group[b] of sums [n_groups][3] in the GROUPED instantiations (group, n_groups: kernel arguments)
   long long* trace;          // optional diagnostic: CTA 0 records clock64() at every hand-over (see dp_set_trace)
   int trace_cap;
   NoiseKey key;              // key.on: z from the keyed stream instead of noise (NULL); runs the KEYED instantiation
@@ -375,8 +376,12 @@ __device__ __forceinline__ __half* tall_elem(uint8_t* smem, int which, int trow,
 // does not carry either.
 // KEYED = true draws z from the keyed stream (a.key, dp_philox.cuh) instead of reading a.noise; the unkeyed instantiations
 // carry none of the Philox code, so their schedule is the one they had before keyed noise existed.
-template <bool TRACE, bool EVAL, bool KEYED>
-__global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg inl) {
+// GROUPED = true (with EVAL only) adds each finished pose to row group[b] of a.sums [n_groups][3] (dp_sample_grouped): every
+// compute warp carries the sums of its current run of equal ids in registers across tiles and flushes them with three
+// atomics when the id changes and after its last tile.  The ids come after the by-value arguments, so the instantiations
+// without GROUPED read their arguments at the offsets they always had.
+template <bool TRACE, bool EVAL, bool KEYED, bool GROUPED>
+__global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg inl, const int* __restrict__ group, int n_groups) {
   auto signal_ready = [](Ctx& c) { signal_ready_t<TRACE>(c); };
   auto signal_ready_tmem = [](Ctx& c) { signal_ready_t<TRACE, false>(c); };
   auto wait_acc = [](Ctx& c) { wait_acc_t<TRACE>(c); };
@@ -743,6 +748,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
 
     float macc = 0.f;     // mean_over_hyp: running hypothesis sum of output element `tid` of the pose being completed
     double ev1 = 0.0, ev2 = 0.0, evn = 0.0;   // fused evaluation: this warp's partial sums (the same on every lane)
+    int ev_run = -1, ev_id = -1;              // GROUPED: the id of those sums, the id of the pose this warp evaluates in this tile
     for (int it = 0; it < my_tiles; ++it) {
       const long g0 = a.mean_over_hyp ? row_lo + (long)it * TP : ((long)blockIdx.x + (long)it * gridDim.x) * TP;
       const int npose = (int)min((long)TP, (a.mean_over_hyp ? row_hi : a.n_rows) - g0);
@@ -776,6 +782,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
           const long g = g0 + p;
           const long b = a.mean_over_hyp ? g / a.n_hyp : g % a.n_pose;
           if (!a.mean_over_hyp || g - b * a.n_hyp == a.n_hyp - 1) evg[idx] = __ldg(a.gt + b * (NP * 3) + (idx - p * (NP * 3)));
+        }
+        if (GROUPED) {    // the tail gives the k-th pose finished in this tile to warp k: its id is requested now as well
+          const int p = a.mean_over_hyp ? (int)(a.n_hyp - 1 - g0 % a.n_hyp) + warp * a.n_hyp : warp;
+          if (p < npose) ev_id = __ldg(group + (a.mean_over_hyp ? (g0 + p) / a.n_hyp : (g0 + p) % a.n_pose));
         }
       }
       bar_compute();
@@ -1048,6 +1058,12 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
             for (int cc = 0; cc < 3; ++cc) { pv[cc] = evp[p * (NP * 3) + j * 3 + cc]; gv[cc] = evp[EV_FLOATS + p * (NP * 3) + j * 3 + cc]; }
             float e1, e2;
             metric::pose_errors(pv, gv, lane, e1, e2);
+            if (GROUPED && ev_id != ev_run) {
+              if (lane == 0 && evn != 0.0 && (unsigned)ev_run < (unsigned)n_groups) {
+                atomicAdd(a.sums + 3 * ev_run, ev1); atomicAdd(a.sums + 3 * ev_run + 1, ev2); atomicAdd(a.sums + 3 * ev_run + 2, evn);
+              }
+              ev_run = ev_id; ev1 = ev2 = evn = 0.0;
+            }
             ev1 += (double)e1; ev2 += (double)e2; evn += 1.0;
           }
           ++cnt;
@@ -1055,7 +1071,11 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
       }
       bar_compute();
     }
-    if ((EVAL && a.gt != nullptr)) {     // one atomic per CTA and quantity
+    if (GROUPED) {                       // the last run of each warp
+      if (lane == 0 && evn != 0.0 && (unsigned)ev_run < (unsigned)n_groups) {
+        atomicAdd(a.sums + 3 * ev_run, ev1); atomicAdd(a.sums + 3 * ev_run + 1, ev2); atomicAdd(a.sums + 3 * ev_run + 2, evn);
+      }
+    } else if ((EVAL && a.gt != nullptr)) {     // one atomic per CTA and quantity
       double* red = reinterpret_cast<double*>(smem + OFF_STAT);      // [3][8], free after the last tile
       if (lane == 0) { red[warp] = ev1; red[8 + warp] = ev2; red[16 + warp] = evn; }
       bar_compute();
@@ -1223,11 +1243,13 @@ int tc2_pack(dp_model* m, cudaStream_t s) {
 int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   const uint8_t* blocks = m->tc2_blocks.get<uint8_t>();
   if (!blocks) { set_error("tensor-core engine: weights are not packed"); return DP_ERR_STATE; }
-  DP_TRY((smem_opt_in<tc2_kernel<false, false, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<true, false, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, false, true>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true, true>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<true, false, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, true, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, true, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, false, true>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, true, true>>(m->device, SMEM_BYTES)));
   const size_t wbytes = (size_t)m->d.n_layer * BLOCKS_PER_LAYER * WBLK_BYTES;
   Tc2Args a{};
   a.w = m->dw.get<Weights>(); a.wpack = blocks; a.ioblocks = blocks + wbytes; a.lparams = blocks + wbytes + 2 * WBLK_BYTES;
@@ -1246,12 +1268,16 @@ int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  // a keyed call runs a keyed instantiation (without the hand-over trace, which only the plain sampler records)
-  if (a.key.on && a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true>, a, *c.inl));
-  else if (a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, true>, a, *c.inl));
-  else if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false>, a, *c.inl));
-  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false, false>, a, *c.inl));
-  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, false>, a, *c.inl));
+  // a keyed call runs a keyed instantiation (without the hand-over trace, which only the plain sampler records); group ids
+  // are only read by the evaluation tail
+  const int* grp = a.gt != nullptr ? c.group : nullptr;
+  if (grp && a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true, true>, a, *c.inl, grp, c.n_groups));
+  else if (grp) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false, true>, a, *c.inl, grp, c.n_groups));
+  else if (a.key.on && a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true, false>, a, *c.inl, grp, c.n_groups));
+  else if (a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, true, false>, a, *c.inl, grp, c.n_groups));
+  else if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false, false>, a, *c.inl, grp, c.n_groups));
+  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false, false, false>, a, *c.inl, grp, c.n_groups));
+  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, false, false>, a, *c.inl, grp, c.n_groups));
   count_launch();
   record_launch(m, grid, kThreads, SMEM_BYTES, TP, DP_ENGINE_TCG, n_tiles);
   return DP_OK;

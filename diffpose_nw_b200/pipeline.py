@@ -5,7 +5,8 @@
 
 Poses are independent, so ranks take contiguous pose ranges, keep all hypotheses of a pose on the same rank and
 exchange nothing inside the loop; one all-reduce of three fp64 partial sums ends the evaluation
-(SURVEY.md section 8e).
+(SURVEY.md section 8e).  The per-action table (common/utils.py:103-152, 247-271) is the same with one row of sums per
+action: group ids travel with the targets, and one all-reduce of [15, 3] ends it (`reduce_action_errors`).
 """
 from __future__ import annotations
 
@@ -14,8 +15,27 @@ import ctypes
 import torch
 
 from . import _lib
-from .metrics import pose_error_sums
+from .metrics import _group_sums, pose_error_sums
 from .sampler import sample
+
+# The 15 Human3.6M actions in the order of the reference's define_actions (common/utils.py), which is the row order of the
+# per-action sums; they are the names of the processed H36M files the reference's loader reads.
+H36M_ACTIONS = ("Directions", "Discussion", "Eating", "Greeting", "Phoning", "Photo", "Posing", "Purchases", "Sitting",
+                "SittingDown", "Smoking", "Waiting", "WalkDog", "Walking", "WalkTogether")
+
+
+def action_groups(actions, names=H36M_ACTIONS):
+    """The loader's per-sample action strings -> int32 CPU tensor of row indices into `names`.  A name is cut at its first
+    space as mpjpe_by_action_p1/p2 do (common/utils.py:103-152), so "Walking 1" is "Walking".  An unknown name raises
+    ValueError.  Move the result to the device (or pin it, for HostStream) like the targets."""
+    index = {a: i for i, a in enumerate(names)}
+    ids = []
+    for a in actions:
+        name = a.split(" ", 1)[0]
+        if name not in index:
+            raise ValueError(f"unknown action {a!r} (known: {', '.join(names)})")
+        ids.append(index[name])
+    return torch.tensor(ids, dtype=torch.int32)
 
 
 def shard_range(n, rank, world):
@@ -26,27 +46,33 @@ def shard_range(n, rank, world):
 
 
 def lift_and_refine(model_diff, x_uvxyz=None, *, model_pose=None, input_2d=None, src_mask=None, seq, betas, eta=0.0,
-                    test_times=1, noise=None, targets=None, sums=None, seed=None, pose_offset=0):
+                    test_times=1, noise=None, targets=None, sums=None, seed=None, pose_offset=0, groups=None):
     """Two-stage inference for one batch.  Give either `x_uvxyz` [B,17,5] or (`model_pose`, `input_2d` [B,17,2]).
     Returns the hypothesis-averaged uvxyz [B,17,5].  With `targets` [B,17,3] and `sums` (CUDA fp64 [3]) the MPJPE / P-MPJPE
     partial sums of the batch are accumulated by the sampler launch itself (`dp_sample` with targets_xyz).  `seed` draws the noise in
-    the kernel (keyed stream, see `sample`); `pose_offset` is the global index of the batch's first pose."""
+    the kernel (keyed stream, see `sample`); `pose_offset` is the global index of the batch's first pose.  `groups` (int32
+    [B], with targets): per-group sums, `sums` is then [n_groups,3] (see `sample`)."""
     if x_uvxyz is None:
         # lift + out-of-place root-centring (SURVEY.md 8a quirk 4) + concat in ONE launch (dp_lift); the sampler below is
         # the second and last launch of the batch (kernel-side repeat, hypothesis mean fused into its final store)
         x_uvxyz = getattr(model_pose, "module", model_pose).lift(input_2d, src_mask)
     return sample(model_diff, x_uvxyz, src_mask, seq, betas, eta=eta, noise=noise, n_hyp=test_times,
-                  repeat_input=True, mean_over_hyp=True, targets=targets, sums=sums, seed=seed, pose_offset=pose_offset)
+                  repeat_input=True, mean_over_hyp=True, targets=targets, sums=sums, seed=seed, pose_offset=pose_offset, groups=groups)
 
 
 def evaluate_shard(model_diff, x_uvxyz, targets_3d, *, src_mask=None, seq, betas, eta=0.0, test_times=1, noise=None,
-                   batch_size=None, model_pose=None, input_2d=None, seed=None, pose_offset=0):
+                   batch_size=None, model_pose=None, input_2d=None, seed=None, pose_offset=0, groups=None, n_groups=None):
     """Sample this rank's poses and return fp64 partial sums [sum mpjpe, sum p_mpjpe, n] (metres) on the device.
     With `seed` the noise is the keyed stream and `pose_offset` the global index of this shard's first pose (the `lo` of
-    `shard_range`): every pose then draws the same noise whatever the number of ranks or the batch size."""
+    `shard_range`): every pose then draws the same noise whatever the number of ranks or the batch size.
+    With `groups` (int32 [n], e.g. `action_groups`) and `n_groups` the sums are [n_groups,3], one row per group, ready for
+    `reduce_action_errors`."""
     n = targets_3d.shape[0]
     dev = targets_3d.device
-    sums = torch.zeros(3, device=dev, dtype=torch.float64)
+    if groups is not None:
+        sums, _ = _group_sums(None, n_groups, dev, "evaluate_shard")
+    else:
+        sums = torch.zeros(3, device=dev, dtype=torch.float64)
     bs = batch_size or max(n, 1)
     for lo in range(0, n, bs):
         hi = min(n, lo + bs)
@@ -58,7 +84,7 @@ def evaluate_shard(model_diff, x_uvxyz, targets_3d, *, src_mask=None, seq, betas
         lift_and_refine(model_diff, None if x_uvxyz is None else x_uvxyz[lo:hi], model_pose=model_pose,
                         input_2d=None if input_2d is None else input_2d[lo:hi], src_mask=src_mask, seq=seq,
                         betas=betas, eta=eta, test_times=test_times, noise=nz, targets=targets_3d[lo:hi], sums=sums,
-                        seed=seed, pose_offset=pose_offset + lo)
+                        seed=seed, pose_offset=pose_offset + lo, groups=None if groups is None else groups[lo:hi])
     return sums
 
 
@@ -73,6 +99,33 @@ def reduce_metrics(sums, group=None):
     if n == 0:
         return float("nan"), float("nan"), 0.0
     return float(s[0]) / n * 1000.0, float(s[1]) / n * 1000.0, n
+
+
+def reduce_action_errors(sums, names=H36M_ACTIONS, group=None):
+    """The per-action table of test_hyber (common/utils.py:247-271 print_error_action after test_calculation) from grouped
+    partial sums [G,3] (`evaluate_shard(groups=...)`, `sample(groups=...)`): ONE all-reduce of the [G,3] tensor across the
+    process group (in place, as reduce_metrics does), then, in millimetres,
+      table     {name: (mpjpe_mm, p_mpjpe_mm, n)} for the G = len(names) rows; an action without poses is (nan, nan, 0);
+      protocol  (protocol #1, protocol #2): the mean over the actions that have poses, each action weighted equally as
+                print_error_action does (the reference would count an action without poses as 0; see DESIGN.md);
+      totals    (mpjpe_mm, p_mpjpe_mm, n) weighted by pose, what reduce_metrics gives for the summed rows (the
+                AverageMeter line of runners/diffpose_frame.py:386-387).
+    Returns (table, protocol, totals) as python floats."""
+    import torch.distributed as dist
+    if sums.dim() != 2 or sums.shape != (len(names), 3):
+        raise RuntimeError(f"reduce_action_errors: sums must be [{len(names)},3] (one row per name), got {tuple(sums.shape)}")
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
+    s = sums.detach().double().cpu()
+    nan = float("nan")
+    table = {}
+    for name, (e1, e2, n) in zip(names, s.tolist()):
+        table[name] = (e1 / n * 1000.0, e2 / n * 1000.0, n) if n > 0 else (nan, nan, 0.0)
+    have = [v for v in table.values() if v[2] > 0]
+    protocol = (sum(v[0] for v in have) / len(have), sum(v[1] for v in have) / len(have)) if have else (nan, nan)
+    tot = s.sum(0).tolist()
+    totals = (tot[0] / tot[2] * 1000.0, tot[1] / tot[2] * 1000.0, tot[2]) if tot[2] > 0 else (nan, nan, 0.0)
+    return table, protocol, totals
 
 
 class HostStream:
@@ -132,11 +185,13 @@ class HostStream:
             _lib.check(rc, "dp_hstream_wait")
         return self.out_host[hb][:n]
 
-    def submit(self, x_host, targets_host=None, sums=None, pose_offset=None):
+    def submit(self, x_host, targets_host=None, sums=None, pose_offset=None, groups_host=None):
         """Queue one pinned host batch [n<=B,17,c] (fp32, contiguous).  Returns the oldest finished result when the ring is
         full, else None.  With `targets_host` [n,17,3] (pinned fp32) and `sums` (CUDA fp64 [3]) the batch's MPJPE / P-MPJPE
         partial sums are accumulated by the sampler launch itself (`dp_hstream_submit` with targets_host).  With a seed, `pose_offset`
-        is the global index of the batch's first pose; it defaults to the number of poses submitted before."""
+        is the global index of the batch's first pose; it defaults to the number of poses submitted before.
+        `groups_host` (pinned int32 [n], with targets_host): group ids that travel with the targets; `sums` is then CUDA
+        fp64 [n_groups,3] and each pose adds to the row of its id (`dp_hstream_submit_grouped`)."""
         n = x_host.shape[0]
         if n > self.B:
             raise RuntimeError(f"batch of {n} poses exceeds the {self.B} this HostStream was built for")
@@ -153,15 +208,26 @@ class HostStream:
             if (targets_host.is_cuda or targets_host.dtype is not torch.float32 or not targets_host.is_contiguous()
                     or tuple(targets_host.shape) != (n, 17, 3)):
                 raise RuntimeError(f"targets_host must be a contiguous fp32 HOST tensor [{n},17,3]")
-            if sums is None or not sums.is_cuda or sums.dtype is not torch.float64 or sums.numel() != 3:
+            if groups_host is not None:
+                if (groups_host.is_cuda or groups_host.dtype is not torch.int32 or not groups_host.is_contiguous()
+                        or tuple(groups_host.shape) != (n,)):
+                    raise RuntimeError(f"groups_host must be a contiguous int32 HOST tensor [{n}]")
+                if sums is None:
+                    raise RuntimeError("grouped evaluation needs `sums`: a CUDA float64 tensor [n_groups,3]")
+                sums, n_groups = _group_sums(sums, None, self.dev, "HostStream.submit")
+            elif sums is None or not sums.is_cuda or sums.dtype is not torch.float64 or sums.numel() != 3:
                 raise RuntimeError("fused evaluation needs `sums`: a CUDA float64 tensor of 3 elements")
+        elif groups_host is not None:
+            raise RuntimeError("HostStream.submit: groups_host needs targets_host and sums")
         key = _lib.noise_key(self.seed, self.n_submitted if pose_offset is None else pose_offset) if self._keyed else None
-        rc = self._lib.dp_hstream_submit(self.hs, x_host.data_ptr(), None if targets_host is None else targets_host.data_ptr(),
-                                         None if targets_host is None else sums.data_ptr(), n, self.steps, self.T, None, key,
-                                         self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
+        rc = self._lib.dp_hstream_submit_grouped(self.hs, x_host.data_ptr(), None if targets_host is None else targets_host.data_ptr(),
+                                                 None if groups_host is None else groups_host.data_ptr(),
+                                                 1 if groups_host is None else n_groups,
+                                                 None if targets_host is None else sums.data_ptr(), n, self.steps, self.T, None, key,
+                                                 self._mask_ptr, self.out_host[hb].data_ptr(), stream, self._slot_ref)
         if rc != 0:
             _lib.check(rc, "dp_hstream_submit")
-        self._pending.append((self._slot.value, hb, n, x_host, targets_host))
+        self._pending.append((self._slot.value, hb, n, x_host, targets_host, groups_host))
         self.n_submitted += n
         return ret
 

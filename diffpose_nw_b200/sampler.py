@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .metrics import _group_ids, _group_sums
 from .model import FusedGCNdiff
 
 
@@ -107,7 +108,7 @@ def _unwrap(model):
 
 
 def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_input=False, mean_over_hyp=False,
-           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0):
+           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0, groups=None):
     """Run the DDIM loop on the device and return x_T.
 
     x: [n_hyp*n_pose,17,c] hypothesis-major (what `.repeat(test_times,1,1)` produces), or [n_pose,17,c] with
@@ -122,6 +123,9 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     targets, sums: fused evaluation (`dp_sample` with targets_xyz): targets [n_pose,17,3] on the device and a CUDA fp64 tensor of 3
     partial sums `[sum mpjpe, sum p_mpjpe, n]` that every finished pose is added to in the same launch (:384-387); with
     n_hyp > 1 this needs mean_over_hyp.  Without them nothing is evaluated.
+    groups: with targets, an int32 tensor [n_pose] of group ids (e.g. `action_groups`); `sums` is then [n_groups,3] and each
+    pose adds to the row of its id, in the same launch on the default engine (`dp_sample_grouped`).  An id outside
+    [0, n_groups) adds to nothing.
     """
     m = _unwrap(model)
     xc = m._check_x(x, m._c_in)
@@ -160,9 +164,17 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     mb = m._mask_bytes(src_mask, dev)
     lib = _lib.load()
     mask_ptr = mb.data_ptr() if mb is not None else None
-    tg = None
+    tg = gid = None
+    n_groups = 1
+    if groups is not None and targets is None:
+        raise RuntimeError("sample: groups= needs targets= and sums=")
     if targets is not None:
-        if sums is None or not sums.is_cuda or sums.dtype is not torch.float64 or sums.numel() != 3:
+        if groups is not None:
+            if sums is None:
+                raise RuntimeError("grouped evaluation needs `sums`: a CUDA float64 tensor [n_groups,3]")
+            sums, n_groups = _group_sums(sums, None, dev, "sample")
+            gid = _group_ids(groups, n_pose, dev, "sample")
+        elif sums is None or not sums.is_cuda or sums.dtype is not torch.float64 or sums.numel() != 3:
             raise RuntimeError("fused evaluation needs `sums`: a CUDA float64 tensor of 3 elements")
         if n_hyp > 1 and not mean_over_hyp:
             raise RuntimeError("fused evaluation with n_hyp > 1 evaluates the hypothesis mean: pass mean_over_hyp=True")
@@ -171,10 +183,10 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
             raise RuntimeError(f"targets must be [{n_pose},{m.n_pts},3], got {tuple(tg.shape)}")
 
     def launch(x_t, out_t, n_p, nz_t, repeated, lo=0):
-        rc = lib.dp_sample(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
-                           nz_t.data_ptr() if nz_t is not None else None, key, mask_ptr, 1 if mean_over_hyp else 0,
-                           None if tg is None else tg[lo:lo + n_p].data_ptr(), None if tg is None else sums.data_ptr(),
-                           torch.cuda.current_stream(dev).cuda_stream)
+        rc = lib.dp_sample_grouped(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
+                                   nz_t.data_ptr() if nz_t is not None else None, key, mask_ptr, 1 if mean_over_hyp else 0,
+                                   None if tg is None else tg[lo:lo + n_p].data_ptr(), None if gid is None else gid[lo:lo + n_p].data_ptr(),
+                                   n_groups, None if tg is None else sums.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
         if rc != 0:
             _lib.check(rc, "dp_sample")
 

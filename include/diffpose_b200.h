@@ -169,6 +169,23 @@ int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, l
               const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
               int mean_over_hyp, const float* targets_xyz, double* sums, void* stream);
 
+/* Group-keyed evaluation: per-action MPJPE / P-MPJPE (common/utils.py:103-152 mpjpe_by_action_p1/p2 and :247-271
+ * print_error_action, as test_calculation calls them at runners/diffpose_frame.py:391) without a copy of the poses to
+ * the host.  dp_sample is dp_sample_grouped with group = NULL, n_groups = 1.
+ *   group     NULL, or int32 [n_pose] on the device: the group (for Human3.6M the action) of each pose, indexed like
+ *             targets_xyz (pose b, not row h*n_pose + b).  sums is then [n_groups][3] doubles, and row g accumulates
+ *             sum mpjpe, sum p_mpjpe and the count over the poses whose id is g.  The per-pose errors are those of the
+ *             ungrouped call (the same computation on the same inputs); only the row each one is added to changes.  A pose
+ *             whose id is outside [0, n_groups) adds to nothing, and nothing outside the [n_groups][3] block is written:
+ *             the ids are never checked on the host (that would need a synchronisation), so this holds for any value a
+ *             device buffer holds, and a batch may be padded with id -1.  The order in which CTAs add to a row is not
+ *             fixed, as for the ungrouped sums: grouped sums equal a serial sum to within reordering, not bit for bit.
+ *             On DP_ENGINE_TCG the grouping is fused into the same single launch.
+ *   Refused with DP_ERR_INVALID, before anything is enqueued: group without targets_xyz, n_groups < 1 with group. */
+int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                      const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+                      int mean_over_hyp, const float* targets_xyz, const int* group, int n_groups, double* sums, void* stream);
+
 /* Writes the keyed stream as out [n_steps][n_hyp*n_pose][n_pts][c] (hypothesis-major: row h*n_pose + p is pose
  * pose_offset + p, hypothesis h; step k is s = step_offset + k) -- the layout of dp_sample's `noise`.  So
  * dp_sample(noise = out) equals dp_sample(key) bit for bit. */
@@ -191,6 +208,9 @@ int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, 
  *            MPJPE / P-MPJPE sums to sums_dev -- the whole body of the evaluation loop (runners/diffpose_frame.py:333-387)
  *            per batch: two H2D copies, one launch, one D2H copy.  A refused combination enqueues nothing.
  *            A slot is reused after `depth` submits: wait for its result before that.
+ *   submit_grouped : the same with groups_host (int32 [n_pose], pinned; requires targets_host) and n_groups as in
+ *            dp_sample_grouped: the ids travel with the targets and sums_dev is [n_groups][3].  dp_hstream_submit is
+ *            dp_hstream_submit_grouped with groups_host = NULL, n_groups = 1.
  *   wait   : blocks the host until the result of `slot` is in its out_host.
  * Results complete in submission order. */
 typedef struct dp_hstream* dp_hstream_t;
@@ -198,6 +218,9 @@ int dp_hstream_create(dp_hstream_t* out, dp_handle h, long max_pose, int n_hyp, 
 int dp_hstream_submit(dp_hstream_t s, const float* x_host, const float* targets_host, double* sums_dev, long n_pose,
                       const dp_step* steps_host, int n_steps, const float* noise_dev, const dp_noise_key* key,
                       const unsigned char* mask_dev, float* out_host, void* stream, int* slot);
+int dp_hstream_submit_grouped(dp_hstream_t s, const float* x_host, const float* targets_host, const int* groups_host, int n_groups,
+                              double* sums_dev, long n_pose, const dp_step* steps_host, int n_steps, const float* noise_dev,
+                              const dp_noise_key* key, const unsigned char* mask_dev, float* out_host, void* stream, int* slot);
 int dp_hstream_wait(dp_hstream_t s, int slot);
 void dp_hstream_destroy(dp_hstream_t s);
 
@@ -206,9 +229,11 @@ void dp_hstream_destroy(dp_hstream_t s);
  * sums[0] += sum_pose mean_joint |pred-gt|, sums[1] += sum_pose P-MPJPE(pose), sums[2] += n.
  *   pred [n,n_pts,pred_stride] with xyz at column pred_offset (2 for uvxyz, 0 for xyz), gt [n,n_pts,3],
  *   sums: 3 doubles on the device (caller zeroes them; per-rank partials feed one all-reduce),
- *   per_pose: optional [n,2] fp32 device output (mpjpe, p_mpjpe per pose) or NULL. */
+ *   group, n_groups: NULL, or int32 [n] device ids as in dp_sample_grouped: sums is then [n_groups][3] and pose i adds to
+ *   row group[i] (to nothing when the id is outside [0, n_groups)); n_groups < 1 with group is DP_ERR_INVALID,
+ *   per_pose: optional [n,2] fp32 device output (mpjpe, p_mpjpe per pose) or NULL, the same with or without group. */
 int dp_metrics(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
-               double* sums, float* per_pose, void* stream);
+               const int* group, int n_groups, double* sums, float* per_pose, void* stream);
 
 /* Number of kernels this library has launched in this process (bench.py reports it as gpu_launches). */
 long dp_launch_count(void);
