@@ -48,6 +48,7 @@ SIGNATURES = {
     "dp_sample": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _P]),
     "dp_sample_grouped": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _I, _P,
                                _P]),
+    "dp_sample_trajectory": (_I, [_P, _P, _I, _P, _L, _I, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _I, _P, _P, _P]),
     "dp_noise_fill": (_I, [ctypes.POINTER(DpNoiseKey), _I, _L, _I, _I, _I, _P, _P]),
     "dp_hstream_create": (_I, [ctypes.POINTER(_P), _P, _L, _I, _I, _I]),
     "dp_hstream_submit": (_I, [_P, _P, _P, _P, _L, ctypes.POINTER(DpStep), _I, _P, ctypes.POINTER(DpNoiseKey), _P, _P, _P,

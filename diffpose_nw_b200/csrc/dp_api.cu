@@ -397,16 +397,10 @@ static int make_key(const dp_noise_key* k, long n_pose, const char* what, NoiseK
   return DP_OK;
 }
 
-int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-              const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
-              int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
-  return dp_sample_grouped(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, key, mask, mean_over_hyp, targets_xyz,
-                           nullptr, 1, sums, stream);
-}
-
-int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
-                      const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
-                      int mean_over_hyp, const float* targets_xyz, const int* group, int n_groups, double* sums, void* stream) {
+static int sample_impl(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                       const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+                       int mean_over_hyp, const float* targets_xyz, const int* group, int n_groups, double* sums, float* xs_traj,
+                       float* x0_traj, void* stream) {
   DP_REQUIRE(h && x_in && x_out && steps_host, "dp_sample: NULL argument");
   DP_REQUIRE(n_pose >= 0 && n_hyp >= 1 && n_steps >= 1, "dp_sample: n_pose >= 0, n_hyp >= 1, n_steps >= 1 required");
   DP_REQUIRE(h->d.has_temb, "dp_sample: handle was created with has_temb = 0 (GCNpose has no sampler)");
@@ -465,6 +459,7 @@ int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* 
   EngineCall c;
   c.x_in = x_in; c.x_is_repeated = x_is_repeated; c.out = x_out; c.n_pose = n_pose; c.n_hyp = n_hyp;
   c.n_steps = n_steps; c.steps_dev = steps_dev; c.inl = &inl; c.noise = noise; c.key = nk; c.mask = mask;
+  c.xs_traj = xs_traj; c.x0_traj = x0_traj;   // hypothesis rows, written by every engine before any mean
   const bool mean = mean_over_hyp && n_hyp > 1;
   const int eng = dp_get_engine(h);
   // default engine: the hypothesis mean -- and, with targets_xyz, the MPJPE / P-MPJPE sums -- are fused into the kernel's
@@ -482,6 +477,27 @@ int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* 
   if (mean) DP_TRY(hyp_mean_launch(c.out, x_out, n_pose, n_hyp, row_floats, s));
   if (targets_xyz != nullptr) DP_TRY(metrics_launch(x_out, d.c_out, d.c_out - 3, targets_xyz, n_pose, d.n_pts, group, n_groups, sums, nullptr, s));
   return DP_OK;
+}
+
+int dp_sample(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+              const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+              int mean_over_hyp, const float* targets_xyz, double* sums, void* stream) {
+  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, key, mask, mean_over_hyp, targets_xyz,
+                     nullptr, 1, sums, nullptr, nullptr, stream);
+}
+
+int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                      const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+                      int mean_over_hyp, const float* targets_xyz, const int* group, int n_groups, double* sums, void* stream) {
+  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, key, mask, mean_over_hyp, targets_xyz,
+                     group, n_groups, sums, nullptr, nullptr, stream);
+}
+
+int dp_sample_trajectory(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                         const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+                         int mean_over_hyp, float* xs_traj, float* x0_traj, void* stream) {
+  return sample_impl(h, x_in, x_is_repeated, x_out, n_pose, n_hyp, steps_host, n_steps, noise, key, mask, mean_over_hyp, nullptr,
+                     nullptr, 1, nullptr, xs_traj, x0_traj, stream);
 }
 
 int dp_noise_fill(const dp_noise_key* key, int n_steps, long n_pose, int n_hyp, int n_pts, int c, float* out, void* stream) {
@@ -609,9 +625,9 @@ int dp_hstream_submit_grouped(dp_hstream_t s, const float* x_host, const float* 
   // the sampler on the caller's stream, once the input is there and the slot's previous result has left the device
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_in[k], 0));
   DP_CUDA(cudaStreamWaitEvent(cs, s->ev_out[k], 0));
-  DP_TRY(dp_sample_grouped(s->h, s->x_dev[k].get<float>(), 0, s->out_dev[k].get<float>(), n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key,
-                           mask_dev, s->mean, targets_host != nullptr ? s->gt_dev[k].get<float>() : nullptr,
-                           groups_host != nullptr ? s->grp_dev[k].get<int>() : nullptr, n_groups, sums_dev, stream));
+  DP_TRY(sample_impl(s->h, s->x_dev[k].get<float>(), 0, s->out_dev[k].get<float>(), n_pose, s->n_hyp, steps_host, n_steps, noise_dev, key,
+                     mask_dev, s->mean, targets_host != nullptr ? s->gt_dev[k].get<float>() : nullptr,
+                     groups_host != nullptr ? s->grp_dev[k].get<int>() : nullptr, n_groups, sums_dev, nullptr, nullptr, stream));
   DP_CUDA(cudaEventRecord(s->ev_done[k], cs));
   // D2H on the copy-out stream
   DP_CUDA(cudaStreamWaitEvent(s->s_out, s->ev_done[k], 0));
@@ -649,7 +665,7 @@ int dp_last_launch_info(dp_handle h, long* out6) {
 }
 
 const char* dp_last_error(void) { return g_err.c_str(); }
-const char* dp_version(void) { return "diffpose_b200 0.4 (sm_100a)"; }
+const char* dp_version(void) { return "diffpose_b200 0.5 (sm_100a)"; }
 int dp_device(dp_handle h) { return h ? h->device : DP_ERR_INVALID; }
 
 void dp_destroy(dp_handle h) { delete h; }

@@ -119,6 +119,8 @@ struct EngineCall {
   NoiseKey key{};                       // key.on: the noise is the keyed stream (dp_philox.cuh) and `noise` is NULL
   const unsigned char* mask = nullptr;
   bool forward_only = false;
+  float* xs_traj = nullptr;      // sampler, every engine: x_t after step k and the x0 of that update, [n_steps][n_pose * n_hyp]
+  float* x0_traj = nullptr;      //   [n_pts][c] hypothesis-major (dp_sample_trajectory); either may be NULL
   // fused by tcg only
   bool mean_over_hyp = false;    // out is [n_pose, n_pts, c], the mean over each pose's hypotheses
   const float* gt = nullptr;     // fused evaluation tail, see dp_sample's targets_xyz

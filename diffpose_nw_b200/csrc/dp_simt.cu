@@ -43,6 +43,8 @@ struct SimtArgs {
   const unsigned char* mask;
   const dp_step* steps_dev;
   int P;
+  float* xs_traj;      // sampler: x_t after each step and the x0 of that update, [n_steps][n_rows][17][c], or NULL
+  float* x0_traj;
 };
 
 __device__ __forceinline__ float warp_sum(float v) {
@@ -330,8 +332,9 @@ __global__ void __launch_bounds__(kThreads, 1) simt_kernel(SimtArgs a, StepsArg 
           const float et = ep[r * 8 + c], xv = xt[r * 8 + c];
           const float x0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(et, st.sqrt_1m_at)), st.sqrt_at);
           float nx = __fmul_rn(st.sqrt_an, x0);
+          const size_t ot = ((size_t)step * a.n_rows + g0) * NP * cin + idx;   // element of the [n_steps][n_rows] arrays
           if (a.noise) {
-            const float z = a.noise[((size_t)step * a.n_rows + g0) * NP * cin + idx];
+            const float z = a.noise[ot];
             nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
           } else if (a.key.on) {
             // hypothesis-major row g = h * n_pose + b
@@ -340,7 +343,10 @@ __global__ void __launch_bounds__(kThreads, 1) simt_kernel(SimtArgs a, StepsArg 
                                           (uint32_t)h, (uint32_t)((r % NP) * cin + c));
             nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
           }
-          xt[r * 8 + c] = __fadd_rn(nx, __fmul_rn(st.c2, et));
+          nx = __fadd_rn(nx, __fmul_rn(st.c2, et));
+          xt[r * 8 + c] = nx;
+          if (a.xs_traj) a.xs_traj[ot] = nx;
+          if (a.x0_traj) a.x0_traj[ot] = x0;
         }
         __syncthreads();
       }
@@ -501,6 +507,7 @@ int simt_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   a.w = m->dw.get<Weights>(); a.d = m->d; a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
   a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_steps = c.n_steps; a.forward_only = c.forward_only;
   a.temb = m->temb.get<float>(); a.noise = c.noise; a.key = c.key; a.mask = c.mask; a.steps_dev = c.steps_dev;
+  a.xs_traj = c.xs_traj; a.x0_traj = c.x0_traj;
   a.P = pick_tile(m, a.n_rows);
   return dispatch_simt(m, a, *c.inl, s);
 }

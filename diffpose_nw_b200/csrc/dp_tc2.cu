@@ -380,8 +380,12 @@ __device__ __forceinline__ __half* tall_elem(uint8_t* smem, int which, int trow,
 // compute warp carries the sums of its current run of equal ids in registers across tiles and flushes them with three
 // atomics when the id changes and after its last tile.  The ids come after the by-value arguments, so the instantiations
 // without GROUPED read their arguments at the offsets they always had.
-template <bool TRACE, bool EVAL, bool KEYED, bool GROUPED>
-__global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg inl, const int* __restrict__ group, int n_groups) {
+// TRAJ = true (without EVAL) also stores, at every step k, the new x_t to xs_traj[k] and the x0 of the same update to
+// x0_traj[k] (dp_sample_trajectory; either may be NULL), both [n_steps][n_rows][17][c] hypothesis-major like the noise.
+// The two pointers come last for the same reason as the ids.
+template <bool TRACE, bool EVAL, bool KEYED, bool GROUPED, bool TRAJ>
+__global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg inl, const int* __restrict__ group, int n_groups,
+                                                          float* __restrict__ xs_traj, float* __restrict__ x0_traj) {
   auto signal_ready = [](Ctx& c) { signal_ready_t<TRACE>(c); };
   auto signal_ready_tmem = [](Ctx& c) { signal_ready_t<TRACE, false>(c); };
   auto wait_acc = [](Ctx& c) { wait_acc_t<TRACE>(c); };
@@ -1005,7 +1009,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_kernel(Tc2Args a, StepsArg in
                   const uint32_t e = e0 + (uint32_t)k;
                   nx = __fadd_rn(nx, __fmul_rn(st.c1, philox_box_muller((e >> 2) == (e0 >> 2) ? qa : qb, e & 3u)));
                 }
-                xt[r * XS + n] = __fadd_rn(nx, __fmul_rn(st.c2, et[k]));
+                nx = __fadd_rn(nx, __fmul_rn(st.c2, et[k]));
+                xt[r * XS + n] = nx;
+                if (TRAJ) {
+                  const size_t ot = (size_t)step * a.n_rows * NP * co + o + n;
+                  if (xs_traj) xs_traj[ot] = nx;
+                  if (x0_traj) x0_traj[ot] = x0;
+                }
               }
             }
           }
@@ -1243,13 +1253,15 @@ int tc2_pack(dp_model* m, cudaStream_t s) {
 int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   const uint8_t* blocks = m->tc2_blocks.get<uint8_t>();
   if (!blocks) { set_error("tensor-core engine: weights are not packed"); return DP_ERR_STATE; }
-  DP_TRY((smem_opt_in<tc2_kernel<false, false, false, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<true, false, false, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true, false, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, false, true, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true, true, false>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true, false, true>>(m->device, SMEM_BYTES)));
-  DP_TRY((smem_opt_in<tc2_kernel<false, true, true, true>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, false, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<true, false, false, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, false, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, true, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, true, false, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, false, true, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, true, true, true, false>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, false, false, true>>(m->device, SMEM_BYTES)));
+  DP_TRY((smem_opt_in<tc2_kernel<false, false, true, false, true>>(m->device, SMEM_BYTES)));
   const size_t wbytes = (size_t)m->d.n_layer * BLOCKS_PER_LAYER * WBLK_BYTES;
   Tc2Args a{};
   a.w = m->dw.get<Weights>(); a.wpack = blocks; a.ioblocks = blocks + wbytes; a.lparams = blocks + wbytes + 2 * WBLK_BYTES;
@@ -1269,15 +1281,20 @@ int tc2_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   // a keyed call runs a keyed instantiation (without the hand-over trace, which only the plain sampler records); group ids
-  // are only read by the evaluation tail
+  // are only read by the evaluation tail; a trajectory (never asked for with the evaluation) runs a TRAJ instantiation
   const int* grp = a.gt != nullptr ? c.group : nullptr;
-  if (grp && a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true, true>, a, *c.inl, grp, c.n_groups));
-  else if (grp) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false, true>, a, *c.inl, grp, c.n_groups));
-  else if (a.key.on && a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true, false>, a, *c.inl, grp, c.n_groups));
-  else if (a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, true, false>, a, *c.inl, grp, c.n_groups));
-  else if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false, false>, a, *c.inl, grp, c.n_groups));
-  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false, false, false>, a, *c.inl, grp, c.n_groups));
-  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, false, false>, a, *c.inl, grp, c.n_groups));
+  float* const xs = c.xs_traj;
+  float* const x0s = c.x0_traj;
+  if (xs || x0s) {
+    if (a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, true, false, true>, a, *c.inl, grp, c.n_groups, xs, x0s));
+    else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, false, false, true>, a, *c.inl, grp, c.n_groups, xs, x0s));
+  } else if (grp && a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true, true, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
+  else if (grp) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false, true, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
+  else if (a.key.on && a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, true, false, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
+  else if (a.key.on) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, true, false, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
+  else if (a.gt != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, true, false, false, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
+  else if (a.trace != nullptr) DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<true, false, false, false, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
+  else DP_CUDA(cudaLaunchKernelEx(&cfg, tc2_kernel<false, false, false, false, false>, a, *c.inl, grp, c.n_groups, nullptr, nullptr));
   count_launch();
   record_launch(m, grid, kThreads, SMEM_BYTES, TP, DP_ENGINE_TCG, n_tiles);
   return DP_OK;

@@ -107,6 +107,8 @@ struct TcxArgs {
   NoiseKey key;              // key.on: z from the keyed stream instead (noise is NULL)
   const unsigned char* mask;
   const dp_step* steps_dev;
+  float* xs_traj;            // sampler: x_t after each step and the x0 of that update, [n_steps][n_rows][17][c], or NULL
+  float* x0_traj;
 };
 
 struct Pipe {
@@ -745,8 +747,9 @@ __global__ void __launch_bounds__(kThreads, 1) tcx_kernel(TcxArgs a, StepsArg in
             const float et = ep[r * XS + c], xv = xt[r * XS + c];
             const float x0 = __fdiv_rn(__fsub_rn(xv, __fmul_rn(et, st.sqrt_1m_at)), st.sqrt_at);
             float nx = __fmul_rn(st.sqrt_an, x0);
+            const size_t ot = ((size_t)step * a.n_rows + g0) * NP * co + idx;   // element of the [n_steps][n_rows] arrays
             if (a.noise) {
-              const float z = a.noise[((size_t)step * a.n_rows + g0) * NP * co + idx];
+              const float z = a.noise[ot];
               nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
             } else if (a.key.on) {
               // hypothesis-major row g = h * n_pose + b
@@ -755,7 +758,10 @@ __global__ void __launch_bounds__(kThreads, 1) tcx_kernel(TcxArgs a, StepsArg in
                                             (uint32_t)h, (uint32_t)((r % NP) * co + c));
               nx = __fadd_rn(nx, __fmul_rn(st.c1, z));
             }
-            xt[r * XS + c] = __fadd_rn(nx, __fmul_rn(st.c2, et));
+            nx = __fadd_rn(nx, __fmul_rn(st.c2, et));
+            xt[r * XS + c] = nx;
+            if (a.xs_traj) a.xs_traj[ot] = nx;
+            if (a.x0_traj) a.x0_traj[ot] = x0;
           }
         }
         bar_compute();
@@ -833,6 +839,7 @@ int tcx_run(dp_model* m, const EngineCall& c, cudaStream_t s) {
   a.x_in = c.x_in; a.x_is_repeated = c.x_is_repeated; a.out = c.out;
   a.n_rows = c.n_pose * c.n_hyp; a.n_pose = c.n_pose; a.n_steps = c.n_steps;
   a.temb = m->temb.get<float>(); a.noise = c.noise; a.key = c.key; a.mask = c.mask; a.steps_dev = c.steps_dev;
+  a.xs_traj = c.xs_traj; a.x0_traj = c.x0_traj;
   const long n_tiles = (a.n_rows + TP - 1) / TP;
   const int grid = (int)(n_tiles < m->sm_count ? n_tiles : m->sm_count);
   tcx_kernel<<<grid, kThreads, SMEM_BYTES, s>>>(a, *c.inl);

@@ -108,7 +108,7 @@ def _unwrap(model):
 
 
 def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_input=False, mean_over_hyp=False,
-           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0, groups=None):
+           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0, groups=None, xs_out=None, x0_out=None):
     """Run the DDIM loop on the device and return x_T.
 
     x: [n_hyp*n_pose,17,c] hypothesis-major (what `.repeat(test_times,1,1)` produces), or [n_pose,17,c] with
@@ -126,6 +126,10 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     groups: with targets, an int32 tensor [n_pose] of group ids (e.g. `action_groups`); `sums` is then [n_groups,3] and each
     pose adds to the row of its id, in the same launch on the default engine (`dp_sample_grouped`).  An id outside
     [0, n_groups) adds to nothing.
+    xs_out, x0_out: optional CUDA fp32 tensors [T, n_hyp*n_pose, 17, c] (hypothesis-major, like `noise`) that receive the
+    denoising path from the same launch (`dp_sample_trajectory`): xs_out[k] is x_t after step k and x0_out[k] the x0
+    prediction that step's update used -- the sampler's own values, before any hypothesis mean.  Either may be given
+    alone.  Not together with `targets`.
     """
     m = _unwrap(model)
     xc = m._check_x(x, m._c_in)
@@ -148,6 +152,16 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     key = None
     if seed is not None and noise is not None:
         raise RuntimeError("sample: pass either seed= (keyed in-kernel noise) or noise=, not both")
+    traj = xs_out is not None or x0_out is not None
+    if traj and targets is not None:
+        raise RuntimeError("sample: a trajectory (xs_out= / x0_out=) is not stored together with the fused evaluation (targets=)")
+    for name, buf in (("xs_out", xs_out), ("x0_out", x0_out)):
+        if buf is None:
+            continue
+        if not torch.is_tensor(buf) or buf.device != dev or buf.dtype is not torch.float32 or not buf.is_contiguous():
+            raise RuntimeError(f"{name} must be a contiguous float32 tensor on {dev}")
+        if tuple(buf.shape) != (T, total, m.n_pts, c):
+            raise RuntimeError(f"{name} must be [{T},{total},{m.n_pts},{c}], got {tuple(buf.shape)}")
     if seed is not None:
         if any(s.c1 != 0.0 for s in steps):   # eta = 0: the seed has no effect, the call is the unkeyed one
             key = _lib.noise_key(seed, pose_offset, step_offset)
@@ -182,7 +196,17 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
         if tuple(tg.shape) != (n_pose, m.n_pts, 3):
             raise RuntimeError(f"targets must be [{n_pose},{m.n_pts},3], got {tuple(tg.shape)}")
 
-    def launch(x_t, out_t, n_p, nz_t, repeated, lo=0):
+    def ptr(t):
+        return None if t is None else t.data_ptr()
+
+    def launch(x_t, out_t, n_p, nz_t, repeated, lo=0, xs_t=None, x0_t=None):
+        if traj:
+            rc = lib.dp_sample_trajectory(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
+                                          ptr(nz_t), key, mask_ptr, 1 if mean_over_hyp else 0, ptr(xs_t), ptr(x0_t),
+                                          torch.cuda.current_stream(dev).cuda_stream)
+            if rc != 0:
+                _lib.check(rc, "dp_sample_trajectory")
+            return
         rc = lib.dp_sample_grouped(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
                                    nz_t.data_ptr() if nz_t is not None else None, key, mask_ptr, 1 if mean_over_hyp else 0,
                                    None if tg is None else tg[lo:lo + n_p].data_ptr(), None if gid is None else gid[lo:lo + n_p].data_ptr(),
@@ -192,7 +216,7 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
 
     def run():
         if not draw:
-            return launch(xc, out, n_pose, nz, not repeat_input)
+            return launch(xc, out, n_pose, nz, not repeat_input, 0, xs_out, x0_out)
         # Device-drawn noise is needed as [T, rows, 17, c] by the kernel (it runs all T steps of a tile in one go).  The
         # reference holds one step's draw at a time; to keep memory bounded like that, a large call is cut into pose chunks
         # whose noise fits NOISE_CHUNK_BYTES (the chunks are independent: poses are).  The random STREAM differs from the
@@ -200,22 +224,29 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
         row_bytes = m.n_pts * c * 4
         per_chunk = max(1, NOISE_CHUNK_BYTES // (T * row_bytes * n_hyp))
         if per_chunk >= n_pose:
-            return launch(xc, out, n_pose, torch.randn(T, total, m.n_pts, c, device=dev, dtype=torch.float32), not repeat_input)
+            return launch(xc, out, n_pose, torch.randn(T, total, m.n_pts, c, device=dev, dtype=torch.float32), not repeat_input, 0,
+                          xs_out, x0_out)
         xv = xc if repeat_input else xc.view(n_hyp, n_pose, m.n_pts, c)
         ov = out if mean_over_hyp else out.view(n_hyp, n_pose, m.n_pts, c)
         buf = torch.empty(T, per_chunk * n_hyp, m.n_pts, c, device=dev, dtype=torch.float32)
+        # a trajectory is hypothesis-major over all poses: each chunk writes its own and is scattered like `out`
+        trv = [None if t is None else t.view(T, n_hyp, n_pose, m.n_pts, c) for t in (xs_out, x0_out)]
         for lo in range(0, n_pose, per_chunk):
             hi = min(n_pose, lo + per_chunk)
             k = hi - lo
             nzc = buf[:, : k * n_hyp] if k == per_chunk else torch.empty(T, k * n_hyp, m.n_pts, c, device=dev, dtype=torch.float32)
             nzc.normal_()
             x_c = xv[lo:hi] if repeat_input else xv[:, lo:hi].reshape(k * n_hyp, m.n_pts, c).contiguous()
+            tr_c = [None if t is None else torch.empty(T, k * n_hyp, m.n_pts, c, device=dev, dtype=torch.float32) for t in trv]
             if mean_over_hyp:
-                launch(x_c, ov[lo:hi], k, nzc, not repeat_input, lo)
+                launch(x_c, ov[lo:hi], k, nzc, not repeat_input, lo, *tr_c)
             else:
                 o_c = torch.empty(k * n_hyp, m.n_pts, c, device=dev, dtype=torch.float32)
-                launch(x_c, o_c, k, nzc, not repeat_input, lo)
+                launch(x_c, o_c, k, nzc, not repeat_input, lo, *tr_c)
                 ov[:, lo:hi] = o_c.view(n_hyp, k, m.n_pts, c)
+            for t, t_c in zip(trv, tr_c):
+                if t is not None:
+                    t[:, :, lo:hi] = t_c.view(T, n_hyp, k, m.n_pts, c)
 
     if torch.cuda.current_device() == dev.index:      # the usual case: no device switch on the per-batch path
         run()
@@ -230,7 +261,8 @@ def generalized_steps(x, src_mask, seq, model, b, **kwargs):
 
     Returns `(xs, x0_preds)` with `xs = [x, x_T]` and `x0_preds = []`: the fused kernel keeps the intermediate
     x_t / x0 on chip (the only consumer in the reference takes `[0][-1]`).  Pass `return_all=True` to get the
-    full per-step lists (one single-step launch per step; slower, for debugging and parity tests).
+    full per-step lists, `xs = [x, x_1, ..., x_T]` and one x0 prediction per step: the values the sampler itself computed,
+    stored from the same single launch (`sample(xs_out=, x0_out=)`), at the cost of two [T, n, 17, c] buffers.
     Extra keyword `noise=[T,n,17,c]` supplies the per-step normal draws; `seed=` draws them in the kernel from the keyed
     stream instead (see `sample`), the same stream with and without `return_all`.
     """
@@ -240,20 +272,12 @@ def generalized_steps(x, src_mask, seq, model, b, **kwargs):
     with torch.no_grad():
         if not kwargs.get("return_all", False):
             return [x, sample(model, x, src_mask, seq, b, eta=eta, noise=noise, seed=seed)], []
-        if seed is not None and noise is not None:
-            raise RuntimeError("generalized_steps: pass either seed= or noise=, not both")
-        steps = ddim_steps(b, seq, eta)
-        xs, x0_preds = [x], []
-        for k in range(len(steps)):
-            one = (_lib.DpStep * 1)(steps[k])
-            xt = xs[-1]
-            nz = None if noise is None else noise[k:k + 1]
-            nxt = sample(model, xt, src_mask, None, b, noise=nz, steps=one, seed=seed, step_offset=k)
-            # x0 is recovered from the update rule: x_next = sqrt(an) x0 + c1 z + c2 eps, eps = (xt - sqrt(at) x0)/sqrt(1-at)
-            et = _unwrap(model)(xt, src_mask, torch.full((xt.shape[0],), steps[k].t, device=xt.device), 0)
-            x0_preds.append((xt - et * steps[k].sqrt_1m_at) / steps[k].sqrt_at)
-            xs.append(nxt)
-        return xs, x0_preds
+        m = _unwrap(model)
+        shape = (len(seq), x.shape[0], m.n_pts, m._c_in)
+        xs_out = torch.empty(shape, device=x.device, dtype=torch.float32)
+        x0_out = torch.empty(shape, device=x.device, dtype=torch.float32)
+        sample(model, x, src_mask, seq, b, eta=eta, noise=noise, seed=seed, xs_out=xs_out, x0_out=x0_out)
+        return [x] + list(xs_out.unbind(0)), list(x0_out.unbind(0))
 
 
 def philox_noise(seed, n_steps, n_pose, n_hyp=1, *, pose_offset=0, step_offset=0, device=None, n_pts=17, c=5):

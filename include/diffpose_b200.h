@@ -186,6 +186,22 @@ int dp_sample_grouped(dp_handle h, const float* x_in, int x_is_repeated, float* 
                       const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
                       int mean_over_hyp, const float* targets_xyz, const int* group, int n_groups, double* sums, void* stream);
 
+/* The denoising path: dp_sample that also stores what the reference's generalized_steps returns as (xs, x0_preds)
+ * (common/utils_diff.py:46-67), from the same single launch and as the values the sampler itself computed.
+ *   xs_traj   NULL, or [n_steps][n_pose*n_hyp][n_pts][c] fp32: xs_traj[k] is x_t after step k (execution order, 0 = the
+ *             largest t), i.e. the reference's xs[k + 1];
+ *   x0_traj   NULL, or the same shape: x0_traj[k] is the x0 prediction (x_t - eps sqrt(1 - abar_t)) / sqrt(abar_t) that
+ *             the update of step k used, the reference's x0_preds[k].
+ * Rows are hypothesis-major (h*n_pose + b), the layout of `noise`, with or without mean_over_hyp: x_out then holds the
+ * mean and the trajectory every hypothesis.  Without the mean, xs_traj[n_steps-1] equals x_out bit for bit.  The caller
+ * allocates and sizes both buffers (n_steps*n_pose*n_hyp*n_pts*c floats each); nothing else is allocated for them, so
+ * the call is CUDA-graph capturable under the same rules as dp_sample.  The fused evaluation is not offered here.
+ * With both pointers NULL this is dp_sample with targets_xyz = sums = NULL; otherwise the same arguments are refused with
+ * DP_ERR_INVALID, before anything is enqueued. */
+int dp_sample_trajectory(dp_handle h, const float* x_in, int x_is_repeated, float* x_out, long n_pose, int n_hyp,
+                         const dp_step* steps_host, int n_steps, const float* noise, const dp_noise_key* key, const unsigned char* mask,
+                         int mean_over_hyp, float* xs_traj, float* x0_traj, void* stream);
+
 /* Writes the keyed stream as out [n_steps][n_hyp*n_pose][n_pts][c] (hypothesis-major: row h*n_pose + p is pose
  * pose_offset + p, hypothesis h; step k is s = step_offset + k) -- the layout of dp_sample's `noise`.  So
  * dp_sample(noise = out) equals dp_sample(key) bit for bit. */
