@@ -58,6 +58,7 @@ SIGNATURES = {
     "dp_hstream_wait": (_I, [_P, _I]),
     "dp_hstream_destroy": (None, [_P]),
     "dp_metrics": (_I, [_P, _I, _I, _P, _L, _I, _P, _I, _P, _P, _P]),
+    "dp_metrics_hyp": (_I, [_P, _I, _I, _I, _P, _L, _I, _P, _I, _P, _P, _P, _P]),
     "dp_selftest_umma": (_I, [_P, _I, _P, _I, _P, _I, _P]),
     "dp_selftest_umma_ts": (_I, [_P, _I, _P, _I, _I, _P, _I, _P, _I, _P]),
     "dp_selftest_cycles": (_I, [ctypes.POINTER(ctypes.c_longlong)]),

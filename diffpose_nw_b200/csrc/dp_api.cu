@@ -520,6 +520,18 @@ int dp_metrics(const float* pred, int pred_stride, int pred_offset, const float*
   return metrics_launch(pred, pred_stride, pred_offset, gt, n, n_pts, group, n_groups, sums, per_pose, static_cast<cudaStream_t>(stream));
 }
 
+int dp_metrics_hyp(const float* pred, int pred_stride, int pred_offset, int n_hyp, const float* gt, long n, int n_pts, const int* group,
+                   int n_groups, double* sums, float* mean_out, float* per_hyp, void* stream) {
+  DP_REQUIRE(pred && gt && sums, "dp_metrics_hyp: NULL argument");
+  DP_REQUIRE(n_hyp >= 1, "dp_metrics_hyp: n_hyp >= 1 required");
+  DP_REQUIRE(n_pts == kMaxPts, "dp_metrics_hyp: n_pts must be 17");
+  DP_REQUIRE(pred_stride >= 3 && pred_offset >= 0 && pred_offset + 3 <= pred_stride, "dp_metrics_hyp: bad pred stride/offset");
+  DP_REQUIRE(!group || n_groups >= 1, "dp_metrics_hyp: group ids need n_groups >= 1");
+  if (n <= 0) return n == 0 ? DP_OK : DP_ERR_INVALID;
+  return metrics_hyp_launch(pred, pred_stride, pred_offset, n_hyp, gt, n, group, n_groups, sums, mean_out, per_hyp,
+                            static_cast<cudaStream_t>(stream));
+}
+
 int dp_selftest_umma(const void* smem_image, int image_bytes, const dp_mma_op* ops_host, int n_ops, float* tmem_out, int ncols,
                      void* stream) {
   DP_REQUIRE(smem_image && ops_host && tmem_out, "dp_selftest_umma: NULL argument");

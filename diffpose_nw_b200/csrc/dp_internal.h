@@ -201,6 +201,9 @@ int tc2_tau(dp_model* m, int n_steps, cudaStream_t s);
 // group != NULL: pose i adds to sums[3 * group[i] ..] of [n_groups][3], and nothing when group[i] is outside [0, n_groups)
 int metrics_launch(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
                    const int* group, int n_groups, double* sums, float* per_pose, cudaStream_t s);
+// dp_metrics_hyp: pred [n_hyp][n][n_pts][pred_stride] hypothesis-major; sums [n_groups][8] (group = NULL: row 0)
+int metrics_hyp_launch(const float* pred, int pred_stride, int pred_offset, int n_hyp, const float* gt, long n, const int* group,
+                       int n_groups, double* sums, float* mean_out, float* per_hyp, cudaStream_t s);
 int hyp_mean_launch(const float* x, float* out, long n_pose, int n_hyp, int row_floats, cudaStream_t s);
 // out[n][n_pts][c_in + c_out] = [uv | xyz - xyz[root]] (runners/diffpose_frame.py:337-343 with out-of-place root-centring)
 int lift_glue_launch(const float* uv, const float* xyz, float* out, long n, int n_pts, int c_in, int c_out, cudaStream_t s);

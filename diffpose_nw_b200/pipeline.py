@@ -6,16 +6,18 @@
 Poses are independent, so ranks take contiguous pose ranges, keep all hypotheses of a pose on the same rank and
 exchange nothing inside the loop; one all-reduce of three fp64 partial sums ends the evaluation
 (SURVEY.md section 8e).  The per-action table (common/utils.py:103-152, 247-271) is the same with one row of sums per
-action: group ids travel with the targets, and one all-reduce of [15, 3] ends it (`reduce_action_errors`).
+action: group ids travel with the targets, and one all-reduce of [15, 3] ends it (`reduce_action_errors`).  With several
+hypotheses per pose, `hyp_sums` / `hyp_metrics=True` score all of them ([8] or [15, 8] sums, `reduce_hyp_errors`).
 """
 from __future__ import annotations
 
 import ctypes
+from typing import NamedTuple
 
 import torch
 
 from . import _lib
-from .metrics import _group_sums, pose_error_sums
+from .metrics import HYP_COLS, _group_sums, pose_error_sums
 from .sampler import sample
 
 # The 15 Human3.6M actions in the order of the reference's define_actions (common/utils.py), which is the row order of the
@@ -46,33 +48,39 @@ def shard_range(n, rank, world):
 
 
 def lift_and_refine(model_diff, x_uvxyz=None, *, model_pose=None, input_2d=None, src_mask=None, seq, betas, eta=0.0,
-                    test_times=1, noise=None, targets=None, sums=None, seed=None, pose_offset=0, groups=None):
+                    test_times=1, noise=None, targets=None, sums=None, seed=None, pose_offset=0, groups=None, hyp_sums=None):
     """Two-stage inference for one batch.  Give either `x_uvxyz` [B,17,5] or (`model_pose`, `input_2d` [B,17,2]).
     Returns the hypothesis-averaged uvxyz [B,17,5].  With `targets` [B,17,3] and `sums` (CUDA fp64 [3]) the MPJPE / P-MPJPE
     partial sums of the batch are accumulated by the sampler launch itself (`dp_sample` with targets_xyz).  `seed` draws the noise in
     the kernel (keyed stream, see `sample`); `pose_offset` is the global index of the batch's first pose.  `groups` (int32
-    [B], with targets): per-group sums, `sums` is then [n_groups,3] (see `sample`)."""
+    [B], with targets): per-group sums, `sums` is then [n_groups,3] (see `sample`).  `hyp_sums` (CUDA fp64 [8] or
+    [n_groups,8], with targets and in place of `sums`): the multi-hypothesis evaluation of `sample(hyp_sums=)`."""
     if x_uvxyz is None:
         # lift + out-of-place root-centring (SURVEY.md 8a quirk 4) + concat in ONE launch (dp_lift); the sampler below is
         # the second and last launch of the batch (kernel-side repeat, hypothesis mean fused into its final store)
         x_uvxyz = getattr(model_pose, "module", model_pose).lift(input_2d, src_mask)
     return sample(model_diff, x_uvxyz, src_mask, seq, betas, eta=eta, noise=noise, n_hyp=test_times,
-                  repeat_input=True, mean_over_hyp=True, targets=targets, sums=sums, seed=seed, pose_offset=pose_offset, groups=groups)
+                  repeat_input=True, mean_over_hyp=True, targets=targets, sums=sums, seed=seed, pose_offset=pose_offset, groups=groups,
+                  hyp_sums=hyp_sums)
 
 
 def evaluate_shard(model_diff, x_uvxyz, targets_3d, *, src_mask=None, seq, betas, eta=0.0, test_times=1, noise=None,
-                   batch_size=None, model_pose=None, input_2d=None, seed=None, pose_offset=0, groups=None, n_groups=None):
+                   batch_size=None, model_pose=None, input_2d=None, seed=None, pose_offset=0, groups=None, n_groups=None,
+                   hyp_metrics=False):
     """Sample this rank's poses and return fp64 partial sums [sum mpjpe, sum p_mpjpe, n] (metres) on the device.
     With `seed` the noise is the keyed stream and `pose_offset` the global index of this shard's first pose (the `lo` of
     `shard_range`): every pose then draws the same noise whatever the number of ranks or the batch size.
     With `groups` (int32 [n], e.g. `action_groups`) and `n_groups` the sums are [n_groups,3], one row per group, ready for
-    `reduce_action_errors`."""
+    `reduce_action_errors`.
+    With `hyp_metrics=True` every hypothesis is scored (`sample(hyp_sums=)`): the sums are [8] or [n_groups,8] with the
+    columns of `hyp_error_sums`, ready for `reduce_hyp_errors`."""
     n = targets_3d.shape[0]
     dev = targets_3d.device
+    cols = HYP_COLS if hyp_metrics else 3
     if groups is not None:
-        sums, _ = _group_sums(None, n_groups, dev, "evaluate_shard")
+        sums, _ = _group_sums(None, n_groups, dev, "evaluate_shard", cols=cols)
     else:
-        sums = torch.zeros(3, device=dev, dtype=torch.float64)
+        sums = torch.zeros(cols, device=dev, dtype=torch.float64)
     bs = batch_size or max(n, 1)
     for lo in range(0, n, bs):
         hi = min(n, lo + bs)
@@ -83,7 +91,8 @@ def evaluate_shard(model_diff, x_uvxyz, targets_3d, *, src_mask=None, seq, betas
         # sampler + metrics of the batch in one launch (two with the lifter in front)
         lift_and_refine(model_diff, None if x_uvxyz is None else x_uvxyz[lo:hi], model_pose=model_pose,
                         input_2d=None if input_2d is None else input_2d[lo:hi], src_mask=src_mask, seq=seq,
-                        betas=betas, eta=eta, test_times=test_times, noise=nz, targets=targets_3d[lo:hi], sums=sums,
+                        betas=betas, eta=eta, test_times=test_times, noise=nz, targets=targets_3d[lo:hi],
+                        sums=None if hyp_metrics else sums, hyp_sums=sums if hyp_metrics else None,
                         seed=seed, pose_offset=pose_offset + lo, groups=None if groups is None else groups[lo:hi])
     return sums
 
@@ -125,6 +134,54 @@ def reduce_action_errors(sums, names=H36M_ACTIONS, group=None):
     protocol = (sum(v[0] for v in have) / len(have), sum(v[1] for v in have) / len(have)) if have else (nan, nan)
     tot = s.sum(0).tolist()
     totals = (tot[0] / tot[2] * 1000.0, tot[1] / tot[2] * 1000.0, tot[2]) if tot[2] > 0 else (nan, nan, 0.0)
+    return table, protocol, totals
+
+
+class HypErrors(NamedTuple):
+    """Multi-hypothesis errors in millimetres, in the column order of the sums (`hyp_error_sums`)."""
+    mean_mpjpe: float        # of the hypothesis mean
+    mean_p_mpjpe: float
+    n: float                 # poses
+    best_mpjpe: float        # best-of-H
+    best_p_mpjpe: float
+    jbest_mpjpe: float       # per-joint best
+    avg_mpjpe: float         # average hypothesis
+    avg_p_mpjpe: float
+
+
+def _hyp_row(row):
+    n = row[2]
+    if n <= 0:
+        nan = float("nan")
+        return HypErrors(nan, nan, 0.0, nan, nan, nan, nan, nan)
+    mm = [v / n * 1000.0 for v in row]
+    return HypErrors(mm[0], mm[1], n, *mm[3:])
+
+
+def reduce_hyp_errors(sums, names=None, group=None):
+    """Multi-hypothesis sums [8] or [G,8] (`hyp_error_sums`, `sample(hyp_sums=)`, `evaluate_shard(hyp_metrics=True)`) ->
+    millimetres: ONE all-reduce of the tensor across the process group (in place, as reduce_metrics does), then
+      without names  the totals over all rows, a HypErrors (pose-weighted; nan when there are no poses);
+      with names     (table, protocol, totals) as reduce_action_errors: table {name: HypErrors} for the G = len(names) rows
+                     (an action without poses is all nan with n = 0), protocol the mean of each column over the actions that
+                     have poses, each action weighted equally (n = their poses), and totals as above.
+    Returns python floats."""
+    import torch.distributed as dist
+    if sums.shape[-1:] != (HYP_COLS,) or sums.dim() not in (1, 2) or (names is not None and tuple(sums.shape) != (len(names), HYP_COLS)):
+        want = f"[{len(names)},{HYP_COLS}] (one row per name)" if names is not None else f"[{HYP_COLS}] or [G,{HYP_COLS}]"
+        raise RuntimeError(f"reduce_hyp_errors: sums must be {want}, got {tuple(sums.shape)}")
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
+    s = sums.detach().double().cpu().reshape(-1, HYP_COLS)
+    totals = _hyp_row(s.sum(0).tolist())
+    if names is None:
+        return totals
+    table = {name: _hyp_row(row) for name, row in zip(names, s.tolist())}
+    have = [v for v in table.values() if v.n > 0]
+    if have:
+        protocol = HypErrors(*[sum(v[k] for v in have) / len(have) if k != 2 else sum(v.n for v in have) for k in range(HYP_COLS)])
+    else:
+        protocol = _hyp_row([0.0] * HYP_COLS)
     return table, protocol, totals
 
 

@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .metrics import _group_ids, _group_sums
+from .metrics import _group_ids, _group_sums, _hyp_sums, _metrics_hyp
 from .model import FusedGCNdiff
 
 
@@ -108,7 +108,8 @@ def _unwrap(model):
 
 
 def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_input=False, mean_over_hyp=False,
-           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0, groups=None, xs_out=None, x0_out=None):
+           steps=None, targets=None, sums=None, seed=None, pose_offset=0, step_offset=0, groups=None, xs_out=None, x0_out=None,
+           hyp_sums=None):
     """Run the DDIM loop on the device and return x_T.
 
     x: [n_hyp*n_pose,17,c] hypothesis-major (what `.repeat(test_times,1,1)` produces), or [n_pose,17,c] with
@@ -130,6 +131,11 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     denoising path from the same launch (`dp_sample_trajectory`): xs_out[k] is x_t after step k and x0_out[k] the x0
     prediction that step's update used -- the sampler's own values, before any hypothesis mean.  Either may be given
     alone.  Not together with `targets`.
+    hyp_sums: with targets, the multi-hypothesis evaluation in place of `sums`: a CUDA fp64 tensor [8] (or [n_groups,8] with
+    `groups`) that receives the columns of `hyp_error_sums` -- mean-pose, best-of-H, per-joint best and average-hypothesis
+    MPJPE / P-MPJPE and the count.  The sampler writes all n_hyp rows of each pose and `dp_metrics_hyp` scores them: two
+    launches, whatever the engine.  The result is the hypothesis mean with mean_over_hyp (written by that second launch,
+    equal to the sampler's own mean bit for bit), else the n_hyp rows.  Not together with `sums` or a trajectory.
     """
     m = _unwrap(model)
     xc = m._check_x(x, m._c_in)
@@ -153,6 +159,13 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     if seed is not None and noise is not None:
         raise RuntimeError("sample: pass either seed= (keyed in-kernel noise) or noise=, not both")
     traj = xs_out is not None or x0_out is not None
+    if hyp_sums is not None:
+        if sums is not None:
+            raise RuntimeError("sample: pass either sums= (hypothesis mean) or hyp_sums= (multi-hypothesis evaluation), not both")
+        if targets is None:
+            raise RuntimeError("sample: hyp_sums= needs targets=")
+        if traj:
+            raise RuntimeError("sample: a trajectory (xs_out= / x0_out=) is not stored together with hyp_sums=")
     if traj and targets is not None:
         raise RuntimeError("sample: a trajectory (xs_out= / x0_out=) is not stored together with the fused evaluation (targets=)")
     for name, buf in (("xs_out", xs_out), ("x0_out", x0_out)):
@@ -182,7 +195,9 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
     n_groups = 1
     if groups is not None and targets is None:
         raise RuntimeError("sample: groups= needs targets= and sums=")
-    if targets is not None:
+    if hyp_sums is not None:
+        hyp_sums, gid, n_groups = _hyp_sums(hyp_sums, groups, None, n_pose, dev, "sample")
+    elif targets is not None:
         if groups is not None:
             if sums is None:
                 raise RuntimeError("grouped evaluation needs `sums`: a CUDA float64 tensor [n_groups,3]")
@@ -192,6 +207,7 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
             raise RuntimeError("fused evaluation needs `sums`: a CUDA float64 tensor of 3 elements")
         if n_hyp > 1 and not mean_over_hyp:
             raise RuntimeError("fused evaluation with n_hyp > 1 evaluates the hypothesis mean: pass mean_over_hyp=True")
+    if targets is not None:
         tg = targets.detach().to(device=dev, dtype=torch.float32).contiguous()
         if tuple(tg.shape) != (n_pose, m.n_pts, 3):
             raise RuntimeError(f"targets must be [{n_pose},{m.n_pts},3], got {tuple(tg.shape)}")
@@ -200,6 +216,19 @@ def sample(model, x, src_mask, seq, b, eta=0.0, noise=None, n_hyp=1, repeat_inpu
         return None if t is None else t.data_ptr()
 
     def launch(x_t, out_t, n_p, nz_t, repeated, lo=0, xs_t=None, x0_t=None):
+        if hyp_sums is not None:
+            # every hypothesis row from the sampler (into out_t itself when it holds them), then the evaluation, which also
+            # writes the mean
+            mean = mean_over_hyp and n_hyp > 1
+            rows = torch.empty(n_p * n_hyp, m.n_pts, c, device=dev, dtype=torch.float32) if mean else out_t
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            rc = lib.dp_sample_grouped(m._handle, x_t.data_ptr(), 1 if repeated else 0, rows.data_ptr(), n_p, n_hyp, steps, T, ptr(nz_t),
+                                       key, mask_ptr, 0, None, None, 1, None, stream)
+            if rc != 0:
+                _lib.check(rc, "dp_sample")
+            _metrics_hyp(lib, rows, c, n_hyp, tg[lo:lo + n_p], n_p, None if gid is None else gid[lo:lo + n_p], n_groups, hyp_sums,
+                         out_t if mean else None, None, stream)
+            return
         if traj:
             rc = lib.dp_sample_trajectory(m._handle, x_t.data_ptr(), 1 if repeated else 0, out_t.data_ptr(), n_p, n_hyp, steps, T,
                                           ptr(nz_t), key, mask_ptr, 1 if mean_over_hyp else 0, ptr(xs_t), ptr(x0_t),

@@ -251,6 +251,33 @@ void dp_hstream_destroy(dp_hstream_t s);
 int dp_metrics(const float* pred, int pred_stride, int pred_offset, const float* gt, long n, int n_pts,
                const int* group, int n_groups, double* sums, float* per_pose, void* stream);
 
+/* Multi-hypothesis evaluation: the scores of probabilistic pose estimators over the H hypotheses of each pose, in one
+ * launch that follows dp_sample with mean_over_hyp = 0 (two launches per batch; the sampler is not changed).
+ *   pred      [n_hyp][n][n_pts][pred_stride] hypothesis-major with xyz at column pred_offset: row h*n + b is hypothesis h of
+ *             pose b, exactly what dp_sample writes with mean_over_hyp = 0;  gt [n][n_pts][3];
+ *   group, n_groups   as in dp_metrics: NULL (sums is one row), or int32 [n] device ids and sums [n_groups][8]; a pose whose
+ *             id is outside [0, n_groups) adds to nothing; atomics make the sums equal a serial sum up to reordering;
+ *   sums      [n_groups][8] fp64 on the device, accumulated into (the caller zeroes them);
+ *   mean_out  NULL, or [n][n_pts][pred_stride]: the hypothesis mean of every channel (the mean dp_sample gives with
+ *             mean_over_hyp = 1);
+ *   per_hyp   NULL, or [n_hyp][n][2] fp32: MPJPE, P-MPJPE of every hypothesis, the values dp_metrics gives for that row.
+ * Definitions (part of the ABI).  Both poses are root-centred out of place; e1_h, e2_h are the MPJPE and P-MPJPE of
+ * hypothesis h (dp_metrics' per_pose on row h*n + b, bit for bit); d_hj is the root-centred distance of joint j in
+ * hypothesis h, computed with the same operations as that MPJPE.  Row g, column k of sums adds over the poses of group g:
+ *   0, 1  MPJPE / P-MPJPE of the hypothesis mean m = (sum_h row_h) / H: fp32, summed from h = 0 upwards starting at 0, then
+ *         one division -- the mean every engine's dp_sample produces, bit for bit
+ *   2     1 (the count)
+ *   3, 4  best-of-H: min_h e1_h and min_h e2_h, each minimised on its own; a NaN (the P-MPJPE of a zero-extent hypothesis)
+ *         propagates, as numpy's min
+ *   5     per-joint best (J-best): (1/17) sum_j min_h d_hj, reduced with the MPJPE's own summation order and division, so
+ *         with H = 1 it equals column 0 per pose, bit for bit
+ *   6, 7  average hypothesis: (sum_h e1_h) / H and (sum_h e2_h) / H, summed in fp64 in h order
+ * Per pose J-best <= best-of-H <= average.  Only enqueues (nothing is allocated): CUDA-graph capturable.  Refused with
+ * DP_ERR_INVALID before anything is enqueued: NULL pred / gt / sums, n_hyp < 1, n_pts != 17, a bad stride / offset,
+ * n_groups < 1 with group. */
+int dp_metrics_hyp(const float* pred, int pred_stride, int pred_offset, int n_hyp, const float* gt, long n, int n_pts,
+                   const int* group, int n_groups, double* sums, float* mean_out, float* per_hyp, void* stream);
+
 /* Number of kernels this library has launched in this process (bench.py reports it as gpu_launches). */
 long dp_launch_count(void);
 
